@@ -5,6 +5,7 @@
   python bench.py --impl reference --gpus N --steps K ...        # the reference's CPU path (oracle port)
   python bench.py --config c3 | c5 ...                           # BASELINE configs C3 / C5 (same arms)
   python bench.py --pool-workers N                               # ONE process, WorkerPool with N GPU workers
+  python bench.py ... --dump-outputs DIR                         # + what the last timed step computed, DIR/<name>.npy
 
 Config C2 (default): a "step" is one pass of the hot path over one batch: 4 x (UNet forward + LCM
 scheduler step) followed by the VAE decode of a batch of 16 images (at N GPUs each rank runs its own
@@ -28,15 +29,19 @@ import os
 import statistics
 import subprocess
 import sys
+import tempfile
 import threading
 import time
 from types import SimpleNamespace
 
+# the benchmark runs from a built tree that may be read-only: it writes nothing there, byte code included
+sys.dont_write_bytecode = True
 ROOT = os.path.dirname(os.path.abspath(__file__))
 if ROOT not in sys.path:
     sys.path.insert(0, ROOT)
 
 UNIT = "images/s"
+DUMP_BYTES_MAX = 64 * 10**6
 # algorithmic GFLOP per sample (2*MAC), SURVEY.md §8(d) / BASELINE.md §3
 CONFIGS = {
     "c2": dict(arch="sd15", size=512, lcm_steps=4, batch=16, gs=1.0, gflop_unet=803.27, gflop_vae=2514.52,
@@ -66,6 +71,21 @@ def peaks():
         d = json.load(open(p))
         return d.get("bf16_tflops_sustained", 1386.3), d.get("bf16_tflops", 1632.4), d.get("hbm_gbs", 6535.7), "measured"
     return 1400.0, 1590.0, 6650.0, "fallback"
+
+
+def dump_outputs(out_dir, **arrays):
+    """Writes each device tensor as out_dir/<name>.npy in float32, so that two builds run with the same arguments
+    (hence the same seeded inputs) can be compared output for output.  Above DUMP_BYTES_MAX in all, every array is
+    cut to a fixed, seeded sample of its flattened elements: the same positions on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.float().cpu().numpy() for k, v in arrays.items()}
+    frac = min(1.0, (DUMP_BYTES_MAX - 4096) / (4 * sum(a.size for a in arrays.values())))
+    for name, a in arrays.items():
+        if frac < 1.0:
+            keep = np.random.default_rng(0).choice(a.size, int(a.size * frac), replace=False)
+            a = a.reshape(-1)[np.sort(keep)]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -228,7 +248,7 @@ def bench_model_dir(c, rank, barrier):
     """Random-init diffusers-layout model directory the worker loads (`MODEL_ROOT/MODEL`): written once
     per box by rank 0."""
     from dreamlab_b200 import synthetic as syn
-    root = os.environ.get("B200_BENCH_MODEL_ROOT", "/tmp/dreamlab_b200_bench_models")
+    root = os.environ.get("B200_BENCH_MODEL_ROOT", os.path.join(tempfile.gettempdir(), "dreamlab_b200_bench_models"))
     name = "sd15-lcm" if c["arch"] == "sd15" else "sdxl-base"
     path = os.path.join(root, name)
     done = os.path.join(path, ".complete")
@@ -309,10 +329,7 @@ def run_b200(args, c):
             dist.all_reduce(t, op=dist.ReduceOp.MAX)
         return t.item()
 
-    import __graft_entry__ as g
-    if rank == 0:
-        g.build()
-    barrier()
+    _lib.load()         # the library __graft_entry__.build() compiled: nothing is compiled at run time
     if c["arch"] == "sdxl":
         return run_b200_c5(args, c, rank, local, world, dev, barrier, max_over_ranks)
     from dreamlab_b200 import lib
@@ -350,6 +367,9 @@ def run_b200(args, c):
         b.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        # what generate(..., return_latents=True) hands its caller: u8 images NHWC and the final latents NHWC
+        dump_outputs(args.dump_outputs, image=gr.img, latents=gr.final)
     step_ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = max_over_ranks(sum(step_ms))
     value = world * B * args.steps / (total_ms / 1e3)
@@ -557,12 +577,14 @@ def run_b200_c5(args, c, rank, local, world, dev, barrier, max_over_ranks):
             img = den.generate(*a, nsteps, gs, use_graph=True, vae_strips=True)
             if host:
                 img_h.copy_(img, non_blocking=True)
+            return img
     else:
         def step(host: bool):
             a = (pe_h, lat_h, noise_h) if host else (pe_d, lat_d, noise_d)
             img = pipe.generate(*a, nsteps, gs, use_graph=True, pooled_embeds=pooled_h if host else pooled_d)
             if host:
                 img_h.copy_(img, non_blocking=True)
+            return img
     n0 = lib.launch_count
     for _ in range(max(args.warmup, 3)):
         step(False)
@@ -577,10 +599,12 @@ def run_b200_c5(args, c, rank, local, world, dev, barrier, max_over_ranks):
     for a, b in evs:
         l2_flush.zero_()
         a.record()
-        step(False)
+        img = step(False)
         b.record()
     barrier()
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, image=img)
     step_ms = [a.elapsed_time(b) for a, b in evs]
     total_ms = max_over_ranks(sum(step_ms))
     value = n_groups * args.steps / (total_ms / 1e3)
@@ -641,8 +665,7 @@ def run_pool(args, c):
     _lib.wait_for_driver()
     if not torch.cuda.is_available():
         raise RuntimeError("bench.py: no CUDA device; the b200 arm has no CPU fallback")
-    import __graft_entry__ as g
-    g.build()
+    _lib.load()
     n = args.pool_workers
     ngpu = min(n, torch.cuda.device_count())      # more workers than GPUs: worker k runs on cuda:(k % GPUs)
     os.environ["B200_PNG"] = os.environ.get("B200_PNG", "").strip().lower() or "gpu"
@@ -695,7 +718,12 @@ def main():
                     help="config c5: ranks per image (default: all ranks shard ONE image); 2 = one image per GPU pair")
     ap.add_argument("--pool-workers", type=int, default=0,
                     help="one process, WorkerPool with this many GPU workers; prints the e2e line only")
+    ap.add_argument("--dump-outputs", metavar="DIR", default="",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (float32, "
+                         f"at most {DUMP_BYTES_MAX // 10**6} MB in all; b200 arm, --config c2 / c3 / c5)")
     args = ap.parse_args()
+    if args.dump_outputs and (args.impl != "b200" or args.pool_workers):
+        ap.error("--dump-outputs: the b200 arm's timed path only (not --impl reference or --pool-workers)")
     c = dict(CONFIGS[args.config])
     if args.batch:
         c["batch"] = args.batch

@@ -11,16 +11,16 @@ torch / PIL to run:
 
 The module itself cannot be imported (it imports `diffusers` and `rknnlite` at load), so the
 function sources are cut out of the file with `ast` and executed UNMODIFIED in a namespace that
-holds numpy / torch / PIL.  `extract()` is used live by tests/test_reference_pin.py when
-/root/reference exists (this container); `python tests/golden/make_reference_host_golden.py` writes
-the committed fixture `reference_host_pieces.npz` that travels to the GPU box, where the reference
-tree does not exist.  Nothing of the reference's source is copied into the repo.
+holds numpy / torch / PIL.  `python tests/golden/make_reference_host_golden.py <reference checkout>`
+writes the committed fixture `reference_host_pieces.npz` that tests/test_reference_pin.py compares
+against.  Nothing of the reference's source is copied into the repo.
 """
 from __future__ import annotations
 
 import ast
 import logging
 import os
+import sys
 import textwrap
 from types import SimpleNamespace
 
@@ -28,7 +28,6 @@ import numpy as np
 import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
-REFERENCE = os.environ.get("DREAMLAB_REFERENCE", "/root/reference")
 FIXTURE = os.path.join(HERE, "reference_host_pieces.npz")
 
 
@@ -48,7 +47,7 @@ def _cut(path: str, names) -> dict:
     return out
 
 
-def extract(reference_root: str = REFERENCE) -> SimpleNamespace:
+def extract(reference_root: str) -> SimpleNamespace:
     """The reference's own functions, executed from its own source text."""
     from typing import List, Optional, Union
     from PIL import Image
@@ -86,8 +85,8 @@ def inputs():
     return image, lat, lat96
 
 
-def generate(ref=None) -> dict:
-    ref = ref or extract()
+def generate(reference_root: str) -> dict:
+    ref = extract(reference_root)
     image, lat, lat96 = inputs()
     out = {"image_in": image, "lat64": lat, "lat96": lat96}
     w = np.asarray(GUIDANCE, dtype=np.float32) - 1.0
@@ -105,5 +104,7 @@ def generate(ref=None) -> dict:
 
 
 if __name__ == "__main__":
-    np.savez_compressed(FIXTURE, **generate())
+    if len(sys.argv) != 2:
+        sys.exit("usage: python tests/golden/make_reference_host_golden.py <checkout of the reference repository>")
+    np.savez_compressed(FIXTURE, **generate(sys.argv[1]))
     print("wrote", FIXTURE, os.path.getsize(FIXTURE), "bytes")

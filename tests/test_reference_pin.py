@@ -5,8 +5,7 @@ tree with `ast` and executes their source unmodified (guidance-scale embedding, 
 prepare_latents: `backends/rknnlcm.py:651-677, 212-264, 423-447`; 8x8 latent pooling:
 `backends/rknn_worker.py:223-248`).  Their outputs on seeded inputs are the committed fixture
 `tests/golden/reference_host_pieces.npz`.  Here:
-  * CPU: the fixture is re-derived live when /root/reference exists (so it cannot go stale), and
-    `oracle/` + the product's host scheduler code are compared against it;
+  * CPU: `oracle/` + the product's host scheduler code are compared against the fixture;
   * GPU (-m gpu): the CUDA kernels that implement the same pieces (u8 image tail — fused conv
     epilogue and the crop kernel —, 8x8 pooling) are compared against it through the C-ABI.
 Bars: bit-exact for u8 / integer work and the latent draw; fp32 results within the rounding of the
@@ -24,17 +23,6 @@ sys.path.insert(0, os.path.join(HERE, "golden"))
 import make_reference_host_golden as mk  # noqa: E402
 
 FIX = np.load(mk.FIXTURE)
-
-
-def test_fixture_is_what_the_reference_computes_here():
-    """Live re-run of the reference's own source (this container only: the GPU box has no reference)."""
-    if not os.path.exists(os.path.join(mk.REFERENCE, "backends", "rknnlcm.py")):
-        pytest.skip("reference tree not present (GPU box): the committed fixture stands")
-    live = mk.generate()
-    assert sorted(live) == sorted(FIX.files)
-    for k in FIX.files:
-        assert live[k].dtype == FIX[k].dtype and live[k].shape == FIX[k].shape, k
-        assert np.array_equal(live[k], FIX[k]), f"fixture {k} differs from the reference run live"
 
 
 def _emb_tol(w, dim):
@@ -122,13 +110,8 @@ def test_cuda_image_crop_u8_bit_exact_vs_reference():
     `postprocess` of those very values byte for byte."""
     lib = _lib()
     img = torch.from_numpy(FIX["image_in"]).to(torch.bfloat16).float()
-    mkref = None
-    if os.path.exists(os.path.join(mk.REFERENCE, "backends", "rknnlcm.py")):
-        mkref = np.stack([np.asarray(im) for im in mk.extract().postprocess_pil(img.numpy())])
     from oracle.pipeline import denormalize_to_u8         # pinned to the reference bit-exactly above
     ref = denormalize_to_u8(img)
-    if mkref is not None:
-        assert np.array_equal(ref, mkref)
     src = img.permute(0, 2, 3, 1).contiguous().cuda()
     n, h, w, c = src.shape
     out = torch.zeros(n, h, w, c, device="cuda", dtype=torch.uint8)
