@@ -259,8 +259,9 @@ int dl_peer_allgather(const void* src, void* dst, long long nbytes, void* const*
  * The same operators with fp32 activations and weights on the CUDA cores (plain tiled kernels,
  * accurate expf / erff): they exist for the parity bar of the fp32 pipeline (noise_pred within
  * 1e-4), not for speed.  Same argument meaning as their bf16 namesakes; dl_igemm_f32 reads the
- * same descriptor (a0/a1/wgt/residual/out are float; GroupNorm partials and clusters ignored;
- * channels multiples of 16).                                                                   */
+ * same descriptor (a0/a1/wgt/residual/out are float; bn ignored; channels multiples of 16).  It has
+ * no fused statistics and no peer stores: a descriptor with gn_partial, row_stats_out, ln_stats or
+ * n_peer_out > 0 is refused.                                                                   */
 int dl_igemm_f32(const dl_igemm_desc* desc, void* stream);
 int dl_groupnorm_f32(const float* x0, int c0, const float* x1, int c1, int nimg, int hw, int groups,
                      float eps, const float* gamma, const float* beta, int apply_silu, float* out,

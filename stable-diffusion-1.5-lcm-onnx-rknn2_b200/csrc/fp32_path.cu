@@ -364,6 +364,12 @@ extern "C" int dl_igemm_f32(const dl_igemm_desc* d, void* stream_) {
                "igemm_f32: taps must be 1, 9, or 4 with tap_phase");
   DL_CHECK_ARG(d->c0 > 0 && d->c0 % 16 == 0 && d->c1 % 16 == 0, "igemm_f32: channels must be multiples of 16");
   DL_CHECK_ARG(d->mode >= 0 && d->mode <= DL_EPI_U8_IMAGE, "igemm_f32: bad epilogue mode");
+  // the fused statistics and peer stores of the bf16 kernel have no fp32 counterpart: refuse them
+  // rather than leave the caller's buffers unwritten
+  DL_CHECK_ARG(!d->gn_partial, "igemm_f32: the fp32 mode has no fused GroupNorm statistics (gn_partial)");
+  DL_CHECK_ARG(!d->row_stats_out, "igemm_f32: the fp32 mode has no fused row statistics (row_stats_out)");
+  DL_CHECK_ARG(!d->ln_stats, "igemm_f32: the fp32 mode has no folded LayerNorm statistics (ln_stats)");
+  DL_CHECK_ARG(d->n_peer_out == 0, "igemm_f32: the fp32 mode has no peer stores (n_peer_out=%d)", d->n_peer_out);
   F32GemmParams p;
   memset(&p, 0, sizeof(p));
   p.a0 = reinterpret_cast<const float*>(d->a0); p.a0_ps = d->a0_pix_stride; p.c0 = d->c0;
