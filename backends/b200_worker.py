@@ -11,6 +11,8 @@ step and VAE decode run in `dreamlab_b200` (hand-written sm_100a kernels, no dif
 Extras the reference does not have (SURVEY.md §8f rank 1): `run_batch(jobs)` generates many
 requests of the same geometry in ONE batched pass (per-request Philox streams preserved) and
 `run_job_with_latents` returns the latent of the same pass instead of re-running the pipeline.
+Requests carrying `init_image` (and `strength`, see `backends/base.py`) run image-to-image through
+the same entry points (`LatentConsistencyModelImg2ImgPipeline` semantics, LCM UNets only).
 """
 from __future__ import annotations
 
@@ -228,11 +230,42 @@ class B200Worker(PipelineWorker):
         (zeros are an SDXL-only convention, `force_zeros_for_empty_prompt`)."""
         return self._text.encode([""] * n)
 
-    def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True):
+    def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True, init=None):
+        """init (image-to-image): (u8 images [B,H,W,3], posterior draw [B,4,h,w], strength); lat is then the
+        add_noise draw."""
         pe = self._text.encode(prompts)
         neg = self._negative(len(prompts)) if self.pipe.cfg_scale_for(gs) is not None else None
+        i2i = {}
+        if init is not None:
+            i2i = dict(init_images=init[0], posterior_noise=init[1], strength=init[2])
         return self.pipe.generate(pe, lat, noise, steps, gs, return_latents=True, use_graph=self._use_graph,
-                                  negative_prompt_embeds=neg, decode=decode)
+                                  negative_prompt_embeds=neg, decode=decode, **i2i)
+
+    def _check_img2img(self) -> None:
+        """Refuse image-to-image where this engine does not implement diffusers' semantics."""
+        if not self.pipe.unet.cfg.time_cond_proj_dim:
+            raise RuntimeError("image-to-image needs an LCM UNet (time_cond_proj_dim): the LCM img2img pipeline has "
+                               "no classifier-free guidance branch, and CFG img2img is not implemented")
+        self.pipe.require_encoder()
+
+    @staticmethod
+    def _init_image(obj, width: int, height: int):
+        """A request's init_image (image bytes PIL opens, or an HxWx3 uint8 array) -> contiguous RGB uint8
+        [height, width, 3].  No resizing: any other size is refused."""
+        import numpy as np
+        if isinstance(obj, (bytes, bytearray, memoryview)):
+            from PIL import Image
+            with Image.open(io.BytesIO(bytes(obj))) as im:
+                arr = np.asarray(im.convert("RGB"))
+        else:
+            arr = np.asarray(obj)
+            if arr.dtype != np.uint8 or arr.ndim != 3 or arr.shape[2] != 3:
+                raise RuntimeError(f"init_image: image bytes or an HxWx3 uint8 array expected, got "
+                                   f"{arr.dtype} {list(arr.shape)}")
+        if arr.shape[:2] != (height, width):
+            raise RuntimeError(f"init_image is {arr.shape[1]}x{arr.shape[0]}, the request's size is "
+                               f"{width}x{height} (init images are not resized)")
+        return np.ascontiguousarray(arr)
 
     # ------------------------------------------------------------------ jobs
     def _parse(self, req):
@@ -249,19 +282,23 @@ class B200Worker(PipelineWorker):
             int(torch.randint(0, 100_000_000, (1,)).item())
         return width, height, seed
 
-    def _draw(self, seed: int, h8: int, w8: int, steps: int, raw: bool = False):
+    def _draw(self, seed: int, h8: int, w8: int, steps: int, raw: bool = False, posterior: bool = False):
         """The reference's per-request Philox stream (`backends/cuda_worker.py:212-213`,
-        SURVEY.md App. A.5): latents first, then one draw per non-final step."""
+        SURVEY.md App. A.5): latents first, then one draw per non-final step.
+        posterior (image-to-image): the posterior sample's draw comes first and is returned third; the
+        "latents" draw is then the add_noise noise (diffusers' prepare_latents order)."""
         gen = torch.Generator(device=self.device)
         gen.manual_seed(seed)
         shape = (1, 4, h8, w8)
+        eps_s = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32) if posterior else None
         lat = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32)
         noise = [torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32)
                  for _ in range(steps - 1)]
         if not raw:
             lat = lat.to(self.dtype).float()
             noise = [z.to(self.dtype).float() for z in noise]
-        return lat, noise
+            eps_s = eps_s.to(self.dtype).float() if posterior else None
+        return (lat, noise, eps_s) if posterior else (lat, noise)
 
     supports_deferred = True      # run_batch(..., deferred=True) -> thunks (see WorkerPool)
 
@@ -285,9 +322,25 @@ class B200Worker(PipelineWorker):
             for (w, h, _), j in zip(parsed, jobs):
                 if (w, h) != (width, height) or int(j.req.num_inference_steps) != steps:
                     raise RuntimeError("run_batch: jobs must share size and num_inference_steps")
+            inits = [getattr(j.req, "init_image", None) for j in jobs]
+            init = None
+            if any(x is not None for x in inits):
+                if any(x is None for x in inits):
+                    raise RuntimeError("run_batch: image-to-image and text-to-image jobs cannot share a batch")
+                strengths = {0.8 if getattr(j.req, "strength", None) is None else float(j.req.strength) for j in jobs}
+                if len(strengths) != 1:
+                    raise RuntimeError("run_batch: image-to-image jobs must share strength")
+                self._check_img2img()
+                # host work on this thread: PNG / JPEG decoding of the init images
+                import numpy as np
+                imgs = torch.from_numpy(np.stack([self._init_image(x, width, height) for x in inits]))
+                init = [imgs, None, next(iter(strengths))]
             # per-request Philox streams; the round trip through the noise dtype (CUDA_DTYPE) is applied once to
             # the assembled batch instead of per tensor (same values, ~8 fewer launches per request)
-            draws = [self._draw(seed, height // 8, width // 8, steps, raw=True) for _, _, seed in parsed]
+            draws = [self._draw(seed, height // 8, width // 8, steps, raw=True, posterior=init is not None)
+                     for _, _, seed in parsed]
+            if init is not None:
+                init[1] = torch.cat([d[2] for d in draws], 0).to(self.dtype).float()
             lat = torch.cat([d[0] for d in draws], 0).to(self.dtype).float()
             noise = (torch.stack([torch.cat([d[1][i] for d in draws], 0) for i in range(steps - 1)]).to(self.dtype).float()
                      if steps > 1 else None)
@@ -298,7 +351,8 @@ class B200Worker(PipelineWorker):
             self._apply_style(*next(iter(styles)))
             try:
                 img, final = self._generate([str(j.req.prompt) for j in jobs], lat, noise, steps, gs,
-                                            height, width, decode=not latents_only)
+                                            height, width, decode=not latents_only,
+                                            **({"init": tuple(init)} if init is not None else {}))
             finally:
                 self._apply_style(None, 0)          # reset: no state bleed into the next job
             from dreamlab_b200 import lib
@@ -387,6 +441,11 @@ class B200SDXLWorker(B200Worker):
     when guidance_scale > 1 (all jobs of one batch must then share the scale), SDXL VAE."""
     _tag = "b200-sdxl"
     _env_what = "SDXL CUDA worker"
+
+    def _check_img2img(self) -> None:
+        raise RuntimeError("image-to-image is not implemented for SDXL: StableDiffusionXLImg2ImgPipeline truncates "
+                           "the full schedule (get_timesteps), which is different semantics from the LCM img2img "
+                           "pipeline built here")
 
     def _make_text_encoder(self, path):
         ucfg = self.pipe.unet.cfg

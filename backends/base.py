@@ -5,6 +5,11 @@ reference `backends/worker_pool.py:84-88`).  A request object is duck-typed: wor
 `req.prompt`, `req.size` ("WIDTHxHEIGHT"), `req.num_inference_steps`, `req.guidance_scale`,
 `req.seed` (optional) and `getattr(req, "style_lora", None)`.
 
+Image-to-image (`LatentConsistencyModelImg2ImgPipeline` semantics) is requested with two more optional
+fields, also read with `getattr`: `init_image` — image bytes PIL can open (PNG, JPEG, ...) or an HxWx3
+uint8 array (what `run_job_array` returns), RGB and exactly `size` (no resizing) — and `strength` in
+(0, 1] (default 0.8): how far the init image is noised before the LCM steps redraw it.
+
 Only names, fields and return conventions are shared with the reference — they ARE the
 interface; everything a caller can observe is pinned by `tests/test_worker_pool.py` and
 `tests/test_worker_factory.py`.
@@ -52,6 +57,8 @@ class GenSpec:
     cfg: float
     seed: Optional[int] = None
     style_lora: StyleLora = field(default_factory=StyleLora)
+    init_image: Any = None                   # image-to-image: image bytes or HxWx3 uint8 array
+    strength: Optional[float] = None         # image-to-image strength (None: 0.8)
 
 
 @dataclass

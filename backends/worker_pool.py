@@ -123,7 +123,8 @@ def _auto_num_workers() -> int:
 
 def _batch_key(job, same_guidance: bool = False):
     """Generation jobs that may share one batched pass: same size, step count and style (and,
-    for workers that run classifier-free guidance on a doubled batch, the same guidance scale)."""
+    for workers that run classifier-free guidance on a doubled batch, the same guidance scale).
+    Image-to-image requests (an `init_image`) also share their strength: ("img2img", strength) is appended."""
     req = getattr(job, "req", None)
     try:
         if same_guidance:
@@ -132,7 +133,11 @@ def _batch_key(job, same_guidance: bool = False):
         style = (getattr(sl, "style", None), int(getattr(sl, "level", 0) or 0)) if sl else (None, 0)
         if not style[0] or style[1] <= 0:
             style = (None, 0)
-        return (str(req.size).lower(), int(req.num_inference_steps), style)
+        key = (str(req.size).lower(), int(req.num_inference_steps), style)
+        if getattr(req, "init_image", None) is not None:
+            st = getattr(req, "strength", None)
+            key += (("img2img", 0.8 if st is None else float(st)),)
+        return key
     except Exception:
         return None
 

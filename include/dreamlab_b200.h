@@ -190,6 +190,10 @@ int dl_im2col_s2(const void* x, int nimg, int h, int w, int c, void* cols, void*
  * y + in_row0 (rows outside [0, in_rows) read as zero); h = logical rows of the strip           */
 int dl_im2col_s2_halo(const void* x, int nimg, int in_rows, int in_row0, int h, int w, int c,
                       void* cols, void* stream);
+/* same layout for the VAE encoder's Downsample2D(padding=0): F.pad(x, (0,1,0,1)) then conv3x3 stride 2
+ * without padding, i.e. tap (ky,kx) of output (yo,xo) reads input (2yo+ky, 2xo+kx), zero past the last
+ * row / column.  h, w even; output (h/2) x (w/2).                                               */
+int dl_im2col_s2_pad01(const void* x, int nimg, int h, int w, int c, void* cols, void* stream);
 /* bf16 [npix, cpad] <- mat . (fp32 NHWC [npix, cin] * scale) + vec, zero-padded to cpad channels
  * (feeds conv_in).  mat/vec: optional fp32 [cin,cin] / [cin] = the VAE post_quant_conv 1x1 and the
  * `latents / scaling_factor` of reference `backends/rknnlcm.py:614` (K13); NULL = identity.     */
@@ -274,6 +278,7 @@ int dl_attention_f32(const float* q, long long ldq, const float* k, long long ld
 int dl_pack_latent_f32(const float* x, long long npix, int cin, int cpad, float scale,
                        const float* mat, const float* vec, float* out, void* stream);
 int dl_im2col_s2_f32(const float* x, int nimg, int h, int w, int c, float* cols, void* stream);
+int dl_im2col_s2_pad01_f32(const float* x, int nimg, int h, int w, int c, float* cols, void* stream);
 int dl_softmax_rows_f32(const float* scores, long long rows, int cols, float* out, void* stream);
 int dl_small_linear_f32(const float* x, int m, int k, const float* w, const float* bias,
                         const float* add, int n, int silu_in, int silu_out, float* out, void* stream);
@@ -296,6 +301,24 @@ long long dl_png_stored_size(int h, int w);
 long long dl_png_stored_workspace_bytes(int nimg, int h);
 int dl_png_stored(const void* img_u8, int nimg, int h, int w, void* out, long long out_stride,
                   void* workspace, void* stream);
+
+/* ---- image-to-image (diffusers LatentConsistencyModelImg2ImgPipeline + AutoencoderKL.encode) -----------------
+ * dl_pack_image_im2col: u8 RGB NHWC init image -> the im2col operand of the encoder's conv_in (3 -> 128, 3x3,
+ * padding 1) as a 1x1 GEMM with K = 64: out[p, tap*3 + c] (tap = ky*3 + kx) = 2 * (u8 / 255) - 1 (IEEE division,
+ * no contraction), 0 for taps outside the h x w window and for K >= 27.  row_stride / img_stride are in bytes, so a
+ * tile window of a larger canvas is read in place (its border taps are zero, not the canvas' neighbour pixels).
+ * out: bf16 (or fp32 for the _f32 variant) [nimg*h*w, 64], 16-byte aligned.
+ * dl_vae_sample_latents: moments fp32 NHWC [n,h,w,8] (mean | logvar) -> latents fp32 NHWC [n,h,w,4]:
+ *   logvar = clamp(logvar, -30, 20); std = expf(0.5 logvar); x0 = scaling_factor * (mean + std * eps_s);
+ *   out = sqrt_alpha * x0 + sqrt_one_minus_alpha * eps_n       (every mul / add rounded on its own)
+ * eps_s / eps_n fp32 NCHW [n,4,h,w] as drawn; mean_out (optional) receives the mean, NHWC [n,h,w,4].         */
+int dl_pack_image_im2col(const void* img_u8, int nimg, int h, int w, long long row_stride, long long img_stride,
+                         void* out, void* stream);
+int dl_pack_image_im2col_f32(const void* img_u8, int nimg, int h, int w, long long row_stride,
+                             long long img_stride, float* out, void* stream);
+int dl_vae_sample_latents(const float* moments, const float* eps_s, const float* eps_n, int nimg, int h, int w,
+                          float scaling_factor, float sqrt_alpha, float sqrt_one_minus_alpha, float* out,
+                          float* mean_out, void* stream);
 
 #ifdef __cplusplus
 }

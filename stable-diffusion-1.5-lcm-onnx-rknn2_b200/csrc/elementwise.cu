@@ -107,9 +107,12 @@ __global__ void upsample2x_kernel(const uint4* __restrict__ x, int nimg, int h, 
   }
 }
 
-// ---- im2col for conv3x3 stride 2 pad 1 (Downsample2D): cols[(n,yo,xo), tap*c + ch] ----------
+// ---- im2col for conv3x3 stride 2 (Downsample2D): cols[(n,yo,xo), tap*c + ch] -----------------
+// pad = 1: the UNet's symmetric padding 1; pad = 0: the VAE encoder's F.pad(x, (0,1,0,1)) followed
+// by an unpadded conv (tap (ky,kx) of output (yo,xo) reads input (2yo+ky, 2xo+kx), the last row and
+// column of taps fall on the zero pad)
 __global__ void im2col_s2_kernel(const uint4* __restrict__ x, int nimg, int h, int w, int V,
-                                 uint4* __restrict__ cols, int in_rows, int in_row0) {
+                                 uint4* __restrict__ cols, int in_rows, int in_row0, int pad) {
   const int ho = h / 2, wo = w / 2;
   const long long total = (long long)nimg * ho * wo * 9 * V;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
@@ -122,8 +125,8 @@ __global__ void im2col_s2_kernel(const uint4* __restrict__ x, int nimg, int h, i
     r /= wo;
     const int yo = (int)(r % ho);
     const int n = (int)(r / ho);
-    const int yi = 2 * yo + tap / 3 - 1 + in_row0;
-    const int xi = 2 * xo + tap % 3 - 1;
+    const int yi = 2 * yo + tap / 3 - pad + in_row0;
+    const int xi = 2 * xo + tap % 3 - pad;
     uint4 val = make_uint4(0, 0, 0, 0);
     if (yi >= 0 && yi < in_rows && xi >= 0 && xi < w)
       val = __ldg(x + (((long long)n * in_rows + yi) * w + xi) * V + v);
@@ -471,8 +474,16 @@ extern "C" int dl_im2col_s2(const void* x, int nimg, int h, int w, int c, void* 
   DL_CHECK_ARG(x && cols && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "im2col_s2: bad args");
   const long long total = (long long)nimg * (h / 2) * (w / 2) * 9 * (c / 8);
   im2col_s2_kernel<<<grid_for(total, 256), 256, 0, STREAM>>>(
-      reinterpret_cast<const uint4*>(x), nimg, h, w, c / 8, reinterpret_cast<uint4*>(cols), h, 0);
+      reinterpret_cast<const uint4*>(x), nimg, h, w, c / 8, reinterpret_cast<uint4*>(cols), h, 0, 1);
   return check_launch("im2col_s2");
+}
+
+extern "C" int dl_im2col_s2_pad01(const void* x, int nimg, int h, int w, int c, void* cols, void* stream_) {
+  DL_CHECK_ARG(x && cols && c % 8 == 0 && h % 2 == 0 && w % 2 == 0, "im2col_s2_pad01: bad args");
+  const long long total = (long long)nimg * (h / 2) * (w / 2) * 9 * (c / 8);
+  im2col_s2_kernel<<<grid_for(total, 256), 256, 0, STREAM>>>(
+      reinterpret_cast<const uint4*>(x), nimg, h, w, c / 8, reinterpret_cast<uint4*>(cols), h, 0, 0);
+  return check_launch("im2col_s2_pad01");
 }
 
 extern "C" int dl_im2col_s2_halo(const void* x, int nimg, int in_rows, int in_row0, int h, int w, int c,
@@ -481,7 +492,7 @@ extern "C" int dl_im2col_s2_halo(const void* x, int nimg, int in_rows, int in_ro
                "im2col_s2_halo: bad args");
   const long long total = (long long)nimg * (h / 2) * (w / 2) * 9 * (c / 8);
   im2col_s2_kernel<<<grid_for(total, 256), 256, 0, STREAM>>>(
-      reinterpret_cast<const uint4*>(x), nimg, h, w, c / 8, reinterpret_cast<uint4*>(cols), in_rows, in_row0);
+      reinterpret_cast<const uint4*>(x), nimg, h, w, c / 8, reinterpret_cast<uint4*>(cols), in_rows, in_row0, 1);
   return check_launch("im2col_s2_halo");
 }
 

@@ -282,8 +282,9 @@ __global__ void f32_pack_latent_kernel(const float* __restrict__ x, long long np
   }
 }
 
+// pad = 1: symmetric padding 1; pad = 0: bottom / right zero pad (see im2col_s2_kernel)
 __global__ void f32_im2col_s2_kernel(const float4* __restrict__ x, int nimg, int h, int w, int V,
-                                     float4* __restrict__ cols) {
+                                     float4* __restrict__ cols, int pad) {
   const int ho = h / 2, wo = w / 2;
   const long long total = (long long)nimg * ho * wo * 9 * V;
   for (long long i = blockIdx.x * (long long)blockDim.x + threadIdx.x; i < total;
@@ -296,7 +297,7 @@ __global__ void f32_im2col_s2_kernel(const float4* __restrict__ x, int nimg, int
     r /= wo;
     const int yo = (int)(r % ho);
     const int n = (int)(r / ho);
-    const int yi = 2 * yo + tap / 3 - 1, xi = 2 * xo + tap % 3 - 1;
+    const int yi = 2 * yo + tap / 3 - pad, xi = 2 * xo + tap % 3 - pad;
     float4 val = make_float4(0.f, 0.f, 0.f, 0.f);
     if (yi >= 0 && yi < h && xi >= 0 && xi < w) val = x[(((long long)n * h + yi) * w + xi) * V + v];
     cols[i] = val;
@@ -445,8 +446,16 @@ extern "C" int dl_im2col_s2_f32(const float* x, int nimg, int h, int w, int c, f
   DL_CHECK_ARG(x && cols && c % 4 == 0 && h % 2 == 0 && w % 2 == 0, "im2col_s2_f32: bad args");
   const long long total = (long long)nimg * (h / 2) * (w / 2) * 9 * (c / 4);
   f32_im2col_s2_kernel<<<f32_grid(total, 256), 256, 0, STREAM>>>(reinterpret_cast<const float4*>(x), nimg, h, w,
-                                                                c / 4, reinterpret_cast<float4*>(cols));
+                                                                c / 4, reinterpret_cast<float4*>(cols), 1);
   return check_launch("im2col_s2_f32");
+}
+
+extern "C" int dl_im2col_s2_pad01_f32(const float* x, int nimg, int h, int w, int c, float* cols, void* stream_) {
+  DL_CHECK_ARG(x && cols && c % 4 == 0 && h % 2 == 0 && w % 2 == 0, "im2col_s2_pad01_f32: bad args");
+  const long long total = (long long)nimg * (h / 2) * (w / 2) * 9 * (c / 4);
+  f32_im2col_s2_kernel<<<f32_grid(total, 256), 256, 0, STREAM>>>(reinterpret_cast<const float4*>(x), nimg, h, w,
+                                                                c / 4, reinterpret_cast<float4*>(cols), 0);
+  return check_launch("im2col_s2_pad01_f32");
 }
 
 extern "C" int dl_softmax_rows_f32(const float* scores, long long rows, int cols, float* out, void* stream_) {

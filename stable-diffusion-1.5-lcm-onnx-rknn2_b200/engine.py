@@ -21,7 +21,7 @@ import torch
 
 from . import lib
 from .scheduler import LCMSchedule, guidance_scale_embedding
-from .weights import Packed, pack_unet, pack_vae_decoder
+from .weights import Packed, has_vae_encoder, pack_unet, pack_vae_decoder, pack_vae_encoder
 
 BF16 = torch.bfloat16
 
@@ -471,6 +471,94 @@ class UNetB200:
 
 
 # ------------------------------------------------------------------------------------------------
+# VAE mid-block attention (shared by the encoder and the decoder)
+# ------------------------------------------------------------------------------------------------
+def _vae_flash_ok(flash, sq, skv, C):
+    return flash and sq % 128 == 0 and skv % 64 == 0 and C % 128 == 0 and C <= 512
+
+
+def vae_mid_attention(ctx, x, a: Packed, *, groups: int, flash: bool):
+    """AutoencoderKL mid-block attention (encoder and decoder): heads=1, d=C (512).  Token counts the wide flash
+    kernel tiles (multiples of 128: every full decode) go through it; otherwise QK^T and PV through the tcgen05 GEMM with fp32 scores per image, or the CUDA-core
+    flash kernel for ragged tiles."""
+    B, H, W, C = x.shape
+    S = H * W
+    hn = groupnorm(ctx, x, a["norm_w"], a["norm_b"], eps=1e-6, silu=False, groups=groups)
+    hn2 = hn.view(B * S, C)
+    if ctx.comm is not None:
+        return _vae_mid_attention_strips(ctx, x, hn2, a, flash)
+    qk = linear(ctx, hn2, a["qk_w"], a["qk_b"], 2 * C)                 # [B*S, 2C]
+    o = ctx.empty(B * S, C)
+    if _vae_flash_ok(flash, S, S, C):
+        # b_v is folded into the out-proj bias (softmax rows sum to 1), as in the other branches
+        v = linear(ctx, hn2, a["v_w"], None, C)
+        lib.attention_wide(qk, qk[:, C:], v, o, batch=B, sq=S, skv=S, d=C, ldq=2 * C, ldk=2 * C, ldv=C, ldo=C,
+                           scale=1.0 / math.sqrt(C))
+        out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C), norm_rows_per_img=S)
+        return _carry_gn(out, out.view(B, H, W, C))
+    if S % 64 or ctx.dt != BF16:
+        # fp32 precision mode, and ragged tiles of a tiled decode (token count not a multiple of the 64-deep GEMM K
+        # chunk, e.g. a 29 x 29 corner tile): the CUDA-core flash kernel takes any length.
+        # b_v is folded into the out-proj bias exactly as below (softmax rows sum to 1).
+        v = linear(ctx, hn2, a["v_w"], None, C)
+        lib.attention(qk, qk[:, C:], v, o, batch=B, sq=S, skv=S, heads=1, d=C, dh_stride=C,
+                      ldq=2 * C, ldk=2 * C, ldv=C, ldo=C, scale=1.0 / math.sqrt(C), impl=lib.ATTN_SIMT)
+        out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C))
+        return out.view(B, H, W, C)
+    scores = ctx.empty(S, S, dtype=torch.float32)
+    probs = ctx.empty(S, S)
+    vt = ctx.empty(C, S)
+    for b in range(B):
+        rows = slice(b * S, (b + 1) * S)
+        # V^T[c, s] = sum_k Wv[c,k] X[s,k]  (bias folded into the out-proj bias)
+        lib.igemm(a["v_w"], hn2[rows], vt, nimg=1, h=1, w=C, taps=1, n=S, a0_stride=C, ldo=S)
+        q, k = qk[rows, :C], qk[rows, C:]
+        lib.igemm(q, k, scores, nimg=1, h=1, w=S, taps=1, n=S, c0=C, a0_stride=2 * C,
+                  mode=lib.EPI_F32, alpha=1.0 / math.sqrt(C), ldo=S)
+        lib.softmax_rows(scores, probs)
+        lib.igemm(probs, vt, o[rows], nimg=1, h=1, w=S, taps=1, n=C, a0_stride=S, ldo=C)
+    out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C), norm_rows_per_img=S)
+    return _carry_gn(out, out.view(B, H, W, C))
+
+
+def _vae_mid_attention_strips(ctx, x, hn2, a: Packed, flash: bool):
+    """Row strips (SURVEY.md §8e, VAE row): the queries of this rank's S tokens attend to the
+    keys / values of all R*S tokens.  ONE exchange: the normalised tokens are all-gathered
+    (rank order = image row order) and every rank projects K and V^T from them itself — the
+    two projections are 2*R*S*C^2 MACs, far cheaper than a second and third gather."""
+    B, H, W, C = x.shape
+    S = H * W
+    comm = ctx.comm
+    hn_all = comm.gather_rows(hn2.view(B, S, C))                        # [B, R*S, C]
+    Sa = hn_all.shape[1]
+    hn_all = hn_all.reshape(B * Sa, C)
+    scale = 1.0 / math.sqrt(C)
+    q = linear(ctx, hn2, a["qk_w"][:C], a["qk_b"][:C], C)               # [B*S, C]
+    k = linear(ctx, hn_all, a["qk_w"][C:], a["qk_b"][C:], C)            # [B*Sa, C]
+    o = ctx.empty(B * S, C)
+    if _vae_flash_ok(flash, S, Sa, C):
+        v = linear(ctx, hn_all, a["v_w"], None, C)
+        lib.attention_wide(q, k, v, o, batch=B, sq=S, skv=Sa, d=C, ldq=C, ldk=C, ldv=C, ldo=C, scale=scale)
+    elif Sa % 64:                     # ragged key count: the CUDA-core flash kernel takes any length
+        v = linear(ctx, hn_all, a["v_w"], None, C)
+        lib.attention(q, k, v, o, batch=B, sq=S, skv=Sa, heads=1, d=C, dh_stride=C,
+                      ldq=C, ldk=C, ldv=C, ldo=C, scale=scale, impl=lib.ATTN_SIMT)
+    else:
+        scores = ctx.empty(S, Sa, dtype=torch.float32)
+        probs = ctx.empty(S, Sa)
+        vt = ctx.empty(C, Sa)
+        for b in range(B):
+            rows, keys = slice(b * S, (b + 1) * S), slice(b * Sa, (b + 1) * Sa)
+            lib.igemm(a["v_w"], hn_all[keys], vt, nimg=1, h=1, w=C, taps=1, n=Sa, a0_stride=C, ldo=Sa)
+            lib.igemm(q[rows], k[keys], scores, nimg=1, h=1, w=S, taps=1, n=Sa, c0=C, a0_stride=C,
+                      mode=lib.EPI_F32, alpha=scale, ldo=Sa)
+            lib.softmax_rows(scores, probs)
+            lib.igemm(probs, vt, o[rows], nimg=1, h=1, w=S, taps=1, n=C, a0_stride=Sa, ldo=C)
+    out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C))
+    return out.view(B, H, W, C)
+
+
+# ------------------------------------------------------------------------------------------------
 # VAE decoder
 # ------------------------------------------------------------------------------------------------
 class VAEDecoderB200:
@@ -495,88 +583,6 @@ class VAEDecoderB200:
             cl = self.P["conv_out_w"].shape[1] // 9
             w27 = self.P["conv_out_w"].view(3, 9, cl).permute(1, 0, 2).reshape(27, cl)
             self.P["conv_out_w27"] = torch.cat([w27, w27.new_zeros(5, cl)], 0).contiguous()
-
-    def _flash_ok(self, sq, skv, C):
-        return self.flash_attention and sq % 128 == 0 and skv % 64 == 0 and C % 128 == 0 and C <= 512
-
-    def _mid_attention(self, ctx, x, a: Packed):
-        """heads=1, d=C (512).  Token counts the wide flash kernel tiles (multiples of 128: every full decode) go
-        through it; otherwise QK^T and PV through the tcgen05 GEMM with fp32 scores per image, or the CUDA-core
-        flash kernel for ragged tiles."""
-        B, H, W, C = x.shape
-        S = H * W
-        hn = groupnorm(ctx, x, a["norm_w"], a["norm_b"], eps=1e-6, silu=False, groups=self.groups)
-        hn2 = hn.view(B * S, C)
-        if ctx.comm is not None:
-            return self._mid_attention_strips(ctx, x, hn2, a)
-        qk = linear(ctx, hn2, a["qk_w"], a["qk_b"], 2 * C)                 # [B*S, 2C]
-        o = ctx.empty(B * S, C)
-        if self._flash_ok(S, S, C):
-            # b_v is folded into the out-proj bias (softmax rows sum to 1), as in the other branches
-            v = linear(ctx, hn2, a["v_w"], None, C)
-            lib.attention_wide(qk, qk[:, C:], v, o, batch=B, sq=S, skv=S, d=C, ldq=2 * C, ldk=2 * C, ldv=C, ldo=C,
-                               scale=1.0 / math.sqrt(C))
-            out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C), norm_rows_per_img=S)
-            return _carry_gn(out, out.view(B, H, W, C))
-        if S % 64 or self.dt != BF16:
-            # fp32 precision mode, and ragged tiles of a tiled decode (token count not a multiple of the 64-deep GEMM K
-            # chunk, e.g. a 29 x 29 corner tile): the CUDA-core flash kernel takes any length.
-            # b_v is folded into the out-proj bias exactly as below (softmax rows sum to 1).
-            v = linear(ctx, hn2, a["v_w"], None, C)
-            lib.attention(qk, qk[:, C:], v, o, batch=B, sq=S, skv=S, heads=1, d=C, dh_stride=C,
-                          ldq=2 * C, ldk=2 * C, ldv=C, ldo=C, scale=1.0 / math.sqrt(C), impl=lib.ATTN_SIMT)
-            out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C))
-            return out.view(B, H, W, C)
-        scores = ctx.empty(S, S, dtype=torch.float32)
-        probs = ctx.empty(S, S)
-        vt = ctx.empty(C, S)
-        for b in range(B):
-            rows = slice(b * S, (b + 1) * S)
-            # V^T[c, s] = sum_k Wv[c,k] X[s,k]  (bias folded into the out-proj bias)
-            lib.igemm(a["v_w"], hn2[rows], vt, nimg=1, h=1, w=C, taps=1, n=S, a0_stride=C, ldo=S)
-            q, k = qk[rows, :C], qk[rows, C:]
-            lib.igemm(q, k, scores, nimg=1, h=1, w=S, taps=1, n=S, c0=C, a0_stride=2 * C,
-                      mode=lib.EPI_F32, alpha=1.0 / math.sqrt(C), ldo=S)
-            lib.softmax_rows(scores, probs)
-            lib.igemm(probs, vt, o[rows], nimg=1, h=1, w=S, taps=1, n=C, a0_stride=S, ldo=C)
-        out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C), norm_rows_per_img=S)
-        return _carry_gn(out, out.view(B, H, W, C))
-
-    def _mid_attention_strips(self, ctx, x, hn2, a: Packed):
-        """Row strips (SURVEY.md §8e, VAE row): the queries of this rank's S tokens attend to the
-        keys / values of all R*S tokens.  ONE exchange: the normalised tokens are all-gathered
-        (rank order = image row order) and every rank projects K and V^T from them itself — the
-        two projections are 2*R*S*C^2 MACs, far cheaper than a second and third gather."""
-        B, H, W, C = x.shape
-        S = H * W
-        comm = ctx.comm
-        hn_all = comm.gather_rows(hn2.view(B, S, C))                        # [B, R*S, C]
-        Sa = hn_all.shape[1]
-        hn_all = hn_all.reshape(B * Sa, C)
-        scale = 1.0 / math.sqrt(C)
-        q = linear(ctx, hn2, a["qk_w"][:C], a["qk_b"][:C], C)               # [B*S, C]
-        k = linear(ctx, hn_all, a["qk_w"][C:], a["qk_b"][C:], C)            # [B*Sa, C]
-        o = ctx.empty(B * S, C)
-        if self._flash_ok(S, Sa, C):
-            v = linear(ctx, hn_all, a["v_w"], None, C)
-            lib.attention_wide(q, k, v, o, batch=B, sq=S, skv=Sa, d=C, ldq=C, ldk=C, ldv=C, ldo=C, scale=scale)
-        elif Sa % 64:                     # ragged key count: the CUDA-core flash kernel takes any length
-            v = linear(ctx, hn_all, a["v_w"], None, C)
-            lib.attention(q, k, v, o, batch=B, sq=S, skv=Sa, heads=1, d=C, dh_stride=C,
-                          ldq=C, ldk=C, ldv=C, ldo=C, scale=scale, impl=lib.ATTN_SIMT)
-        else:
-            scores = ctx.empty(S, Sa, dtype=torch.float32)
-            probs = ctx.empty(S, Sa)
-            vt = ctx.empty(C, Sa)
-            for b in range(B):
-                rows, keys = slice(b * S, (b + 1) * S), slice(b * Sa, (b + 1) * Sa)
-                lib.igemm(a["v_w"], hn_all[keys], vt, nimg=1, h=1, w=C, taps=1, n=Sa, a0_stride=C, ldo=Sa)
-                lib.igemm(q[rows], k[keys], scores, nimg=1, h=1, w=S, taps=1, n=Sa, c0=C, a0_stride=C,
-                          mode=lib.EPI_F32, alpha=scale, ldo=Sa)
-                lib.softmax_rows(scores, probs)
-                lib.igemm(probs, vt, o[rows], nimg=1, h=1, w=S, taps=1, n=C, a0_stride=Sa, ldo=C)
-        out = linear(ctx, o, a["o_w"], a["o_b"], C, residual=x.view(B * S, C))
-        return out.view(B, H, W, C)
 
     @torch.no_grad()
     def decode(self, latents_nhwc: torch.Tensor, out_u8: Optional[torch.Tensor] = None,
@@ -664,7 +670,7 @@ class VAEDecoderB200:
             z = ctx.pad_rows(z)
         h = conv3x3(ctx, z, P["conv_in_w"], P["conv_in_b"], ch[-1], feeds_norm=True)
         h = resnet(ctx, h, P["mid_res"][0], eps=1e-6, groups=g)
-        h = self._mid_attention(ctx, h, P["mid_attn"])
+        h = vae_mid_attention(ctx, h, P["mid_attn"], groups=g, flash=self.flash_attention)
         h = resnet(ctx, h, P["mid_res"][1], eps=1e-6, groups=g)
         for blk in P["up"]:
             for r in blk["resnets"]:
@@ -695,6 +701,116 @@ class VAEDecoderB200:
 
 
 # ------------------------------------------------------------------------------------------------
+# VAE encoder (image-to-image)
+# ------------------------------------------------------------------------------------------------
+class VAEEncoderB200:
+    """`AutoencoderKL.encode` up to the posterior's moments: encoder + quant_conv, untiled or tiled
+    (`enable_tiling()`).  The u8 image goes straight into conv_in's im2col operand (`dl_pack_image_im2col`),
+    conv_in runs as a 1x1 GEMM with K = 64, Downsample2D(padding=0) through `dl_im2col_s2_pad01`, quant_conv
+    in fp32 in the latent-packing kernel.  Moments are fp32 NHWC [B, H/8, W/8, 2 * latent_channels]."""
+
+    def __init__(self, state_dict, cfg, device="cuda:0", precision="bf16"):
+        lib.require_cuda()
+        lib.load()
+        self.device = torch.device(device)
+        self.cfg = cfg
+        self.dt = _dt_of(precision)
+        if cfg.latent_channels != 4:
+            raise RuntimeError(f"VAE encoder: latent_channels={cfg.latent_channels}, only 4 is implemented")
+        from .weights import pack_dtype
+        with pack_dtype(self.dt):
+            self.P = pack_vae_encoder(state_dict, cfg, self.device)
+        self.groups = cfg.norm_num_groups
+        import os
+        self.fuse_gn_stats = os.environ.get("DL_VAE_GN_FUSE", "1") not in ("0", "false")
+        self.flash_attention = os.environ.get("DL_VAE_FLASH", "1") not in ("0", "false") and self.dt == BF16
+
+    @torch.no_grad()
+    def moments(self, img_u8: torch.Tensor, tiling: bool = False, comm=None) -> torch.Tensor:
+        """img_u8: u8 NHWC [B,H,W,3] on the device (H, W multiples of 8).  tiling: images larger than
+        sample_size in either dim are encoded tile by tile and blended (`tiled_encode`)."""
+        if comm is not None:
+            raise RuntimeError("VAE encoder: strip-parallel encode is not implemented")
+        t = self.cfg.sample_size
+        if tiling and (img_u8.shape[1] > t or img_u8.shape[2] > t):
+            return self.tiled_moments(img_u8)
+        return self._encode(img_u8)
+
+    @torch.no_grad()
+    def tiled_moments(self, img_u8: torch.Tensor) -> torch.Tensor:
+        """diffusers `AutoencoderKL.tiled_encode`: tiles of sample_size pixels at stride 0.75 tile, each encoded
+        on its own (own GroupNorm statistics and attention, zero padding at the tile border), moments blended
+        over sample_size/32 latents with the already blended upper / left neighbour, cropped to 0.75 of a tile
+        and written into the result."""
+        B, H, W, _ = img_u8.shape
+        t = self.cfg.sample_size
+        stride = int(t * (1 - 0.25))
+        tl = t // 8
+        blend = int(tl * 0.25)
+        limit = tl - blend
+        out = torch.empty(B, H // 8, W // 8, 2 * self.cfg.latent_channels, device=self.device, dtype=torch.float32)
+        prev_row = []
+        oy = 0
+        for i in range(0, H, stride):
+            row = []
+            ox = 0
+            for jn, j in enumerate(range(0, W, stride)):
+                tile = self._encode(img_u8[:, i:i + t, j:j + t])           # a view: read in place
+                if i > 0:
+                    up = prev_row[jn]
+                    lib.tile_blend(up, tile, min(up.shape[1], tile.shape[1], blend), vertical=True)
+                if jn > 0:
+                    left = row[jn - 1]
+                    lib.tile_blend(left, tile, min(left.shape[2], tile.shape[2], blend), vertical=False)
+                row.append(tile)
+                ch, cw = min(limit, tile.shape[1]), min(limit, tile.shape[2])
+                out[:, oy:oy + ch, ox:ox + cw].copy_(tile[:, :ch, :cw])
+                ox += cw
+            prev_row = row
+            oy += min(limit, row[0].shape[1])
+        return out
+
+    def _downsample(self, ctx, x, p: Packed):
+        """Downsample2D(padding=0): F.pad(x, (0,1,0,1)) + conv3x3 stride 2, as im2col + GEMM."""
+        B, H, W, C = x.shape
+        cols = ctx.empty(B * (H // 2) * (W // 2), 9 * C)
+        lib.im2col_s2_pad01(x, cols, nimg=B, h=H, w=W)
+        out = linear(ctx, cols, p["w"], p["b"], C, norm_rows_per_img=(H // 2) * (W // 2))
+        return _carry_gn(out, out.view(B, H // 2, W // 2, C))
+
+    @torch.no_grad()
+    def _encode(self, img_u8: torch.Tensor) -> torch.Tensor:
+        """One untiled encode (img_u8 may be a window of a larger canvas)."""
+        P = self.P
+        B, H, W, _ = img_u8.shape
+        if H % 8 or W % 8:
+            raise RuntimeError(f"VAE encoder: image {W}x{H} is not a multiple of 8")
+        g = self.groups
+        ctx = _Ctx(self.device, B, gn_fuse=g if self.fuse_gn_stats else 0, dt=self.dt)
+        ch = self.cfg.block_out_channels
+        cols = ctx.empty(B * H * W, 64)
+        lib.pack_image_im2col(img_u8, cols)
+        h = linear(ctx, cols, P["conv_in_w"], P["conv_in_b"], ch[0], norm_rows_per_img=H * W)
+        h = _carry_gn(h, h.view(B, H, W, ch[0]))
+        for blk in P["down"]:
+            for r in blk["resnets"]:
+                h = resnet(ctx, h, r, eps=1e-6, groups=g)
+            if blk["down"] is not None:
+                h = self._downsample(ctx, h, blk["down"])
+        h = resnet(ctx, h, P["mid_res"][0], eps=1e-6, groups=g)
+        h = vae_mid_attention(ctx, h, P["mid_attn"], groups=g, flash=self.flash_attention)
+        h = resnet(ctx, h, P["mid_res"][1], eps=1e-6, groups=g)
+        hn = groupnorm(ctx, h, P["norm_out_w"], P["norm_out_b"], eps=1e-6, silu=True, groups=g)
+        Bo, Ho, Wo, _ = h.shape
+        m = P["q_w"].shape[0]
+        raw = torch.empty(Bo, Ho, Wo, m, device=self.device, dtype=torch.float32)
+        conv3x3(ctx, hn, P["conv_out_w"], P["conv_out_b"], m, mode=lib.EPI_F32, out=raw, ldo=m)
+        mom = torch.empty_like(raw)
+        lib.pack_latent(raw, mom, cin=m, mat=P["q_w"], vec=P["q_b"])         # quant_conv, fp32
+        return mom
+
+
+# ------------------------------------------------------------------------------------------------
 # pipeline: denoise loop + decode
 # ------------------------------------------------------------------------------------------------
 # Warm-up + capture of ALL pipelines of the process are serialised: the WorkerPool runs one worker thread
@@ -714,9 +830,11 @@ def _pinned(x: torch.Tensor) -> torch.Tensor:
 
 
 class _StaticGraph:
-    """One captured CUDA graph of the whole hot path for a fixed (B, h, w, steps[, gs])."""
+    """One captured CUDA graph of the whole hot path for a fixed (B, h, w, steps[, gs][, strength]).
+    strength set: image-to-image; the init images and the posterior draw are static inputs too, and `lat`
+    holds the add_noise draw."""
 
-    def __init__(self, pipe: "LCMPipelineB200", B, h, w, steps, cfg_scale=None, decode=True):
+    def __init__(self, pipe: "LCMPipelineB200", B, h, w, steps, cfg_scale=None, decode=True, strength=None):
         dev = pipe.device
         ucfg = pipe.unet.cfg
         D = ucfg.cross_attention_dim
@@ -732,8 +850,13 @@ class _StaticGraph:
         self.lat = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
         self.noise = torch.zeros(max(steps - 1, 1), B, 4, h, w, device=dev, dtype=torch.float32)
         self.steps = steps
+        self.init_u8 = self.eps_s = None
+        if strength is not None:
+            self.init_u8 = torch.zeros(B, 8 * h, 8 * w, 3, device=dev, dtype=torch.uint8)
+            self.eps_s = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
         args = (self.pe, self.w_emb, self.lat, self.noise, steps)
-        kw = dict(add=self.add, cfg_scale=cfg_scale, decode=decode)
+        kw = dict(add=self.add, cfg_scale=cfg_scale, decode=decode, init_u8=self.init_u8, eps_s=self.eps_s,
+                  strength=strength)
         with CAPTURE_LOCK:
             # warm-up on a side stream (lazy per-device init: smem attributes, module load)
             s = torch.cuda.Stream(device=dev)
@@ -771,6 +894,9 @@ class LCMPipelineB200:
         self.dt = _dt_of(precision)
         self.unet = UNetB200(unet_sd, unet_cfg, device, precision)
         self.vae = VAEDecoderB200(vae_sd, vae_cfg, device, precision)
+        # image-to-image needs the encoder half of the VAE; a VAE shipped without it still serves text-to-image
+        self.vae_encoder = (VAEEncoderB200(vae_sd, vae_cfg, device, precision) if has_vae_encoder(vae_sd)
+                            else None)
         self.vae_tiling = vae_tiling
         self._graphs = {}
 
@@ -798,19 +924,48 @@ class LCMPipelineB200:
 
     @torch.no_grad()
     def run_static(self, pe_bf16, w_emb, lat_nchw, noise_nchw, steps: int, record: dict = None,
-                   add=None, cfg_scale: Optional[float] = None, teacher=None, decode: bool = True):
+                   add=None, cfg_scale: Optional[float] = None, teacher=None, decode: bool = True,
+                   init_u8=None, eps_s=None, strength: Optional[float] = None):
         """Everything on device, no host sync, graph-capturable.  Returns (u8 images, latents).
-        pe_bf16 / add carry 2B rows ([uncond, cond]) when cfg_scale is set."""
+        pe_bf16 / add carry 2B rows ([uncond, cond]) when cfg_scale is set.
+        init_u8 (image-to-image): u8 NHWC init images; the pass becomes encode -> posterior sample with eps_s ->
+        add_noise at the first timestep of the strength schedule with lat_nchw as the noise -> denoise -> decode."""
         B = lat_nchw.shape[0]
         Bu = 2 * B if cfg_scale is not None else B
-        sched = LCMSchedule(steps)
+        sched = LCMSchedule(steps) if init_u8 is None else LCMSchedule(steps, strength)
         kvs = self.unet.encode_context(pe_bf16)
         aug = self.unet.addition_embedding(*add) if add is not None else None
         tembs = self.unet.time_embeddings(sched.timesteps, Bu, w_emb, aug)
-        lat = self.denoise(lat_nchw, noise_nchw, sched, kvs, tembs, record, cfg_scale=cfg_scale, teacher=teacher)
+        start = None
+        if init_u8 is not None:
+            start = self.init_latents(init_u8, eps_s, lat_nchw, sched, record)
+        lat = self.denoise(lat_nchw, noise_nchw, sched, kvs, tembs, record, cfg_scale=cfg_scale, teacher=teacher,
+                           start_nhwc=start)
         if not decode:                   # latent-only callers (candidate scoring): no VAE pass at all
             return None, lat
         return self.vae.decode(lat, tiling=self.vae_tiling), lat
+
+    def init_latents(self, init_u8, eps_s, eps_n, sched: LCMSchedule, record: dict = None) -> torch.Tensor:
+        """`LatentConsistencyModelImg2ImgPipeline.prepare_latents`: moments of the init images, posterior sample
+        mean + std * eps_s, times scaling_factor, then `add_noise` with eps_n at t0 = sched.timesteps[0], in one
+        kernel.  -> fp32 NHWC latents [B, h, w, 4]."""
+        enc = self.require_encoder()
+        mom = enc.moments(init_u8, tiling=self.vae_tiling)
+        B, h, w, _ = mom.shape
+        x = torch.empty(B, h, w, 4, device=self.device, dtype=torch.float32)
+        sa, sb = sched.add_noise_coeffs()
+        lib.vae_sample_latents(mom, eps_s, eps_n, x, scaling_factor=self.vae.cfg.scaling_factor, sqrt_alpha=sa,
+                               sqrt_one_minus_alpha=sb)
+        if record is not None:
+            record["moments"] = mom.permute(0, 3, 1, 2).clone()
+            record["init_latents"] = x.permute(0, 3, 1, 2).clone()
+        return x
+
+    def require_encoder(self) -> VAEEncoderB200:
+        if self.vae_encoder is None:
+            raise RuntimeError("image-to-image needs the VAE encoder, and this model's VAE has no encoder weights "
+                               "(encoder.* / quant_conv.*)")
+        return self.vae_encoder
 
     max_graphs = 12       # captured geometries kept per pipeline
     # batch sizes a CUDA graph is captured for: a request batch is padded up to the next one (micro-batching
@@ -822,27 +977,33 @@ class LCMPipelineB200:
             self._pool = torch.cuda.graph_pool_handle()
         return self._pool
 
-    def graph_for(self, B, h, w, steps, cfg_scale=None, decode=True) -> _StaticGraph:
+    def graph_for(self, B, h, w, steps, cfg_scale=None, decode=True, strength=None) -> _StaticGraph:
         key = (B, h, w, steps, cfg_scale, decode)
+        if strength is not None:                                 # image-to-image: its own graph per strength
+            key += ("img2img", strength)
         g = self._graphs.pop(key, None)
         if g is None:
             while len(self._graphs) >= self.max_graphs:          # least recently used goes first
                 self._graphs.pop(next(iter(self._graphs)))
             with torch.cuda.device(self.device):
-                g = _StaticGraph(self, B, h, w, steps, cfg_scale, decode)
+                g = _StaticGraph(self, B, h, w, steps, cfg_scale, decode, strength)
         self._graphs[key] = g                                     # dict order = recency
         return g
 
     @torch.no_grad()
     def denoise(self, latents_nchw, step_noise_nchw, sched, kvs, tembs, record: dict = None,
-                cfg_scale: Optional[float] = None, teacher=None):
+                cfg_scale: Optional[float] = None, teacher=None, start_nhwc=None):
         """latents fp32 NCHW [B,4,h,w]; step_noise [steps-1,B,4,h,w].  Returns final latents NHWC.
+        start_nhwc (image-to-image): the initial latents, already NHWC; latents_nchw then only gives the shape.
         teacher (parity tests): fp32 NCHW [steps,B,4,h,w] — the latents fed to the UNet at step i
         come from this tensor (an oracle trajectory) instead of from the previous step, so every
         step's noise_pred is compared on identical inputs (teacher forcing)."""
         B, C, H, W = latents_nchw.shape
-        x = torch.empty(B, H, W, C, device=self.device, dtype=torch.float32)
-        lib.nchw_to_nhwc_f32(latents_nchw, x)
+        if start_nhwc is not None:
+            x = start_nhwc
+        else:
+            x = torch.empty(B, H, W, C, device=self.device, dtype=torch.float32)
+            lib.nchw_to_nhwc_f32(latents_nchw, x)
         n = sched.num_inference_steps
         noise = None
         if n > 1:
@@ -903,12 +1064,31 @@ class LCMPipelineB200:
                  guidance_scale=1.0, record: dict = None, return_latents: bool = False,
                  use_graph: bool = False, pooled_embeds=None, time_ids=None,
                  negative_prompt_embeds=None, negative_pooled_embeds=None, teacher_latents=None,
-                 decode: bool = True):
+                 decode: bool = True, init_images=None, strength: Optional[float] = None, posterior_noise=None):
         """Public entry: host or device tensors in -> u8 images [B,H,W,3] on device (and the
         final latents NHWC fp32 if asked).  With use_graph the whole pass is one CUDA-graph
-        replay; the returned tensors are the graph's static outputs (consume before next call)."""
+        replay; the returned tensors are the graph's static outputs (consume before next call).
+
+        Image-to-image (`LatentConsistencyModelImg2ImgPipeline`): init_images u8 [B,H,W,3] (H = 8h, W = 8w),
+        strength in (0, 1] (default 0.8), posterior_noise fp32 [B,4,h,w] (the posterior sample's draw);
+        latents_nchw is then the add_noise draw.  Needs an LCM UNet (time_cond_proj_dim) and VAE encoder
+        weights."""
         B, _, h, w = latents_nchw.shape
         steps = int(num_inference_steps)
+        if init_images is not None:
+            strength = 0.8 if strength is None else float(strength)
+            if not self.unet.cfg.time_cond_proj_dim:
+                raise RuntimeError("image-to-image is implemented for LCM UNets (time_cond_proj_dim) only: the LCM "
+                                   "img2img pipeline has no classifier-free guidance branch")
+            self.require_encoder()
+            if tuple(init_images.shape) != (B, 8 * h, 8 * w, 3) or init_images.dtype != torch.uint8:
+                raise RuntimeError(f"init_images: u8 [{B}, {8 * h}, {8 * w}, 3] expected, got "
+                                   f"{init_images.dtype} {list(init_images.shape)}")
+            if posterior_noise is None or tuple(posterior_noise.shape) != (B, 4, h, w):
+                raise RuntimeError(f"image-to-image needs posterior_noise [{B}, 4, {h}, {w}]")
+            LCMSchedule(steps, strength)                  # ValueError for a strength the schedule cannot serve
+        else:
+            strength = None
         if use_graph and record is None and teacher_latents is None:
             Bp = next((b for b in self.batch_buckets if b >= B), B)
             if Bp != B:
@@ -926,7 +1106,9 @@ class LCMPipelineB200:
                                     pad(gs) if gs.numel() > 1 else guidance_scale, return_latents=True, use_graph=True,
                                     pooled_embeds=pad(pooled_embeds), time_ids=pad(time_ids),
                                     negative_prompt_embeds=pad(negative_prompt_embeds),
-                                    negative_pooled_embeds=pad(negative_pooled_embeds), decode=decode)
+                                    negative_pooled_embeds=pad(negative_pooled_embeds), decode=decode,
+                                    init_images=pad(init_images), strength=strength,
+                                    posterior_noise=pad(posterior_noise))
                 img, lat = out
                 img = img[:B] if img is not None else None
                 return (img, lat[:B]) if return_latents else img
@@ -936,7 +1118,7 @@ class LCMPipelineB200:
                                          negative_pooled_embeds, cfg_scale, 8 * h, 8 * w)
         with torch.cuda.device(self.device):
             if use_graph and record is None and teacher_latents is None:
-                g = self.graph_for(B, h, w, steps, cfg_scale, decode)
+                g = self.graph_for(B, h, w, steps, cfg_scale, decode, strength)
                 # host inputs go through pinned staging: a copy from PAGEABLE host memory first waits for the stream to
                 # drain (CUDA's documented behaviour), i.e. for the previous batch — the thread could then not enqueue
                 # this batch behind it
@@ -949,6 +1131,9 @@ class LCMPipelineB200:
                 g.lat.copy_(_pinned(latents_nchw), non_blocking=True)
                 if steps > 1:
                     g.noise.copy_(_pinned(step_noise_nchw), non_blocking=True)
+                if strength is not None:
+                    g.init_u8.copy_(_pinned(init_images), non_blocking=True)
+                    g.eps_s.copy_(_pinned(posterior_noise), non_blocking=True)
                 g.graph.replay()
                 img, lat = g.img, g.final
             else:
@@ -959,6 +1144,11 @@ class LCMPipelineB200:
                 lat0 = latents_nchw.to(self.device, torch.float32).contiguous()
                 nz = (step_noise_nchw.to(self.device, torch.float32).contiguous()
                       if steps > 1 else None)
+                init = eps = None
+                if strength is not None:
+                    init = init_images.to(self.device).contiguous()
+                    eps = posterior_noise.to(self.device, torch.float32).contiguous()
                 img, lat = self.run_static(pe, we, lat0, nz, steps, record, add=add, cfg_scale=cfg_scale,
-                                           teacher=teacher_latents, decode=decode)
+                                           teacher=teacher_latents, decode=decode, init_u8=init, eps_s=eps,
+                                           strength=strength)
         return (img, lat) if return_latents else img

@@ -29,6 +29,8 @@ EXPORTS = [
     "dl_peer_allgather", "dl_igemm_f32", "dl_groupnorm_f32", "dl_layernorm_f32", "dl_attention_f32", "dl_pack_latent_f32",
     "dl_im2col_s2_f32", "dl_softmax_rows_f32", "dl_small_linear_f32",
     "dl_png_stored_size", "dl_png_stored_workspace_bytes", "dl_png_stored", "dl_conv_tapsum",
+    "dl_im2col_s2_pad01", "dl_im2col_s2_pad01_f32", "dl_pack_image_im2col", "dl_pack_image_im2col_f32",
+    "dl_vae_sample_latents",
 ]
 
 
@@ -155,6 +157,16 @@ def load() -> C.CDLL:
                                             C.c_void_p, C.c_void_p]
             lib.dl_conv_tapsum.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
                                            C.c_void_p, C.c_int, C.c_void_p]
+            lib.dl_im2col_s2_pad01.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                               C.c_void_p]
+            lib.dl_im2col_s2_pad01_f32.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_int, C.c_void_p,
+                                                   C.c_void_p]
+            for f in (lib.dl_pack_image_im2col, lib.dl_pack_image_im2col_f32):
+                f.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_longlong, C.c_void_p,
+                              C.c_void_p]
+            lib.dl_vae_sample_latents.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
+                                                  C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p,
+                                                  C.c_void_p]
             lib.dl_png_stored_size.restype = C.c_longlong
             lib.dl_png_stored_size.argtypes = [C.c_int, C.c_int]
             lib.dl_png_stored_workspace_bytes.restype = C.c_longlong
@@ -505,6 +517,42 @@ def im2col_s2_halo(x, cols, *, nimg, in_rows, in_row0, h, w):
     with _timed("im2col_s2", 0.0, 2.0 * x.numel() + 2.0 * cols.numel()):
         _check(load().dl_im2col_s2_halo(x.data_ptr(), nimg, in_rows, in_row0, h, w, x.shape[-1],
                                         cols.data_ptr(), _stream()), "im2col_s2_halo")
+    _count()
+
+
+def im2col_s2_pad01(x, cols, *, nimg, h, w):
+    """Downsample2D(padding=0) of the VAE encoder: bottom / right zero pad, then conv3x3 stride 2."""
+    if x.dtype == torch.float32:
+        _check(load().dl_im2col_s2_pad01_f32(x.data_ptr(), nimg, h, w, x.shape[-1], cols.data_ptr(), _stream()),
+               "im2col_s2_pad01_f32")
+        _count()
+        return
+    with _timed("im2col_s2_pad01", 0.0, 2.0 * x.numel() + 2.0 * cols.numel()):
+        _check(load().dl_im2col_s2_pad01(x.data_ptr(), nimg, h, w, x.shape[-1], cols.data_ptr(), _stream()),
+               "im2col_s2_pad01")
+    _count()
+
+
+def pack_image_im2col(img, out):
+    """img: u8 [n,h,w,3] (a view with unit channel and 3-byte pixel stride: a tile window of a canvas is fine);
+    out: bf16 or fp32 [n*h*w, 64] conv_in im2col operand (K = tap*3 + c, zero padded)."""
+    n, h, w, c = img.shape
+    if c != 3 or img.dtype != torch.uint8 or img.stride(3) != 1 or img.stride(2) != 3:
+        raise RuntimeError("pack_image_im2col: u8 [n,h,w,3] with packed RGB pixels expected")
+    fn = load().dl_pack_image_im2col_f32 if out.dtype == torch.float32 else load().dl_pack_image_im2col
+    with _timed("pack_image_im2col", 0.0, float(img.numel()) + out.element_size() * out.numel()):
+        _check(fn(img.data_ptr(), n, h, w, img.stride(1), img.stride(0), out.data_ptr(), _stream()),
+               "pack_image_im2col")
+    _count()
+
+
+def vae_sample_latents(moments, eps_s, eps_n, out, *, scaling_factor, sqrt_alpha, sqrt_one_minus_alpha,
+                       mean_out=None):
+    """moments fp32 NHWC [n,h,w,8]; eps_s / eps_n fp32 NCHW [n,4,h,w]; out (mean_out) fp32 NHWC [n,h,w,4]."""
+    n, h, w, _ = moments.shape
+    _check(load().dl_vae_sample_latents(moments.data_ptr(), eps_s.data_ptr(), eps_n.data_ptr(), n, h, w,
+                                        float(scaling_factor), float(sqrt_alpha), float(sqrt_one_minus_alpha),
+                                        out.data_ptr(), _ptr(mean_out), _stream()), "vae_sample_latents")
     _count()
 
 

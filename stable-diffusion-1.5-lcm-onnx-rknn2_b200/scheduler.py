@@ -32,12 +32,19 @@ def alphas_cumprod() -> torch.Tensor:
     return torch.cumprod(1.0 - betas, dim=0)
 
 
-def lcm_timesteps(num_inference_steps: int) -> List[int]:
+def lcm_timesteps(num_inference_steps: int, strength: float = 1.0) -> List[int]:
+    """`LCMScheduler.set_timesteps(n, strength=strength)`: image-to-image (strength < 1) draws the n steps from
+    the first int(50 * strength) entries of the original 50-step schedule, counted from t = 19 upwards."""
     if not 1 <= num_inference_steps <= ORIGINAL_INFERENCE_STEPS:
         raise ValueError(f"num_inference_steps must be in [1, {ORIGINAL_INFERENCE_STEPS}], "
                          f"got {num_inference_steps}")
+    if not 0.0 < strength <= 1.0:
+        raise ValueError(f"strength must be in (0, 1], got {strength}")
     k = NUM_TRAIN_TIMESTEPS // ORIGINAL_INFERENCE_STEPS
-    origin = (np.arange(1, ORIGINAL_INFERENCE_STEPS + 1) * k - 1)[::-1]
+    origin = (np.arange(1, int(ORIGINAL_INFERENCE_STEPS * strength) + 1) * k - 1)[::-1]
+    if len(origin) // num_inference_steps < 1:
+        raise ValueError(f"strength {strength} leaves {len(origin)} of the {ORIGINAL_INFERENCE_STEPS} original "
+                         f"timesteps: fewer than num_inference_steps={num_inference_steps}")
     idx = np.floor(np.linspace(0, len(origin), num=num_inference_steps, endpoint=False)).astype(np.int64)
     return [int(t) for t in origin[idx]]
 
@@ -45,9 +52,10 @@ def lcm_timesteps(num_inference_steps: int) -> List[int]:
 class LCMSchedule:
     """Timesteps + per-step coefficient tuples for `lib.lcm_step`."""
 
-    def __init__(self, num_inference_steps: int):
+    def __init__(self, num_inference_steps: int, strength: float = 1.0):
         self.num_inference_steps = num_inference_steps
-        self.timesteps = lcm_timesteps(num_inference_steps)
+        self.strength = strength
+        self.timesteps = lcm_timesteps(num_inference_steps, strength)
         ac = alphas_cumprod()
         self._coeffs: List[Tuple[float, ...]] = []
         for i, t in enumerate(self.timesteps):
@@ -58,6 +66,11 @@ class LCMSchedule:
             c_out = s / (s ** 2 + SIGMA_DATA ** 2) ** 0.5
             self._coeffs.append((a_t.sqrt().item(), (1 - a_t).sqrt().item(), c_skip.item(),
                                  c_out.item(), a_prev.sqrt().item(), (1 - a_prev).sqrt().item()))
+
+    def add_noise_coeffs(self) -> Tuple[float, float]:
+        """`LCMScheduler.add_noise` at t0 = timesteps[0]: fp32 (sqrt(ac[t0]), sqrt(1 - ac[t0])) as `** 0.5`."""
+        a = alphas_cumprod()[self.timesteps[0]]
+        return (a ** 0.5).item(), ((1 - a) ** 0.5).item()
 
     def coeffs(self, i: int) -> Tuple[float, ...]:
         return self._coeffs[i]

@@ -5,8 +5,9 @@ The reference loads such files with `StableDiffusionPipeline.from_single_file` /
 its `modes.yaml.example` is one).  diffusers is not a dependency here, so the key renaming it performs
 (`convert_ldm_unet_checkpoint` / `convert_ldm_vae_checkpoint` / the text-encoder converters) is restated as
 tables generated from the architecture: the b200 engine then packs the result exactly like a diffusers
-directory.  Covered: SD1.x (UNet + VAE decoder + CLIP-L text tower) and SDXL-base (UNet + VAE decoder +
-CLIP-L + OpenCLIP-bigG text towers).  Only the decoder half of the VAE is converted (the hot path never encodes).
+directory.  Covered: SD1.x (UNet + VAE + CLIP-L text tower) and SDXL-base (UNet + VAE + CLIP-L + OpenCLIP-bigG
+text towers).  The VAE's decoder and encoder halves are converted separately (`convert_vae_decoder`,
+`convert_vae_encoder`); the encoder serves image-to-image only.
 """
 from __future__ import annotations
 
@@ -142,6 +143,41 @@ def convert_vae_decoder(sd: Dict[str, torch.Tensor], cfg: dict) -> Dict[str, tor
     return out
 
 
+def vae_encoder_module_map(cfg: dict) -> Tuple[Dict[str, str], set]:
+    """Encoder levels keep their order in LDM (unlike the decoder's up levels)."""
+    n, lpb = len(cfg["block_out_channels"]), cfg["layers_per_block"]
+    m = {"quant_conv": "quant_conv", "encoder.conv_in": "encoder.conv_in",
+         "encoder.norm_out": "encoder.conv_norm_out", "encoder.conv_out": "encoder.conv_out",
+         "encoder.mid.block_1": "encoder.mid_block.resnets.0", "encoder.mid.block_2": "encoder.mid_block.resnets.1",
+         "encoder.mid.attn_1": "encoder.mid_block.attentions.0"}
+    for i in range(n):
+        for j in range(lpb):
+            m[f"encoder.down.{i}.block.{j}"] = f"encoder.down_blocks.{i}.resnets.{j}"
+        if i != n - 1:
+            m[f"encoder.down.{i}.downsample.conv"] = f"encoder.down_blocks.{i}.downsamplers.0.conv"
+    return m, {"encoder.mid.attn_1"}
+
+
+def convert_vae_encoder(sd: Dict[str, torch.Tensor], cfg: dict) -> Dict[str, torch.Tensor]:
+    """Encoder + quant_conv keys of a single-file checkpoint (empty when it has none)."""
+    modules, attn = vae_encoder_module_map(cfg)
+    out = {}
+    for k, v in sd.items():
+        if not k.startswith(VAE_PREFIX):
+            continue
+        k2 = k[len(VAE_PREFIX):]
+        if not (k2.startswith("encoder.") or k2.startswith("quant_conv.")):
+            continue
+        src = max((s for s in modules if k2 == s or k2.startswith(s + ".")), key=len, default=None)
+        if src is None:
+            raise RuntimeError(f"single-file VAE: no diffusers name for '{k}'")
+        new = _rename(k2, modules, _VAE_ATTN if src in attn else _VAE_RES)
+        if src in attn and v.dim() == 4:                 # 1x1 convs -> Linear weights
+            v = v.reshape(v.shape[0], v.shape[1])
+        out[new] = v
+    return out
+
+
 def convert_clip_hf(sd, prefix: str) -> Dict[str, torch.Tensor]:
     """CLIP-L ships in transformers' own naming under `prefix` (…transformer.)."""
     return {k[len(prefix):]: v for k, v in sd.items()
@@ -212,7 +248,8 @@ def load_single_file(path: str) -> dict:
     probe = next(k for k in sorted(sd) if k.startswith(UNET_PREFIX) and k.endswith("attn2.to_k.weight"))
     ucfg["cross_attention_dim"] = sd[probe].shape[1]
     vcfg = dict(SDXL_VAE if sdxl else SD_VAE)
-    out = {"unet": (ucfg, convert_unet(sd, ucfg)), "vae": (vcfg, convert_vae_decoder(sd, vcfg)),
+    out = {"unet": (ucfg, convert_unet(sd, ucfg)),
+           "vae": (vcfg, {**convert_vae_decoder(sd, vcfg), **convert_vae_encoder(sd, vcfg)}),
            "text_encoder": None, "text_encoder_2": None,
            "model_index": {"_class_name": "StableDiffusionXLPipeline" if sdxl else "StableDiffusionPipeline",
                            "force_zeros_for_empty_prompt": True}}

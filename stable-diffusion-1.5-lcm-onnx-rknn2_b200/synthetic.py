@@ -162,6 +162,34 @@ def vae_decoder_shapes(cfg) -> Dict[str, Tuple[int, ...]]:
     return s
 
 
+def vae_encoder_shapes(cfg) -> Dict[str, Tuple[int, ...]]:
+    """AutoencoderKL encoder (double_z) + quant_conv, diffusers names."""
+    s: Dict[str, Tuple[int, ...]] = {}
+    ch = cfg.block_out_channels
+    m = 2 * cfg.latent_channels
+    d = "encoder."
+    s[d + "conv_in.weight"] = (ch[0], 3, 3, 3); s[d + "conv_in.bias"] = (ch[0],)
+    prev = ch[0]
+    for i, c in enumerate(ch):
+        for j in range(cfg.layers_per_block):
+            _resnet(s, d + f"down_blocks.{i}.resnets.{j}.", prev if j == 0 else c, c, 0)
+        if i != len(ch) - 1:
+            s[d + f"down_blocks.{i}.downsamplers.0.conv.weight"] = (c, c, 3, 3)
+            s[d + f"down_blocks.{i}.downsamplers.0.conv.bias"] = (c,)
+        prev = c
+    top = ch[-1]
+    _resnet(s, d + "mid_block.resnets.0.", top, top, 0)
+    a = d + "mid_block.attentions.0."
+    s[a + "group_norm.weight"] = (top,); s[a + "group_norm.bias"] = (top,)
+    for n in ("to_q", "to_k", "to_v", "to_out.0"):
+        s[a + n + ".weight"] = (top, top); s[a + n + ".bias"] = (top,)
+    _resnet(s, d + "mid_block.resnets.1.", top, top, 0)
+    s[d + "conv_norm_out.weight"] = (top,); s[d + "conv_norm_out.bias"] = (top,)
+    s[d + "conv_out.weight"] = (m, top, 3, 3); s[d + "conv_out.bias"] = (m,)
+    s["quant_conv.weight"] = (m, m, 1, 1); s["quant_conv.bias"] = (m,)
+    return s
+
+
 def random_state_dict(shapes: Dict[str, Tuple[int, ...]], seed: int = 0,
                       dtype=torch.float32) -> Dict[str, torch.Tensor]:
     g = torch.Generator().manual_seed(seed)
@@ -242,9 +270,12 @@ def write_text_encoder(model_dir: str, hidden: int = 768, layers: int = 12, head
     save_file(sd, os.path.join(te, "model.safetensors"))
 
 
-def write_model_dir(path: str, unet_cfg=None, vae_cfg=None, seed: int = 0, dtype=torch.float16):
+def write_model_dir(path: str, unet_cfg=None, vae_cfg=None, seed: int = 0, dtype=torch.float16,
+                    vae_encoder: bool = False):
     """A diffusers-layout directory (model_index.json, unet/, vae/) with random-init weights —
-    what `MODEL_ROOT/MODEL` points at for offline tests of the b200 worker."""
+    what `MODEL_ROOT/MODEL` points at for offline tests of the b200 worker.  vae_encoder: also write the
+    VAE's encoder + quant_conv (image-to-image), from a seed of their own: the decoder weights are the same
+    either way."""
     from safetensors.torch import save_file
     unet_cfg = unet_cfg or sd15_lcm_unet_cfg()
     vae_cfg = vae_cfg or sd_vae_cfg()
@@ -282,6 +313,8 @@ def write_model_dir(path: str, unet_cfg=None, vae_cfg=None, seed: int = 0, dtype
                    "scaling_factor": vae_cfg.scaling_factor, "sample_size": vae_cfg.sample_size}, f)
     save_file(random_state_dict(unet_shapes(unet_cfg), seed, dtype),
               os.path.join(path, "unet", "diffusion_pytorch_model.safetensors"))
-    save_file(random_state_dict(vae_decoder_shapes(vae_cfg), seed + 1, dtype),
-              os.path.join(path, "vae", "diffusion_pytorch_model.safetensors"))
+    vae_sd = random_state_dict(vae_decoder_shapes(vae_cfg), seed + 1, dtype)
+    if vae_encoder:
+        vae_sd.update(random_state_dict(vae_encoder_shapes(vae_cfg), seed + 3, dtype))
+    save_file(vae_sd, os.path.join(path, "vae", "diffusion_pytorch_model.safetensors"))
     return path

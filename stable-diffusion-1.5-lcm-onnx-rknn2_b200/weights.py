@@ -273,17 +273,8 @@ def pack_unet(sd: Dict[str, torch.Tensor], cfg, device) -> Packed:
     return P
 
 
-def pack_vae_decoder(sd: Dict[str, torch.Tensor], cfg, device) -> Packed:
-    P = Packed()
-    P["cfg"] = cfg
-    # post_quant_conv (1x1, 4->4) is applied in fp32 by the latent-packing kernel
-    P["pq_w"] = _f32(sd["post_quant_conv.weight"].reshape(cfg.latent_channels, cfg.latent_channels), device)
-    P["pq_b"] = _f32(sd["post_quant_conv.bias"], device)
-    d = "decoder."
-    P["conv_in_w"] = pack_conv3x3(sd[d + "conv_in.weight"], device, pad_in_to=64)
-    P["conv_in_b"] = _f32(sd[d + "conv_in.bias"], device)
-    P["mid_res"] = [pack_resnet(sd, d + f"mid_block.resnets.{i}.", device) for i in range(2)]
-    a = d + "mid_block.attentions.0."
+def pack_vae_attention(sd: Dict[str, torch.Tensor], a: str, device) -> Packed:
+    """The one-head mid-block attention of the AutoencoderKL encoder and decoder (prefix `a`)."""
     att = Packed()
     att["norm_w"], att["norm_b"] = _f32(sd[a + "group_norm.weight"], device), _f32(sd[a + "group_norm.bias"], device)
     wq, wk, wv, wo = (sd[a + f"{n}.weight"].float() for n in ("to_q", "to_k", "to_v", "to_out.0"))
@@ -295,7 +286,54 @@ def pack_vae_decoder(sd: Dict[str, torch.Tensor], cfg, device) -> Packed:
     # softmax rows sum to 1  =>  P (V + 1 b_v^T) = P V + b_v^T : fold b_v into the out-proj bias
     att["o_b"] = _f32(bo + wo @ bv, device)
     att["c"] = wq.shape[0]
-    P["mid_attn"] = att
+    return att
+
+
+def has_vae_encoder(sd: Dict[str, torch.Tensor]) -> bool:
+    return "encoder.conv_in.weight" in sd and "quant_conv.weight" in sd
+
+
+def pack_vae_encoder(sd: Dict[str, torch.Tensor], cfg, device) -> Packed:
+    """AutoencoderKL encoder + quant_conv.  conv_in (3 -> C, 3x3) runs as a 1x1 GEMM over the image im2col
+    (`dl_pack_image_im2col`): weight [C, 27] with K = (ky*3 + kx)*3 + c, zero-padded to 64.  quant_conv
+    (1x1, 2L -> 2L) is applied in fp32 by the latent-packing kernel, like post_quant_conv."""
+    P = Packed()
+    P["cfg"] = cfg
+    d = "encoder."
+    w = sd[d + "conv_in.weight"].float()
+    P["conv_in_w"] = _bf(torch.nn.functional.pad(w.permute(0, 2, 3, 1).reshape(w.shape[0], -1), (0, 64 - 27)), device)
+    P["conv_in_b"] = _f32(sd[d + "conv_in.bias"], device)
+    P["down"] = []
+    n = len(cfg.block_out_channels)
+    for i in range(n):
+        blk = Packed(resnets=[pack_resnet(sd, d + f"down_blocks.{i}.resnets.{j}.", device)
+                              for j in range(cfg.layers_per_block)], down=None)
+        k = d + f"down_blocks.{i}.downsamplers.0.conv."
+        if k + "weight" in sd:
+            blk["down"] = Packed(w=pack_conv3x3(sd[k + "weight"], device), b=_f32(sd[k + "bias"], device))
+        P["down"].append(blk)
+    P["mid_res"] = [pack_resnet(sd, d + f"mid_block.resnets.{i}.", device) for i in range(2)]
+    P["mid_attn"] = pack_vae_attention(sd, d + "mid_block.attentions.0.", device)
+    P["norm_out_w"], P["norm_out_b"] = _f32(sd[d + "conv_norm_out.weight"], device), _f32(sd[d + "conv_norm_out.bias"], device)
+    P["conv_out_w"] = pack_conv3x3(sd[d + "conv_out.weight"], device)
+    P["conv_out_b"] = _f32(sd[d + "conv_out.bias"], device)
+    m = sd["quant_conv.weight"].shape[0]
+    P["q_w"] = _f32(sd["quant_conv.weight"].reshape(m, m), device)
+    P["q_b"] = _f32(sd["quant_conv.bias"], device)
+    return P
+
+
+def pack_vae_decoder(sd: Dict[str, torch.Tensor], cfg, device) -> Packed:
+    P = Packed()
+    P["cfg"] = cfg
+    # post_quant_conv (1x1, 4->4) is applied in fp32 by the latent-packing kernel
+    P["pq_w"] = _f32(sd["post_quant_conv.weight"].reshape(cfg.latent_channels, cfg.latent_channels), device)
+    P["pq_b"] = _f32(sd["post_quant_conv.bias"], device)
+    d = "decoder."
+    P["conv_in_w"] = pack_conv3x3(sd[d + "conv_in.weight"], device, pad_in_to=64)
+    P["conv_in_b"] = _f32(sd[d + "conv_in.bias"], device)
+    P["mid_res"] = [pack_resnet(sd, d + f"mid_block.resnets.{i}.", device) for i in range(2)]
+    P["mid_attn"] = pack_vae_attention(sd, d + "mid_block.attentions.0.", device)
     P["up"] = []
     n_up = len(cfg.block_out_channels)
     for i in range(n_up):
