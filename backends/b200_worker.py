@@ -12,7 +12,8 @@ Extras the reference does not have (SURVEY.md §8f rank 1): `run_batch(jobs)` ge
 requests of the same geometry in ONE batched pass (per-request Philox streams preserved) and
 `run_job_with_latents` returns the latent of the same pass instead of re-running the pipeline.
 Requests carrying `init_image` (and `strength`, see `backends/base.py`) run image-to-image through
-the same entry points (`LatentConsistencyModelImg2ImgPipeline` semantics, LCM UNets only).
+the same entry points (`LatentConsistencyModelImg2ImgPipeline` semantics, LCM UNets only); with a `mask_image`
+as well they run inpainting (`StableDiffusionInpaintPipeline` semantics with `LCMScheduler`, 4- and 9-channel UNets).
 """
 from __future__ import annotations
 
@@ -232,12 +233,14 @@ class B200Worker(PipelineWorker):
 
     def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True, init=None):
         """init (image-to-image): (u8 images [B,H,W,3], posterior draw [B,4,h,w], strength); lat is then the
-        add_noise draw."""
+        add_noise draw.  Inpainting appends (u8 masks [B,H,W], the masked image's posterior draw)."""
         pe = self._text.encode(prompts)
         neg = self._negative(len(prompts)) if self.pipe.cfg_scale_for(gs) is not None else None
         i2i = {}
         if init is not None:
             i2i = dict(init_images=init[0], posterior_noise=init[1], strength=init[2])
+            if len(init) > 3:
+                i2i.update(mask_images=init[3], masked_posterior_noise=init[4])
         return self.pipe.generate(pe, lat, noise, steps, gs, return_latents=True, use_graph=self._use_graph,
                                   negative_prompt_embeds=neg, decode=decode, **i2i)
 
@@ -247,6 +250,36 @@ class B200Worker(PipelineWorker):
             raise RuntimeError("image-to-image needs an LCM UNet (time_cond_proj_dim): the LCM img2img pipeline has "
                                "no classifier-free guidance branch, and CFG img2img is not implemented")
         self.pipe.require_encoder()
+
+    def _check_inpaint(self) -> None:
+        """Refuse inpainting where this engine does not implement diffusers' semantics."""
+        self.pipe.require_encoder()
+
+    def _inpaint_plan(self, steps: int, strength: float):
+        """-> (steps of the truncated schedule, whether the image's posterior draw is consumed: diffusers encodes the
+        image only for a 4-channel UNet or strength < 1).  ValueError when the strength leaves no step."""
+        from dreamlab_b200.scheduler import LCMSchedule
+        k = len(LCMSchedule(steps, strength, truncate=True).timesteps)
+        return k, getattr(self.pipe.unet.cfg, "in_channels", 4) != 9 or strength < 1.0
+
+    @staticmethod
+    def _mask_image(obj, width: int, height: int):
+        """A request's mask_image (image bytes PIL opens, converted to "L", or an HxW uint8 array of L values) ->
+        contiguous uint8 [height, width].  No resizing: any other size is refused."""
+        import numpy as np
+        if isinstance(obj, (bytes, bytearray, memoryview)):
+            from PIL import Image
+            with Image.open(io.BytesIO(bytes(obj))) as im:
+                arr = np.asarray(im.convert("L"))
+        else:
+            arr = np.asarray(obj)
+            if arr.dtype != np.uint8 or arr.ndim != 2:
+                raise RuntimeError(f"mask_image: image bytes or an HxW uint8 array expected, got "
+                                   f"{arr.dtype} {list(arr.shape)}")
+        if arr.shape != (height, width):
+            raise RuntimeError(f"mask_image is {arr.shape[1]}x{arr.shape[0]}, the request's size is "
+                               f"{width}x{height} (masks are not resized)")
+        return np.ascontiguousarray(arr)
 
     @staticmethod
     def _init_image(obj, width: int, height: int):
@@ -282,22 +315,29 @@ class B200Worker(PipelineWorker):
             int(torch.randint(0, 100_000_000, (1,)).item())
         return width, height, seed
 
-    def _draw(self, seed: int, h8: int, w8: int, steps: int, raw: bool = False, posterior: bool = False):
+    def _draw(self, seed: int, h8: int, w8: int, steps: int, raw: bool = False, posterior: bool = False,
+              masked: bool = False):
         """The reference's per-request Philox stream (`backends/cuda_worker.py:212-213`,
         SURVEY.md App. A.5): latents first, then one draw per non-final step.
         posterior (image-to-image): the posterior sample's draw comes first and is returned third; the
-        "latents" draw is then the add_noise noise (diffusers' prepare_latents order)."""
+        "latents" draw is then the add_noise noise (diffusers' prepare_latents order).
+        masked (inpainting): the masked image's posterior draw follows the latents draw (prepare_mask_latents runs
+        after prepare_latents) and is returned fourth; steps is then the truncated schedule's length."""
         gen = torch.Generator(device=self.device)
         gen.manual_seed(seed)
         shape = (1, 4, h8, w8)
         eps_s = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32) if posterior else None
         lat = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32)
+        eps_m = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32) if masked else None
         noise = [torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32)
                  for _ in range(steps - 1)]
         if not raw:
             lat = lat.to(self.dtype).float()
             noise = [z.to(self.dtype).float() for z in noise]
             eps_s = eps_s.to(self.dtype).float() if posterior else None
+            eps_m = eps_m.to(self.dtype).float() if masked else None
+        if masked:
+            return lat, noise, eps_s, eps_m
         return (lat, noise, eps_s) if posterior else (lat, noise)
 
     supports_deferred = True      # run_batch(..., deferred=True) -> thunks (see WorkerPool)
@@ -323,27 +363,45 @@ class B200Worker(PipelineWorker):
                 if (w, h) != (width, height) or int(j.req.num_inference_steps) != steps:
                     raise RuntimeError("run_batch: jobs must share size and num_inference_steps")
             inits = [getattr(j.req, "init_image", None) for j in jobs]
+            masks = [getattr(j.req, "mask_image", None) for j in jobs]
+            inpaint = any(m is not None for m in masks)
             init = None
-            if any(x is not None for x in inits):
-                if any(x is None for x in inits):
-                    raise RuntimeError("run_batch: image-to-image and text-to-image jobs cannot share a batch")
-                strengths = {0.8 if getattr(j.req, "strength", None) is None else float(j.req.strength) for j in jobs}
+            k, posterior = steps, False           # steps that run; whether the image's posterior draw is consumed
+            if inpaint or any(x is not None for x in inits):
+                if len({(x is not None, m is not None) for x, m in zip(inits, masks)}) != 1:
+                    raise RuntimeError("run_batch: inpainting, image-to-image and text-to-image jobs cannot share a "
+                                       "batch")
+                if inits[0] is None:
+                    raise RuntimeError("mask_image without init_image: inpainting repaints part of a given picture")
+                default = 1.0 if inpaint else 0.8
+                strengths = {default if getattr(j.req, "strength", None) is None else float(j.req.strength)
+                             for j in jobs}
                 if len(strengths) != 1:
-                    raise RuntimeError("run_batch: image-to-image jobs must share strength")
-                self._check_img2img()
-                # host work on this thread: PNG / JPEG decoding of the init images
+                    raise RuntimeError("run_batch: image-to-image and inpainting jobs must share strength")
+                strength = next(iter(strengths))
+                if inpaint:
+                    self._check_inpaint()
+                else:
+                    self._check_img2img()
+                # host work on this thread: PNG / JPEG decoding of the init images (and masks)
                 import numpy as np
                 imgs = torch.from_numpy(np.stack([self._init_image(x, width, height) for x in inits]))
-                init = [imgs, None, next(iter(strengths))]
+                init = [imgs, None, strength]
+                posterior = True
+                if inpaint:
+                    init += [torch.from_numpy(np.stack([self._mask_image(m, width, height) for m in masks])), None]
+                    k, posterior = self._inpaint_plan(steps, strength)
             # per-request Philox streams; the round trip through the noise dtype (CUDA_DTYPE) is applied once to
             # the assembled batch instead of per tensor (same values, ~8 fewer launches per request)
-            draws = [self._draw(seed, height // 8, width // 8, steps, raw=True, posterior=init is not None)
+            draws = [self._draw(seed, height // 8, width // 8, k, raw=True, posterior=posterior, masked=inpaint)
                      for _, _, seed in parsed]
-            if init is not None:
+            if posterior:
                 init[1] = torch.cat([d[2] for d in draws], 0).to(self.dtype).float()
+            if inpaint:
+                init[4] = torch.cat([d[3] for d in draws], 0).to(self.dtype).float()
             lat = torch.cat([d[0] for d in draws], 0).to(self.dtype).float()
-            noise = (torch.stack([torch.cat([d[1][i] for d in draws], 0) for i in range(steps - 1)]).to(self.dtype).float()
-                     if steps > 1 else None)
+            noise = (torch.stack([torch.cat([d[1][i] for d in draws], 0) for i in range(k - 1)]).to(self.dtype).float()
+                     if k > 1 else None)
             gs = torch.tensor([float(j.req.guidance_scale) for j in jobs])
             styles = {self._style_of(j.req) for j in jobs}
             if len(styles) != 1:
@@ -446,6 +504,10 @@ class B200SDXLWorker(B200Worker):
         raise RuntimeError("image-to-image is not implemented for SDXL: StableDiffusionXLImg2ImgPipeline truncates "
                            "the full schedule (get_timesteps), which is different semantics from the LCM img2img "
                            "pipeline built here")
+
+    def _check_inpaint(self) -> None:
+        raise RuntimeError("inpainting is not implemented for SDXL: StableDiffusionXLInpaintPipeline is not built, "
+                           "only the SD1.5-class inpainting pipeline")
 
     def _make_text_encoder(self, path):
         ucfg = self.pipe.unet.cfg

@@ -10,6 +10,12 @@ fields, also read with `getattr`: `init_image` — image bytes PIL can open (PNG
 uint8 array (what `run_job_array` returns), RGB and exactly `size` (no resizing) — and `strength` in
 (0, 1] (default 0.8): how far the init image is noised before the LCM steps redraw it.
 
+Inpainting (`StableDiffusionInpaintPipeline` semantics with `LCMScheduler`) adds `mask_image` to `init_image`, also
+read with `getattr`: image bytes PIL can open (converted to "L") or an HxW uint8 array of L values, exactly `size`.
+Pixels with L >= 128 are repainted, the others kept.  `strength` then defaults to 1.0 and truncates the full step
+schedule (int(steps * strength) of its last steps run).  A model whose UNet has 9 input channels (an inpainting UNet)
+serves only such requests.
+
 Only names, fields and return conventions are shared with the reference — they ARE the
 interface; everything a caller can observe is pinned by `tests/test_worker_pool.py` and
 `tests/test_worker_factory.py`.
@@ -58,7 +64,8 @@ class GenSpec:
     seed: Optional[int] = None
     style_lora: StyleLora = field(default_factory=StyleLora)
     init_image: Any = None                   # image-to-image: image bytes or HxWx3 uint8 array
-    strength: Optional[float] = None         # image-to-image strength (None: 0.8)
+    strength: Optional[float] = None         # image-to-image strength (None: 0.8; inpainting: 1.0)
+    mask_image: Any = None                   # inpainting: image bytes or HxW uint8 array, with init_image
 
 
 @dataclass

@@ -124,7 +124,8 @@ def _auto_num_workers() -> int:
 def _batch_key(job, same_guidance: bool = False):
     """Generation jobs that may share one batched pass: same size, step count and style (and,
     for workers that run classifier-free guidance on a doubled batch, the same guidance scale).
-    Image-to-image requests (an `init_image`) also share their strength: ("img2img", strength) is appended."""
+    Image-to-image requests (an `init_image`) also share their strength: ("img2img", strength) is appended;
+    inpainting requests (a `mask_image`) append ("inpaint", strength) instead (default strength 1.0)."""
     req = getattr(job, "req", None)
     try:
         if same_guidance:
@@ -134,7 +135,10 @@ def _batch_key(job, same_guidance: bool = False):
         if not style[0] or style[1] <= 0:
             style = (None, 0)
         key = (str(req.size).lower(), int(req.num_inference_steps), style)
-        if getattr(req, "init_image", None) is not None:
+        if getattr(req, "mask_image", None) is not None:
+            st = getattr(req, "strength", None)
+            key += (("inpaint", 1.0 if st is None else float(st)),)
+        elif getattr(req, "init_image", None) is not None:
             st = getattr(req, "strength", None)
             key += (("img2img", 0.8 if st is None else float(st)),)
         return key

@@ -320,6 +320,36 @@ int dl_vae_sample_latents(const float* moments, const float* eps_s, const float*
                           float scaling_factor, float sqrt_alpha, float sqrt_one_minus_alpha, float* out,
                           float* mean_out, void* stream);
 
+/* ---- inpainting (diffusers StableDiffusionInpaintPipeline with LCMScheduler) -------------------------------------
+ * dl_pack_image_im2col_masked: dl_pack_image_im2col of the masked image: mask u8 [nimg, h, w] (row / image strides in
+ *   bytes, so a tile window is read in place like the image); a pixel with m >= 128 reads as 0.0 (the normalised
+ *   middle grey of image * (binarised mask < 0.5)) before the zero padding.
+ * dl_inpaint_latent_mask: u8 full-resolution masks [nimg, 8h, 8w] -> fp32 latent mask [nimg, h, w]:
+ *   out[n, i, j] = mask[n, 8i, 8j] >= 128 ? 1 : 0 (binarise at 0.5, then F.interpolate's default nearest).
+ * dl_pack_latent_inpaint: the operand of a 9-channel UNet's conv_in, bf16 (or fp32 for _f32) [repeat*npix, 64]:
+ *   channels 0-3 latents, 4 mask, 5-8 masked_image_latents, 9-63 zero; latents / masked fp32 NHWC [npix, 4],
+ *   mask fp32 [npix]; the npix pixels are written `repeat` times (classifier-free guidance halves).
+ * dl_lcm_step_inpaint: dl_lcm_step (same roundings) followed by the 4-channel UNet's blend, fp32 NHWC [npix, 4]:
+ *   proper = last ? image_latents : sqrt_alpha * image_latents + sqrt_one_minus_alpha * noise0
+ *   x_next = (1 - mask) * proper + mask * prev_sample      (every mul / add / sub rounded on its own)
+ *   with (sqrt_alpha, sqrt_one_minus_alpha) the add_noise coefficients of the next timestep; noise (the step's draw)
+ *   may be NULL on the last step, noise0 (the draw that made the starting latents) may be NULL when last != 0.   */
+int dl_pack_image_im2col_masked(const void* img_u8, const void* mask_u8, int nimg, int h, int w, long long row_stride,
+                                long long img_stride, long long mask_row_stride, long long mask_img_stride, void* out,
+                                void* stream);
+int dl_pack_image_im2col_masked_f32(const void* img_u8, const void* mask_u8, int nimg, int h, int w,
+                                    long long row_stride, long long img_stride, long long mask_row_stride,
+                                    long long mask_img_stride, float* out, void* stream);
+int dl_inpaint_latent_mask(const void* mask_u8, int nimg, int h, int w, float* out, void* stream);
+int dl_pack_latent_inpaint(const float* latents, const float* mask, const float* masked, long long npix, int repeat,
+                           void* out, void* stream);
+int dl_pack_latent_inpaint_f32(const float* latents, const float* mask, const float* masked, long long npix,
+                               int repeat, float* out, void* stream);
+int dl_lcm_step_inpaint(const float* eps, const float* x, const float* noise, const float* image_latents,
+                        const float* noise0, const float* mask, float* x_next, float* denoised, long long npix,
+                        const dl_lcm_coeffs* k, float sqrt_alpha, float sqrt_one_minus_alpha, int last,
+                        void* stream);
+
 #ifdef __cplusplus
 }
 #endif

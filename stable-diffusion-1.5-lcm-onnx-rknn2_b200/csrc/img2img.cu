@@ -10,9 +10,13 @@ namespace dl {
 // h x w window), 0 for 27 <= k < 64.  Each value is VaeImageProcessor's 2 * (u8 / 255) - 1 with IEEE division and
 // no contraction; the zero padding applies to the normalised image (out-of-window taps are 0.0, not -1).
 // One thread per 8 consecutive k of one pixel.
+// mask (inpainting, nullable): u8 [nimg, h, w] at its own strides; a pixel with m >= 128 reads as 0.0 before the
+// zero padding (StableDiffusionInpaintPipeline's masked_image = image * (binarised mask < 0.5)).
 template <typename T>
 __global__ void pack_image_im2col_kernel(const uint8_t* __restrict__ img, int nimg, int h, int w,
-                                         long long row_stride, long long img_stride, T* __restrict__ out) {
+                                         long long row_stride, long long img_stride, T* __restrict__ out,
+                                         const uint8_t* __restrict__ mask, long long mask_row_stride,
+                                         long long mask_img_stride) {
   const long long total = (long long)nimg * h * w * 8;
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < total;
        i += (long long)gridDim.x * blockDim.x) {
@@ -30,7 +34,8 @@ __global__ void pack_image_im2col_kernel(const uint8_t* __restrict__ img, int ni
       if (k < 27) {
         const int tap = k / 3, c = k % 3;
         const int yi = y + tap / 3 - 1, xi = x + tap % 3 - 1;
-        if (yi >= 0 && yi < h && xi >= 0 && xi < w) {
+        if (yi >= 0 && yi < h && xi >= 0 && xi < w &&
+            (mask == nullptr || mask[n * mask_img_stride + yi * mask_row_stride + xi] < 128)) {
           const float u = (float)img[n * img_stride + yi * row_stride + 3LL * xi + c];
           v[j] = __fsub_rn(__fmul_rn(2.f, __fdiv_rn(u, 255.f)), 1.f);
         }
@@ -94,7 +99,7 @@ extern "C" int dl_pack_image_im2col(const void* img_u8, int nimg, int h, int w, 
   const long long total = (long long)nimg * h * w * 8;
   pack_image_im2col_kernel<__nv_bfloat16><<<i2i_grid(total, 256), 256, 0, STREAM>>>(
       reinterpret_cast<const uint8_t*>(img_u8), nimg, h, w, row_stride, img_stride,
-      reinterpret_cast<__nv_bfloat16*>(out));
+      reinterpret_cast<__nv_bfloat16*>(out), nullptr, 0, 0);
   return check_launch("pack_image_im2col");
 }
 
@@ -104,8 +109,35 @@ extern "C" int dl_pack_image_im2col_f32(const void* img_u8, int nimg, int h, int
                (nimg == 1 || img_stride >= row_stride * h), "pack_image_im2col_f32: bad args");
   const long long total = (long long)nimg * h * w * 8;
   pack_image_im2col_kernel<float><<<i2i_grid(total, 256), 256, 0, STREAM>>>(
-      reinterpret_cast<const uint8_t*>(img_u8), nimg, h, w, row_stride, img_stride, out);
+      reinterpret_cast<const uint8_t*>(img_u8), nimg, h, w, row_stride, img_stride, out, nullptr, 0, 0);
   return check_launch("pack_image_im2col_f32");
+}
+
+extern "C" int dl_pack_image_im2col_masked(const void* img_u8, const void* mask_u8, int nimg, int h, int w,
+                                           long long row_stride, long long img_stride, long long mask_row_stride,
+                                           long long mask_img_stride, void* out, void* stream_) {
+  DL_CHECK_ARG(img_u8 && mask_u8 && out && nimg > 0 && h > 0 && w > 0 && row_stride >= 3LL * w &&
+               (nimg == 1 || img_stride >= row_stride * h) && mask_row_stride >= w &&
+               (nimg == 1 || mask_img_stride >= mask_row_stride * h), "pack_image_im2col_masked: bad args");
+  const long long total = (long long)nimg * h * w * 8;
+  pack_image_im2col_kernel<__nv_bfloat16><<<i2i_grid(total, 256), 256, 0, STREAM>>>(
+      reinterpret_cast<const uint8_t*>(img_u8), nimg, h, w, row_stride, img_stride,
+      reinterpret_cast<__nv_bfloat16*>(out), reinterpret_cast<const uint8_t*>(mask_u8), mask_row_stride,
+      mask_img_stride);
+  return check_launch("pack_image_im2col_masked");
+}
+
+extern "C" int dl_pack_image_im2col_masked_f32(const void* img_u8, const void* mask_u8, int nimg, int h, int w,
+                                               long long row_stride, long long img_stride, long long mask_row_stride,
+                                               long long mask_img_stride, float* out, void* stream_) {
+  DL_CHECK_ARG(img_u8 && mask_u8 && out && nimg > 0 && h > 0 && w > 0 && row_stride >= 3LL * w &&
+               (nimg == 1 || img_stride >= row_stride * h) && mask_row_stride >= w &&
+               (nimg == 1 || mask_img_stride >= mask_row_stride * h), "pack_image_im2col_masked_f32: bad args");
+  const long long total = (long long)nimg * h * w * 8;
+  pack_image_im2col_kernel<float><<<i2i_grid(total, 256), 256, 0, STREAM>>>(
+      reinterpret_cast<const uint8_t*>(img_u8), nimg, h, w, row_stride, img_stride, out,
+      reinterpret_cast<const uint8_t*>(mask_u8), mask_row_stride, mask_img_stride);
+  return check_launch("pack_image_im2col_masked_f32");
 }
 
 extern "C" int dl_vae_sample_latents(const float* moments, const float* eps_s, const float* eps_n, int nimg, int h,

@@ -404,10 +404,14 @@ class UNetB200:
 
     @torch.no_grad()
     def forward(self, latents_nhwc: torch.Tensor, temb: torch.Tensor, kvs: List[List[torch.Tensor]],
-                eps_out: Optional[torch.Tensor] = None, repeat: int = 1, comm=None) -> torch.Tensor:
+                eps_out: Optional[torch.Tensor] = None, repeat: int = 1, comm=None, inpaint_cond=None) -> torch.Tensor:
         """latents_nhwc fp32 [b,h,w,4] -> noise_pred fp32 [b*repeat,h,w,4].  repeat=2 is the
         classifier-free-guidance doubled batch `cat([latents]*2)`: the same latents are packed
         twice, temb / kvs carry the [uncond, cond] halves.
+
+        inpaint_cond (a 9-channel inpainting UNet, and only there): (latent mask fp32 [b,h,w], masked_image_latents
+        fp32 NHWC [b,h,w,4]); the UNet input is cat([latents, mask, masked_image_latents]) per image, doubled
+        together with the latents under guidance.
 
         comm (patch parallel, SURVEY.md §8e): this rank computes rows
         [rank*h/R, (rank+1)*h/R) of every image and returns that strip [b*repeat, h/R, w, 4];
@@ -418,6 +422,14 @@ class UNetB200:
         if comm is not None and self.dt != BF16:
             raise RuntimeError("patch parallel runs on the bf16 path only (the split GroupNorm kernels have no "
                                "fp32 variant); the fp32 precision mode is a one-GPU parity mode")
+        if comm is not None and inpaint_cond is not None:
+            raise RuntimeError("patch parallel does not implement the inpainting conditioning (9-channel conv_in)")
+        cin_model = getattr(self.cfg, "in_channels", 4)
+        if cin_model == 9 and inpaint_cond is None:
+            raise RuntimeError("this UNet has in_channels=9 (an inpainting UNet): it needs the mask and the masked "
+                               "image latents; text-to-image and image-to-image are not defined for it")
+        if cin_model != 9 and inpaint_cond is not None:
+            raise RuntimeError(f"inpaint_cond is the input of a 9-channel UNet, this one has in_channels={cin_model}")
         g = self.groups
         # GroupNorm statistics from the producers' epilogues (per-channel records): every GroupNorm of the
         # UNet becomes finalize + ONE pass; DL_UNET_GN_FUSE=0 keeps the cooperative two-phase kernel (A/B)
@@ -426,8 +438,11 @@ class UNetB200:
         kv_it = iter(kvs)
         if comm is None:
             xin = ctx.empty(B, H, W, 64)
-            for r in range(repeat):
-                lib.pack_latent(latents_nhwc, xin[r * b0:(r + 1) * b0], cin=Cin)
+            if inpaint_cond is not None:
+                lib.pack_latent_inpaint(latents_nhwc, inpaint_cond[0], inpaint_cond[1], xin, repeat=repeat)
+            else:
+                for r in range(repeat):
+                    lib.pack_latent(latents_nhwc, xin[r * b0:(r + 1) * b0], cin=Cin)
         else:
             n_lv = len(ch)
             if H % (comm.world << (n_lv - 1)):
@@ -464,9 +479,10 @@ class UNetB200:
             if blk["up"] is not None:
                 h = upsample(ctx, h, blk["up"])
         hn = groupnorm(ctx, h, P["norm_out_w"], P["norm_out_b"], eps=1e-5, silu=True, groups=g, halo=True)
+        cout = getattr(self.cfg, "out_channels", Cin)
         if eps_out is None:
-            eps_out = torch.empty(B, H, W, Cin, device=self.device, dtype=torch.float32)
-        conv3x3(ctx, hn, P["conv_out_w"], P["conv_out_b"], Cin, mode=lib.EPI_F32, out=eps_out, ldo=Cin)
+            eps_out = torch.empty(B, H, W, cout, device=self.device, dtype=torch.float32)
+        conv3x3(ctx, hn, P["conv_out_w"], P["conv_out_b"], cout, mode=lib.EPI_F32, out=eps_out, ldo=cout)
         return eps_out
 
 
@@ -726,18 +742,21 @@ class VAEEncoderB200:
         self.flash_attention = os.environ.get("DL_VAE_FLASH", "1") not in ("0", "false") and self.dt == BF16
 
     @torch.no_grad()
-    def moments(self, img_u8: torch.Tensor, tiling: bool = False, comm=None) -> torch.Tensor:
+    def moments(self, img_u8: torch.Tensor, tiling: bool = False, comm=None, mask=None,
+                keep_unmasked: bool = False) -> torch.Tensor:
         """img_u8: u8 NHWC [B,H,W,3] on the device (H, W multiples of 8).  tiling: images larger than
-        sample_size in either dim are encoded tile by tile and blended (`tiled_encode`)."""
+        sample_size in either dim are encoded tile by tile and blended (`tiled_encode`).
+        mask (inpainting): u8 [B,H,W]; the masked images (pixels with m >= 128 at 0.0) are encoded instead, or,
+        with keep_unmasked, after the unmasked ones in one batch of 2B: moments [2B, ...] = [image; masked image]."""
         if comm is not None:
             raise RuntimeError("VAE encoder: strip-parallel encode is not implemented")
         t = self.cfg.sample_size
         if tiling and (img_u8.shape[1] > t or img_u8.shape[2] > t):
-            return self.tiled_moments(img_u8)
-        return self._encode(img_u8)
+            return self.tiled_moments(img_u8, mask, keep_unmasked)
+        return self._encode(img_u8, mask, keep_unmasked)
 
     @torch.no_grad()
-    def tiled_moments(self, img_u8: torch.Tensor) -> torch.Tensor:
+    def tiled_moments(self, img_u8: torch.Tensor, mask=None, keep_unmasked: bool = False) -> torch.Tensor:
         """diffusers `AutoencoderKL.tiled_encode`: tiles of sample_size pixels at stride 0.75 tile, each encoded
         on its own (own GroupNorm statistics and attention, zero padding at the tile border), moments blended
         over sample_size/32 latents with the already blended upper / left neighbour, cropped to 0.75 of a tile
@@ -748,14 +767,16 @@ class VAEEncoderB200:
         tl = t // 8
         blend = int(tl * 0.25)
         limit = tl - blend
-        out = torch.empty(B, H // 8, W // 8, 2 * self.cfg.latent_channels, device=self.device, dtype=torch.float32)
+        nb = 2 * B if mask is not None and keep_unmasked else B
+        out = torch.empty(nb, H // 8, W // 8, 2 * self.cfg.latent_channels, device=self.device, dtype=torch.float32)
         prev_row = []
         oy = 0
         for i in range(0, H, stride):
             row = []
             ox = 0
             for jn, j in enumerate(range(0, W, stride)):
-                tile = self._encode(img_u8[:, i:i + t, j:j + t])           # a view: read in place
+                tile = self._encode(img_u8[:, i:i + t, j:j + t],          # views: read in place
+                                    None if mask is None else mask[:, i:i + t, j:j + t], keep_unmasked)
                 if i > 0:
                     up = prev_row[jn]
                     lib.tile_blend(up, tile, min(up.shape[1], tile.shape[1], blend), vertical=True)
@@ -779,17 +800,21 @@ class VAEEncoderB200:
         return _carry_gn(out, out.view(B, H // 2, W // 2, C))
 
     @torch.no_grad()
-    def _encode(self, img_u8: torch.Tensor) -> torch.Tensor:
-        """One untiled encode (img_u8 may be a window of a larger canvas)."""
+    def _encode(self, img_u8: torch.Tensor, mask=None, keep_unmasked: bool = False) -> torch.Tensor:
+        """One untiled encode (img_u8 and mask may be windows of a larger canvas)."""
         P = self.P
-        B, H, W, _ = img_u8.shape
+        B0, H, W, _ = img_u8.shape
         if H % 8 or W % 8:
             raise RuntimeError(f"VAE encoder: image {W}x{H} is not a multiple of 8")
+        B = 2 * B0 if mask is not None and keep_unmasked else B0
         g = self.groups
         ctx = _Ctx(self.device, B, gn_fuse=g if self.fuse_gn_stats else 0, dt=self.dt)
         ch = self.cfg.block_out_channels
         cols = ctx.empty(B * H * W, 64)
-        lib.pack_image_im2col(img_u8, cols)
+        if mask is None or keep_unmasked:
+            lib.pack_image_im2col(img_u8, cols[:B0 * H * W])
+        if mask is not None:
+            lib.pack_image_im2col(img_u8, cols[(B - B0) * H * W:], mask=mask)
         h = linear(ctx, cols, P["conv_in_w"], P["conv_in_b"], ch[0], norm_rows_per_img=H * W)
         h = _carry_gn(h, h.view(B, H, W, ch[0]))
         for blk in P["down"]:
@@ -830,11 +855,13 @@ def _pinned(x: torch.Tensor) -> torch.Tensor:
 
 
 class _StaticGraph:
-    """One captured CUDA graph of the whole hot path for a fixed (B, h, w, steps[, gs][, strength]).
+    """One captured CUDA graph of the whole hot path for a fixed (B, h, w, steps[, gs][, strength][, inpaint]).
     strength set: image-to-image; the init images and the posterior draw are static inputs too, and `lat`
-    holds the add_noise draw."""
+    holds the add_noise draw.  inpaint: the masks and the masked image's posterior draw are static inputs as well,
+    and `noise` holds one draw per non-final step of the truncated schedule."""
 
-    def __init__(self, pipe: "LCMPipelineB200", B, h, w, steps, cfg_scale=None, decode=True, strength=None):
+    def __init__(self, pipe: "LCMPipelineB200", B, h, w, steps, cfg_scale=None, decode=True, strength=None,
+                 inpaint=False):
         dev = pipe.device
         ucfg = pipe.unet.cfg
         D = ucfg.cross_attention_dim
@@ -848,15 +875,19 @@ class _StaticGraph:
             self.add = (torch.zeros(Bc, pdim, device=dev, dtype=torch.float32),
                         torch.zeros(Bc, 6, device=dev, dtype=torch.float32))
         self.lat = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
-        self.noise = torch.zeros(max(steps - 1, 1), B, 4, h, w, device=dev, dtype=torch.float32)
+        k = len(pipe.schedule(steps, strength, inpaint).timesteps) if inpaint else steps
+        self.noise = torch.zeros(max(k - 1, 1), B, 4, h, w, device=dev, dtype=torch.float32)
         self.steps = steps
-        self.init_u8 = self.eps_s = None
+        self.init_u8 = self.eps_s = self.mask_u8 = self.eps_m = None
         if strength is not None:
             self.init_u8 = torch.zeros(B, 8 * h, 8 * w, 3, device=dev, dtype=torch.uint8)
             self.eps_s = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
+        if inpaint:
+            self.mask_u8 = torch.zeros(B, 8 * h, 8 * w, device=dev, dtype=torch.uint8)
+            self.eps_m = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
         args = (self.pe, self.w_emb, self.lat, self.noise, steps)
         kw = dict(add=self.add, cfg_scale=cfg_scale, decode=decode, init_u8=self.init_u8, eps_s=self.eps_s,
-                  strength=strength)
+                  strength=strength, mask_u8=self.mask_u8, eps_m=self.eps_m)
         with CAPTURE_LOCK:
             # warm-up on a side stream (lazy per-device init: smem attributes, module load)
             s = torch.cuda.Stream(device=dev)
@@ -925,22 +956,26 @@ class LCMPipelineB200:
     @torch.no_grad()
     def run_static(self, pe_bf16, w_emb, lat_nchw, noise_nchw, steps: int, record: dict = None,
                    add=None, cfg_scale: Optional[float] = None, teacher=None, decode: bool = True,
-                   init_u8=None, eps_s=None, strength: Optional[float] = None):
+                   init_u8=None, eps_s=None, strength: Optional[float] = None, mask_u8=None, eps_m=None):
         """Everything on device, no host sync, graph-capturable.  Returns (u8 images, latents).
         pe_bf16 / add carry 2B rows ([uncond, cond]) when cfg_scale is set.
         init_u8 (image-to-image): u8 NHWC init images; the pass becomes encode -> posterior sample with eps_s ->
-        add_noise at the first timestep of the strength schedule with lat_nchw as the noise -> denoise -> decode."""
+        add_noise at the first timestep of the strength schedule with lat_nchw as the noise -> denoise -> decode.
+        mask_u8 (inpainting, with init_u8): u8 [B,H,W] masks; see `inpaint_latents`, eps_m is the masked image's
+        posterior draw, the schedule is the truncated one and noise_nchw holds its non-final steps' draws."""
         B = lat_nchw.shape[0]
         Bu = 2 * B if cfg_scale is not None else B
-        sched = LCMSchedule(steps) if init_u8 is None else LCMSchedule(steps, strength)
+        sched = self.schedule(steps, strength if init_u8 is not None else None, mask_u8 is not None)
         kvs = self.unet.encode_context(pe_bf16)
         aug = self.unet.addition_embedding(*add) if add is not None else None
         tembs = self.unet.time_embeddings(sched.timesteps, Bu, w_emb, aug)
-        start = None
-        if init_u8 is not None:
+        start = inpaint = None
+        if mask_u8 is not None:
+            start, inpaint = self.inpaint_latents(init_u8, mask_u8, eps_s, eps_m, lat_nchw, sched, record)
+        elif init_u8 is not None:
             start = self.init_latents(init_u8, eps_s, lat_nchw, sched, record)
         lat = self.denoise(lat_nchw, noise_nchw, sched, kvs, tembs, record, cfg_scale=cfg_scale, teacher=teacher,
-                           start_nhwc=start)
+                           start_nhwc=start, inpaint=inpaint)
         if not decode:                   # latent-only callers (candidate scoring): no VAE pass at all
             return None, lat
         return self.vae.decode(lat, tiling=self.vae_tiling), lat
@@ -961,10 +996,63 @@ class LCMPipelineB200:
             record["init_latents"] = x.permute(0, 3, 1, 2).clone()
         return x
 
+    def inpaint_latents(self, init_u8, mask_u8, eps_s, eps_m, noise_nchw, sched: LCMSchedule, record: dict = None):
+        """`StableDiffusionInpaintPipeline.prepare_latents` + `prepare_mask_latents`.  image_latents =
+        scaling_factor * posterior sample (eps_s) of the image, only where diffusers computes it (a 4-channel UNet, or
+        strength < 1); masked_image_latents likewise of the masked image (eps_m), for a 9-channel UNet only (a
+        4-channel UNet never reads it).  Both encodes run as one batch.  The starting latents are the noise draw
+        itself at strength 1, else add_noise(image_latents, noise, timesteps[0]).
+        -> (starting latents fp32 NHWC [B,h,w,4], dict(cond=(mask, masked) for a 9-channel UNet or None,
+        blend=(image_latents, noise NHWC, mask) for a 4-channel UNet or None)); mask is the fp32 latent mask [B,h,w]."""
+        enc = self.require_encoder()
+        nine = getattr(self.unet.cfg, "in_channels", 4) == 9
+        need_img = not nine or sched.strength < 1.0
+        B, H, W, _ = init_u8.shape
+        h, w = H // 8, W // 8
+        f32 = dict(device=self.device, dtype=torch.float32)
+        sf = self.vae.cfg.scaling_factor
+        mom = enc.moments(init_u8, tiling=self.vae_tiling, mask=mask_u8 if nine else None, keep_unmasked=need_img)
+        mask = torch.empty(B, h, w, **f32)
+        lib.inpaint_latent_mask(mask_u8, mask)
+        noise = torch.empty(B, h, w, 4, **f32)
+        lib.nchw_to_nhwc_f32(noise_nchw, noise)
+        image = masked = None
+        if need_img:          # (sqrt_alpha, sqrt_one_minus_alpha) = (1, 0): the scaled posterior sample itself
+            image = torch.empty(B, h, w, 4, **f32)
+            lib.vae_sample_latents(mom[:B], eps_s, eps_s, image, scaling_factor=sf, sqrt_alpha=1.0,
+                                   sqrt_one_minus_alpha=0.0)
+        if nine:
+            masked = torch.empty(B, h, w, 4, **f32)
+            lib.vae_sample_latents(mom[mom.shape[0] - B:], eps_m, eps_m, masked, scaling_factor=sf, sqrt_alpha=1.0,
+                                   sqrt_one_minus_alpha=0.0)
+        if sched.strength >= 1.0:            # is_strength_max: latents = noise * init_noise_sigma (1.0)
+            start = noise
+        else:
+            start = torch.empty(B, h, w, 4, **f32)
+            sa, sb = sched.add_noise_coeffs()
+            lib.vae_sample_latents(mom[:B], eps_s, noise_nchw, start, scaling_factor=sf, sqrt_alpha=sa,
+                                   sqrt_one_minus_alpha=sb)
+        if record is not None:
+            record["moments"] = mom.permute(0, 3, 1, 2).clone()
+            record["mask"] = mask.clone()
+            record["init_latents"] = start.permute(0, 3, 1, 2).clone()
+            if image is not None:
+                record["image_latents"] = image.permute(0, 3, 1, 2).clone()
+            if masked is not None:
+                record["masked_image_latents"] = masked.permute(0, 3, 1, 2).clone()
+        return start, dict(cond=(mask, masked) if nine else None, blend=None if nine else (image, noise, mask))
+
+    def schedule(self, steps: int, strength: Optional[float] = None, inpaint: bool = False) -> LCMSchedule:
+        """The pass's schedule: text-to-image (strength None), image-to-image (re-spaced by strength) or
+        inpainting (the full schedule truncated by strength)."""
+        if inpaint:
+            return LCMSchedule(steps, strength, truncate=True)
+        return LCMSchedule(steps) if strength is None else LCMSchedule(steps, strength)
+
     def require_encoder(self) -> VAEEncoderB200:
         if self.vae_encoder is None:
-            raise RuntimeError("image-to-image needs the VAE encoder, and this model's VAE has no encoder weights "
-                               "(encoder.* / quant_conv.*)")
+            raise RuntimeError("image-to-image and inpainting need the VAE encoder, and this model's VAE has no "
+                               "encoder weights (encoder.* / quant_conv.*)")
         return self.vae_encoder
 
     max_graphs = 12       # captured geometries kept per pipeline
@@ -977,24 +1065,29 @@ class LCMPipelineB200:
             self._pool = torch.cuda.graph_pool_handle()
         return self._pool
 
-    def graph_for(self, B, h, w, steps, cfg_scale=None, decode=True, strength=None) -> _StaticGraph:
+    def graph_for(self, B, h, w, steps, cfg_scale=None, decode=True, strength=None, inpaint=False) -> _StaticGraph:
         key = (B, h, w, steps, cfg_scale, decode)
-        if strength is not None:                                 # image-to-image: its own graph per strength
+        if inpaint:                                              # inpainting: its own graph per strength
+            key += ("inpaint", strength)
+        elif strength is not None:                               # image-to-image: its own graph per strength
             key += ("img2img", strength)
         g = self._graphs.pop(key, None)
         if g is None:
             while len(self._graphs) >= self.max_graphs:          # least recently used goes first
                 self._graphs.pop(next(iter(self._graphs)))
             with torch.cuda.device(self.device):
-                g = _StaticGraph(self, B, h, w, steps, cfg_scale, decode, strength)
+                g = _StaticGraph(self, B, h, w, steps, cfg_scale, decode, strength, inpaint)
         self._graphs[key] = g                                     # dict order = recency
         return g
 
     @torch.no_grad()
     def denoise(self, latents_nchw, step_noise_nchw, sched, kvs, tembs, record: dict = None,
-                cfg_scale: Optional[float] = None, teacher=None, start_nhwc=None):
-        """latents fp32 NCHW [B,4,h,w]; step_noise [steps-1,B,4,h,w].  Returns final latents NHWC.
-        start_nhwc (image-to-image): the initial latents, already NHWC; latents_nchw then only gives the shape.
+                cfg_scale: Optional[float] = None, teacher=None, start_nhwc=None, inpaint=None):
+        """latents fp32 NCHW [B,4,h,w]; step_noise [steps-1,B,4,h,w] (steps = len(sched.timesteps)).  Returns final
+        latents NHWC.
+        start_nhwc (image-to-image, inpainting): the initial latents, already NHWC; latents_nchw then only gives the
+        shape.  inpaint: the second result of `inpaint_latents` — the 9-channel UNet input, or the 4-channel UNet's
+        blend fused into the scheduler step.
         teacher (parity tests): fp32 NCHW [steps,B,4,h,w] — the latents fed to the UNet at step i
         come from this tensor (an oracle trajectory) instead of from the previous step, so every
         step's noise_pred is compared on identical inputs (teacher forcing)."""
@@ -1004,7 +1097,7 @@ class LCMPipelineB200:
         else:
             x = torch.empty(B, H, W, C, device=self.device, dtype=torch.float32)
             lib.nchw_to_nhwc_f32(latents_nchw, x)
-        n = sched.num_inference_steps
+        n = len(sched.timesteps)
         noise = None
         if n > 1:
             noise = torch.empty(n - 1, B, H, W, C, device=self.device, dtype=torch.float32)
@@ -1016,19 +1109,30 @@ class LCMPipelineB200:
             tx = torch.empty(n, B, H, W, C, device=self.device, dtype=torch.float32)
             lib.nchw_to_nhwc_f32(teacher.to(self.device, torch.float32).reshape(n * B, C, H, W).contiguous(),
                                  tx.view(n * B, H, W, C))
+        cond = inpaint["cond"] if inpaint is not None else None
+        blend = inpaint["blend"] if inpaint is not None else None
         for i in range(n):
             if tx is not None:
                 x = tx[i]
             if cfg_scale is None:
-                eps = self.unet.forward(x, tembs[i], kvs)
+                eps = self.unet.forward(x, tembs[i], kvs, inpaint_cond=cond)
             else:
-                eps2 = self.unet.forward(x, tembs[i], kvs, repeat=2)
+                eps2 = self.unet.forward(x, tembs[i], kvs, repeat=2, inpaint_cond=cond)
                 eps = torch.empty_like(x)
                 lib.cfg_combine(eps2[:B], eps2[B:], cfg_scale, eps)
                 if record is not None:      # the UNet output before guidance: [uncond; text]
                     record.setdefault("noise_pred_raw", []).append(eps2.permute(0, 3, 1, 2).clone())
             x_next = torch.empty_like(x)
-            lib.lcm_step(eps, x, noise[i] if sched.has_noise(i) else None, x_next, den, sched.coeffs(i))
+            z = noise[i] if sched.has_noise(i) else None
+            if blend is not None:
+                # latents = (1 - m) * add_noise(image_latents, noise, timesteps[i + 1]) + m * latents; image_latents
+                # itself after the last step
+                last = i == n - 1
+                lib.lcm_step_inpaint(eps, x, z, blend[0], None if last else blend[1], blend[2], x_next, den,
+                                     sched.coeffs(i), (1.0, 0.0) if last else
+                                     sched.add_noise_coeffs(sched.timesteps[i + 1]), last)
+            else:
+                lib.lcm_step(eps, x, z, x_next, den, sched.coeffs(i))
             if record is not None:
                 record.setdefault("noise_pred", []).append(eps.permute(0, 3, 1, 2).clone())
                 record.setdefault("latents", []).append(x_next.permute(0, 3, 1, 2).clone())
@@ -1064,7 +1168,8 @@ class LCMPipelineB200:
                  guidance_scale=1.0, record: dict = None, return_latents: bool = False,
                  use_graph: bool = False, pooled_embeds=None, time_ids=None,
                  negative_prompt_embeds=None, negative_pooled_embeds=None, teacher_latents=None,
-                 decode: bool = True, init_images=None, strength: Optional[float] = None, posterior_noise=None):
+                 decode: bool = True, init_images=None, strength: Optional[float] = None, posterior_noise=None,
+                 mask_images=None, masked_posterior_noise=None):
         """Public entry: host or device tensors in -> u8 images [B,H,W,3] on device (and the
         final latents NHWC fp32 if asked).  With use_graph the whole pass is one CUDA-graph
         replay; the returned tensors are the graph's static outputs (consume before next call).
@@ -1072,10 +1177,40 @@ class LCMPipelineB200:
         Image-to-image (`LatentConsistencyModelImg2ImgPipeline`): init_images u8 [B,H,W,3] (H = 8h, W = 8w),
         strength in (0, 1] (default 0.8), posterior_noise fp32 [B,4,h,w] (the posterior sample's draw);
         latents_nchw is then the add_noise draw.  Needs an LCM UNet (time_cond_proj_dim) and VAE encoder
-        weights."""
+        weights.
+
+        Inpainting (`StableDiffusionInpaintPipeline` with `LCMScheduler`): init_images as above plus mask_images u8
+        [B,H,W] (L values; m >= 128 is repainted), strength in (0, 1] (default 1.0) truncating the full schedule.
+        latents_nchw is the latents / add_noise draw, posterior_noise the image's posterior draw (needed by a 4-channel
+        UNet, and by a 9-channel one at strength < 1), masked_posterior_noise the masked image's (9-channel UNets);
+        step_noise_nchw holds len(truncated schedule) - 1 draws.  A 9-channel (inpainting) UNet serves nothing else;
+        classifier-free guidance applies as for text-to-image."""
         B, _, h, w = latents_nchw.shape
         steps = int(num_inference_steps)
-        if init_images is not None:
+        nine = getattr(self.unet.cfg, "in_channels", 4) == 9
+        inpaint = mask_images is not None
+        k = steps                                         # steps that run (inpainting: the truncated schedule's)
+        if nine and not inpaint:
+            raise RuntimeError("this model's UNet has in_channels=9 (an inpainting UNet): it serves inpainting only "
+                               "(init_images + mask_images); text-to-image and image-to-image are not defined for it")
+        if inpaint:
+            if init_images is None:
+                raise RuntimeError("mask_images without init_images: inpainting repaints part of a given picture")
+            strength = 1.0 if strength is None else float(strength)
+            self.require_encoder()
+            if tuple(init_images.shape) != (B, 8 * h, 8 * w, 3) or init_images.dtype != torch.uint8:
+                raise RuntimeError(f"init_images: u8 [{B}, {8 * h}, {8 * w}, 3] expected, got "
+                                   f"{init_images.dtype} {list(init_images.shape)}")
+            if tuple(mask_images.shape) != (B, 8 * h, 8 * w) or mask_images.dtype != torch.uint8:
+                raise RuntimeError(f"mask_images: u8 [{B}, {8 * h}, {8 * w}] expected, got "
+                                   f"{mask_images.dtype} {list(mask_images.shape)}")
+            k = len(LCMSchedule(steps, strength, truncate=True).timesteps)     # ValueError when no step remains
+            if (not nine or strength < 1.0) and (posterior_noise is None or
+                                                 tuple(posterior_noise.shape) != (B, 4, h, w)):
+                raise RuntimeError(f"inpainting needs posterior_noise [{B}, 4, {h}, {w}] (the image's posterior draw)")
+            if nine and (masked_posterior_noise is None or tuple(masked_posterior_noise.shape) != (B, 4, h, w)):
+                raise RuntimeError(f"inpainting with a 9-channel UNet needs masked_posterior_noise [{B}, 4, {h}, {w}]")
+        elif init_images is not None:
             strength = 0.8 if strength is None else float(strength)
             if not self.unet.cfg.time_cond_proj_dim:
                 raise RuntimeError("image-to-image is implemented for LCM UNets (time_cond_proj_dim) only: the LCM "
@@ -1102,13 +1237,14 @@ class LCMPipelineB200:
                     return torch.cat([t] + [t[tuple(idx)]] * (Bp - B), dim)
                 gs = torch.as_tensor(guidance_scale, dtype=torch.float32).reshape(-1)
                 out = self.generate(pad(prompt_embeds), pad(latents_nchw),
-                                    pad(step_noise_nchw, 1) if steps > 1 else step_noise_nchw, steps,
+                                    pad(step_noise_nchw, 1) if k > 1 else step_noise_nchw, steps,
                                     pad(gs) if gs.numel() > 1 else guidance_scale, return_latents=True, use_graph=True,
                                     pooled_embeds=pad(pooled_embeds), time_ids=pad(time_ids),
                                     negative_prompt_embeds=pad(negative_prompt_embeds),
                                     negative_pooled_embeds=pad(negative_pooled_embeds), decode=decode,
                                     init_images=pad(init_images), strength=strength,
-                                    posterior_noise=pad(posterior_noise))
+                                    posterior_noise=pad(posterior_noise), mask_images=pad(mask_images),
+                                    masked_posterior_noise=pad(masked_posterior_noise))
                 img, lat = out
                 img = img[:B] if img is not None else None
                 return (img, lat[:B]) if return_latents else img
@@ -1118,7 +1254,7 @@ class LCMPipelineB200:
                                          negative_pooled_embeds, cfg_scale, 8 * h, 8 * w)
         with torch.cuda.device(self.device):
             if use_graph and record is None and teacher_latents is None:
-                g = self.graph_for(B, h, w, steps, cfg_scale, decode, strength)
+                g = self.graph_for(B, h, w, steps, cfg_scale, decode, strength, inpaint)
                 # host inputs go through pinned staging: a copy from PAGEABLE host memory first waits for the stream to
                 # drain (CUDA's documented behaviour), i.e. for the previous batch — the thread could then not enqueue
                 # this batch behind it
@@ -1129,11 +1265,16 @@ class LCMPipelineB200:
                     g.add[0].copy_(_pinned(add[0]), non_blocking=True)
                     g.add[1].copy_(_pinned(add[1]), non_blocking=True)
                 g.lat.copy_(_pinned(latents_nchw), non_blocking=True)
-                if steps > 1:
+                if k > 1:
                     g.noise.copy_(_pinned(step_noise_nchw), non_blocking=True)
                 if strength is not None:
                     g.init_u8.copy_(_pinned(init_images), non_blocking=True)
-                    g.eps_s.copy_(_pinned(posterior_noise), non_blocking=True)
+                    if posterior_noise is not None:
+                        g.eps_s.copy_(_pinned(posterior_noise), non_blocking=True)
+                if inpaint:
+                    g.mask_u8.copy_(_pinned(mask_images), non_blocking=True)
+                    if masked_posterior_noise is not None:
+                        g.eps_m.copy_(_pinned(masked_posterior_noise), non_blocking=True)
                 g.graph.replay()
                 img, lat = g.img, g.final
             else:
@@ -1143,12 +1284,17 @@ class LCMPipelineB200:
                     add = (add[0].to(self.device), add[1].to(self.device))
                 lat0 = latents_nchw.to(self.device, torch.float32).contiguous()
                 nz = (step_noise_nchw.to(self.device, torch.float32).contiguous()
-                      if steps > 1 else None)
-                init = eps = None
+                      if k > 1 else None)
+                init = eps = mask = eps_m = None
                 if strength is not None:
                     init = init_images.to(self.device).contiguous()
-                    eps = posterior_noise.to(self.device, torch.float32).contiguous()
+                    if posterior_noise is not None:
+                        eps = posterior_noise.to(self.device, torch.float32).contiguous()
+                if inpaint:
+                    mask = mask_images.to(self.device).contiguous()
+                    if masked_posterior_noise is not None:
+                        eps_m = masked_posterior_noise.to(self.device, torch.float32).contiguous()
                 img, lat = self.run_static(pe, we, lat0, nz, steps, record, add=add, cfg_scale=cfg_scale,
                                            teacher=teacher_latents, decode=decode, init_u8=init, eps_s=eps,
-                                           strength=strength)
+                                           strength=strength, mask_u8=mask, eps_m=eps_m)
         return (img, lat) if return_latents else img

@@ -30,7 +30,8 @@ EXPORTS = [
     "dl_im2col_s2_f32", "dl_softmax_rows_f32", "dl_small_linear_f32",
     "dl_png_stored_size", "dl_png_stored_workspace_bytes", "dl_png_stored", "dl_conv_tapsum",
     "dl_im2col_s2_pad01", "dl_im2col_s2_pad01_f32", "dl_pack_image_im2col", "dl_pack_image_im2col_f32",
-    "dl_vae_sample_latents",
+    "dl_vae_sample_latents", "dl_pack_image_im2col_masked", "dl_pack_image_im2col_masked_f32",
+    "dl_inpaint_latent_mask", "dl_pack_latent_inpaint", "dl_pack_latent_inpaint_f32", "dl_lcm_step_inpaint",
 ]
 
 
@@ -167,6 +168,15 @@ def load() -> C.CDLL:
             lib.dl_vae_sample_latents.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int,
                                                   C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_void_p,
                                                   C.c_void_p]
+            for f in (lib.dl_pack_image_im2col_masked, lib.dl_pack_image_im2col_masked_f32):
+                f.argtypes = [C.c_void_p, C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_longlong, C.c_longlong,
+                              C.c_longlong, C.c_longlong, C.c_void_p, C.c_void_p]
+            lib.dl_inpaint_latent_mask.argtypes = [C.c_void_p, C.c_int, C.c_int, C.c_int, C.c_void_p, C.c_void_p]
+            for f in (lib.dl_pack_latent_inpaint, lib.dl_pack_latent_inpaint_f32):
+                f.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong, C.c_int, C.c_void_p, C.c_void_p]
+            lib.dl_lcm_step_inpaint.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong,
+                                                C.POINTER(LcmCoeffs), C.c_float, C.c_float, C.c_int, C.c_void_p]
             lib.dl_png_stored_size.restype = C.c_longlong
             lib.dl_png_stored_size.argtypes = [C.c_int, C.c_int]
             lib.dl_png_stored_workspace_bytes.restype = C.c_longlong
@@ -533,16 +543,59 @@ def im2col_s2_pad01(x, cols, *, nimg, h, w):
     _count()
 
 
-def pack_image_im2col(img, out):
+def pack_image_im2col(img, out, mask=None):
     """img: u8 [n,h,w,3] (a view with unit channel and 3-byte pixel stride: a tile window of a canvas is fine);
-    out: bf16 or fp32 [n*h*w, 64] conv_in im2col operand (K = tap*3 + c, zero padded)."""
+    out: bf16 or fp32 [n*h*w, 64] conv_in im2col operand (K = tap*3 + c, zero padded).
+    mask (inpainting): u8 [n,h,w] with unit pixel stride (a window too); pixels with m >= 128 read as 0.0."""
     n, h, w, c = img.shape
     if c != 3 or img.dtype != torch.uint8 or img.stride(3) != 1 or img.stride(2) != 3:
         raise RuntimeError("pack_image_im2col: u8 [n,h,w,3] with packed RGB pixels expected")
-    fn = load().dl_pack_image_im2col_f32 if out.dtype == torch.float32 else load().dl_pack_image_im2col
-    with _timed("pack_image_im2col", 0.0, float(img.numel()) + out.element_size() * out.numel()):
-        _check(fn(img.data_ptr(), n, h, w, img.stride(1), img.stride(0), out.data_ptr(), _stream()),
-               "pack_image_im2col")
+    nbytes = float(img.numel()) + out.element_size() * out.numel()
+    if mask is None:
+        fn = load().dl_pack_image_im2col_f32 if out.dtype == torch.float32 else load().dl_pack_image_im2col
+        with _timed("pack_image_im2col", 0.0, nbytes):
+            _check(fn(img.data_ptr(), n, h, w, img.stride(1), img.stride(0), out.data_ptr(), _stream()),
+                   "pack_image_im2col")
+        _count()
+        return
+    if tuple(mask.shape) != (n, h, w) or mask.dtype != torch.uint8 or mask.stride(2) != 1:
+        raise RuntimeError(f"pack_image_im2col: mask u8 [{n},{h},{w}] with unit pixel stride expected")
+    fn = load().dl_pack_image_im2col_masked_f32 if out.dtype == torch.float32 else load().dl_pack_image_im2col_masked
+    with _timed("pack_image_im2col_masked", 0.0, nbytes + mask.numel()):
+        _check(fn(img.data_ptr(), mask.data_ptr(), n, h, w, img.stride(1), img.stride(0), mask.stride(1),
+                  mask.stride(0), out.data_ptr(), _stream()), "pack_image_im2col_masked")
+    _count()
+
+
+def inpaint_latent_mask(mask, out):
+    """mask u8 [n, 8h, 8w] (contiguous) -> out fp32 [n, h, w]: the binarised pixel (8i, 8j) of each latent."""
+    n, h, w = out.shape
+    if tuple(mask.shape) != (n, 8 * h, 8 * w) or mask.dtype != torch.uint8 or not mask.is_contiguous():
+        raise RuntimeError(f"inpaint_latent_mask: contiguous u8 [{n},{8 * h},{8 * w}] expected")
+    _check(load().dl_inpaint_latent_mask(mask.data_ptr(), n, h, w, out.data_ptr(), _stream()), "inpaint_latent_mask")
+    _count()
+
+
+def pack_latent_inpaint(latents, mask, masked, out, repeat=1):
+    """latents / masked fp32 NHWC [n,h,w,4], mask fp32 [n,h,w] -> out bf16 or fp32 [repeat*n, h, w, 64]:
+    [latents | mask | masked | 0...], the n images written `repeat` times."""
+    npix = mask.numel()
+    if latents.numel() != 4 * npix or masked.numel() != 4 * npix or out.numel() != 64 * npix * repeat:
+        raise RuntimeError("pack_latent_inpaint: shapes do not match")
+    fn = load().dl_pack_latent_inpaint_f32 if out.dtype == torch.float32 else load().dl_pack_latent_inpaint
+    _check(fn(latents.data_ptr(), mask.data_ptr(), masked.data_ptr(), npix, repeat, out.data_ptr(), _stream()),
+           "pack_latent_inpaint")
+    _count()
+
+
+def lcm_step_inpaint(eps, x, noise, image_latents, noise0, mask, x_next, denoised, coeffs, add_noise, last):
+    """`lcm_step` + the 4-channel UNet's blend; add_noise = (sqrt_alpha, sqrt_one_minus_alpha) of the next timestep
+    (ignored on the last step, where the blend target is image_latents itself)."""
+    k = LcmCoeffs(*[float(v) for v in coeffs])
+    _check(load().dl_lcm_step_inpaint(eps.data_ptr(), x.data_ptr(), _ptr(noise), image_latents.data_ptr(),
+                                      _ptr(noise0), mask.data_ptr(), x_next.data_ptr(), denoised.data_ptr(),
+                                      mask.numel(), C.byref(k), float(add_noise[0]), float(add_noise[1]), int(last),
+                                      _stream()), "lcm_step_inpaint")
     _count()
 
 

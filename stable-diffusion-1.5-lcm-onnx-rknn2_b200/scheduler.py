@@ -50,16 +50,35 @@ def lcm_timesteps(num_inference_steps: int, strength: float = 1.0) -> List[int]:
 
 
 class LCMSchedule:
-    """Timesteps + per-step coefficient tuples for `lib.lcm_step`."""
+    """Timesteps + per-step coefficient tuples for `lib.lcm_step`.
 
-    def __init__(self, num_inference_steps: int, strength: float = 1.0):
+    truncate=True (inpainting, `StableDiffusionInpaintPipeline.get_timesteps`): the full n-step schedule of
+    `set_timesteps(n)`, of which only the tail from t_start = n - min(int(n * strength), n) runs
+    (`set_begin_index(t_start)`).  Step i then uses the coefficients of full index t_start + i with
+    prev_t = full[t_start + i + 1], i.e. those of the tail itself, and no noise is drawn at full index n - 1.
+    Otherwise strength re-spaces the schedule (`set_timesteps(n, strength)`, image-to-image)."""
+
+    def __init__(self, num_inference_steps: int, strength: float = 1.0, truncate: bool = False):
         self.num_inference_steps = num_inference_steps
         self.strength = strength
-        self.timesteps = lcm_timesteps(num_inference_steps, strength)
+        self.begin_index = 0
+        if truncate:
+            if not 0.0 < strength <= 1.0:
+                raise ValueError(f"strength must be in (0, 1], got {strength}")
+            full = lcm_timesteps(num_inference_steps)
+            init_timestep = min(int(num_inference_steps * strength), num_inference_steps)
+            self.begin_index = max(num_inference_steps - init_timestep, 0)
+            self.timesteps = full[self.begin_index:]
+            if len(self.timesteps) < 1:
+                raise ValueError(f"strength {strength} leaves no step of num_inference_steps={num_inference_steps} "
+                                 f"(int(n * strength) = 0)")
+        else:
+            self.timesteps = lcm_timesteps(num_inference_steps, strength)
         ac = alphas_cumprod()
         self._coeffs: List[Tuple[float, ...]] = []
+        n = len(self.timesteps)
         for i, t in enumerate(self.timesteps):
-            prev_t = self.timesteps[i + 1] if i + 1 < num_inference_steps else t
+            prev_t = self.timesteps[i + 1] if i + 1 < n else t
             a_t, a_prev = ac[t], ac[prev_t]
             s = torch.as_tensor(t, dtype=torch.int64) * TIMESTEP_SCALING       # fp32 0-dim
             c_skip = SIGMA_DATA ** 2 / (s ** 2 + SIGMA_DATA ** 2)
@@ -67,16 +86,16 @@ class LCMSchedule:
             self._coeffs.append((a_t.sqrt().item(), (1 - a_t).sqrt().item(), c_skip.item(),
                                  c_out.item(), a_prev.sqrt().item(), (1 - a_prev).sqrt().item()))
 
-    def add_noise_coeffs(self) -> Tuple[float, float]:
-        """`LCMScheduler.add_noise` at t0 = timesteps[0]: fp32 (sqrt(ac[t0]), sqrt(1 - ac[t0])) as `** 0.5`."""
-        a = alphas_cumprod()[self.timesteps[0]]
+    def add_noise_coeffs(self, t: int = None) -> Tuple[float, float]:
+        """`LCMScheduler.add_noise` at t (default t0 = timesteps[0]): fp32 (sqrt(ac[t]), sqrt(1 - ac[t])) as `** 0.5`."""
+        a = alphas_cumprod()[self.timesteps[0] if t is None else t]
         return (a ** 0.5).item(), ((1 - a) ** 0.5).item()
 
     def coeffs(self, i: int) -> Tuple[float, ...]:
         return self._coeffs[i]
 
     def has_noise(self, i: int) -> bool:
-        return i != self.num_inference_steps - 1
+        return i != len(self.timesteps) - 1
 
 
 def guidance_scale_embedding(w: torch.Tensor, embedding_dim: int = 256) -> torch.Tensor:

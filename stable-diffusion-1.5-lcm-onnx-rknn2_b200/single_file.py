@@ -247,6 +247,7 @@ def load_single_file(path: str) -> dict:
         ucfg["time_cond_proj_dim"] = sd[UNET_PREFIX + "time_embed.cond_proj.weight"].shape[1]
     probe = next(k for k in sorted(sd) if k.startswith(UNET_PREFIX) and k.endswith("attn2.to_k.weight"))
     ucfg["cross_attention_dim"] = sd[probe].shape[1]
+    ucfg["in_channels"] = sd[UNET_PREFIX + "input_blocks.0.0.weight"].shape[1]     # 9: an inpainting UNet
     vcfg = dict(SDXL_VAE if sdxl else SD_VAE)
     out = {"unet": (ucfg, convert_unet(sd, ucfg)),
            "vae": (vcfg, {**convert_vae_decoder(sd, vcfg), **convert_vae_encoder(sd, vcfg)}),
