@@ -275,30 +275,17 @@ def test_attention_x_short_keys(B, Sq, Skv, heads, d):
     (1, 512, 512, 2, 40), (2, 1024, 1024, 3, 40), (1, 300, 600, 2, 40), (1, 4096, 4096, 1, 40),
     (1, 768, 1000, 2, 56), (1, 512, 640, 2, 48), (2, 9216, 9216, 1, 40),
 ])
-@pytest.mark.parametrize("poly", ["0", "3"])
-def test_attention_pp_two_query_tiles(B, Sq, Skv, heads, d, poly):
-    _attention_pp_case(B, Sq, Skv, heads, d, poly)
-
-
-def _attention_pp_case(B, Sq, Skv, heads, d, poly):
-    """attention_pp.cu (256 queries per CTA, one softmax thread per row, P in its own TMEM columns):
-    ragged key tiles, query counts that are not a multiple of 256, both K-step variants, all-MUFU and
-    3/8-polynomial exponentials; and the same inputs through the older kernel agree with it."""
-    import subprocess, sys, os
-    e1 = _attn_case(L(), B, Sq, Skv, heads, d, 0, v_ones=True)
-    assert e1 < 2e-2, f"rel err {e1}"
-    e2 = _attn_case(L(), B, Sq, Skv, heads, d, 0, v_ones=True, qscale=6.0, seed=7)
-    assert e2 < 2e-2, f"rel err (peaked rows) {e2}"
-    if poly == "0":
-        # the env knobs are read once per process: check the all-MUFU variant in a child
-        code = ("import sys; sys.path.insert(0, %r); sys.path.insert(0, %r); import test_kernels_gpu as t; "
-                "e = t._attn_case(t.L(), %d, %d, %d, %d, %d, 0, v_ones=True); assert e < 2e-2, e; print(e)"
-                % (os.path.dirname(os.path.dirname(os.path.abspath(__file__))), os.path.dirname(os.path.abspath(__file__)),
-                   B, Sq, Skv, heads, d))
-        # ... with two query tiles per CTA (the default is one tile per CTA, two CTAs per SM)
-        env = dict(os.environ, DL_ATTN_PP_POLY="0", DL_ATTN_PP_NQ="2")
-        r = subprocess.run([sys.executable, "-c", code], env=env, capture_output=True, text=True, timeout=300)
-        assert r.returncode == 0, r.stdout + r.stderr
+@pytest.mark.parametrize("inputs", ["random", "peaked"])
+def test_attention_pp_two_query_tiles(B, Sq, Skv, heads, d, inputs):
+    """attention_pp.cu (one softmax thread per row, P in its own TMEM columns) on the default path: ragged key
+    tiles, query counts that are not a multiple of 256, both K-step variants; random and peaked rows (the running
+    max moves and O is rescaled).  The variants of the DL_ATTN_PP_POLY / DL_ATTN_PP_NQ knobs are checked in
+    test_attention_edges_gpu.py::test_attention_knob_variants."""
+    if inputs == "random":
+        e = _attn_case(L(), B, Sq, Skv, heads, d, 0, v_ones=True)
+    else:
+        e = _attn_case(L(), B, Sq, Skv, heads, d, 0, v_ones=True, qscale=6.0, seed=7)
+    assert e < 2e-2, f"rel err ({inputs}) {e}"
 
 
 @pytest.mark.parametrize("B,Sq,Skv,d", [

@@ -1,4 +1,4 @@
-"""`poly_exp2` (csrc/common.cuh) — the MUFU-free 2^x the attention kernel uses for a quarter of its
+"""`poly_exp2` (csrc/common.cuh) — the MUFU-free 2^x the attention kernels use for a quarter of their
 exponentials.  The constants are read out of the CUDA source and the same float32 / int32
 arithmetic is evaluated with numpy, so a changed coefficient or clamp is caught on the CPU."""
 import os
@@ -20,6 +20,26 @@ def _constants():
     c1, c0 = [float(m) for m in re.findall(r"fmaf\(p, f, ([0-9.eE+-]+)f\)", body)]
     assert "<< 23" in body
     return clamp, magic, (c0, c1, c2, c3)
+
+
+def _packed_constants():
+    """The same constants from the packed (f32x2) copy that attn_pp_kernel (csrc/attention_pp.cu, the SD1.5 head
+    dim 40 path) inlines: clamp, rounding constant, -1 of the Cody-Waite step and the four coefficients, each pair
+    with the same value in both lanes."""
+    src = open(os.path.join(os.path.dirname(SRC), "attention_pp.cu")).read()
+    body = src[src.index("packed 2^x on the FMA / ALU pipes"):]
+    body = body[:body.index("} else {")]
+    clamps = {float(v) for v in re.findall(r"fmaxf\(x[01], (-?[0-9.]+)f\)", body)}
+    assert len(clamps) == 1, clamps
+    pairs = re.findall(r"f2_pack\((-?[0-9.eE+-]+)f, (-?[0-9.eE+-]+)f\)", body)
+    assert all(a == b for a, b in pairs), pairs
+    vals = [float(a) for a, _ in pairs]
+    # r = x + magic, t = r - magic, f = t * -1 + x, then c3 * f + c2, * f + c1, * f + c0
+    assert len(vals) == 7, vals
+    magic, neg_magic, neg_one, c3, c2, c1, c0 = vals
+    assert neg_magic == -magic and neg_one == -1.0, vals
+    assert "<< 23" in body
+    return clamps.pop(), magic, (c0, c1, c2, c3)
 
 
 def _poly_exp2(x, clamp, magic, c):
@@ -58,3 +78,8 @@ def test_poly_exp2_edge_cases():
     assert abs(y[8] - 256.0) < 256 * 1e-4
     # the row maximum gets P = 1.0 exactly after the bf16 rounding (8 mantissa bits)
     assert np.float32(y[3]).view(np.uint32) + 0x8000 >> 16 == 0x3F80
+
+
+def test_attn_pp_packed_copy_matches_common():
+    """attn_pp_kernel's inlined packed 2^x must be the polynomial pinned above, constant for constant."""
+    assert _packed_constants() == _constants()
