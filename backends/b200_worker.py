@@ -141,6 +141,11 @@ class B200Worker(PipelineWorker):
         if not single and not (os.path.isdir(path) and os.path.exists(os.path.join(path, "model_index.json"))):
             raise RuntimeError(f"b200 worker needs a diffusers-layout model directory or a single-file "
                                f".safetensors checkpoint, got: {path}")
+        # `LCMScheduler.from_config(pipe.scheduler.config)` (reference `backends/cuda_worker.py:88`, `:387`): the
+        # model's scheduler/scheduler_config.json (prediction type, beta schedule, ...); a single-file checkpoint
+        # carries none and keeps the defaults.  A config this engine cannot serve is refused here, naming the key.
+        from dreamlab_b200.scheduler import SchedulerConfig
+        self.scheduler_config = SchedulerConfig.load(None if single else path)
         if not torch.cuda.is_available():
             raise RuntimeError("b200 worker needs a CUDA device (sm_100a); there is no CPU fallback")
 
@@ -176,7 +181,7 @@ class B200Worker(PipelineWorker):
         vcfg = taesd_cfg_from_json(vcfg_json) if vae_kind == "taesd" else vae_cfg_from_json(vcfg_json)
         self.pipe = LCMPipelineB200(unet_sd, unet_cfg_from_json(ucfg_json), vae_sd, vcfg, self.device,
                                     vae_tiling=True, precision="fp32" if dtype_str == "fp32" else "bf16",
-                                    vae_kind=vae_kind)
+                                    vae_kind=vae_kind, scheduler_config=self.scheduler_config)
         self._text = self._make_text_encoder(path)
         self._single = None                               # the converted state dicts are packed: drop the copies
         # the attributes the reference's worker tests look for on `pipe` (`tests/test_sdxl_worker.py:127-130`)

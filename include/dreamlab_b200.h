@@ -217,6 +217,24 @@ typedef struct dl_lcm_coeffs {
 } dl_lcm_coeffs;
 int dl_lcm_step(const float* eps, const float* x, const float* noise, float* x_next,
                 float* denoised, long long n, const dl_lcm_coeffs* coeffs /* host */, void* stream);
+/* dl_lcm_step_ex: the step of a model whose scheduler config sets prediction_type / clip_sample
+ * (`LCMScheduler.from_config(model config)`).  x0 from the model output mo, in diffusers' op order:
+ *   DL_PRED_EPSILON  x0 = (x - sqrt(1-a_t) mo)/sqrt(a_t)     (= dl_lcm_step, bit for bit)
+ *   DL_PRED_V        x0 = sqrt(a_t) x - sqrt(1-a_t) mo        (v_prediction)
+ *   DL_PRED_SAMPLE   x0 = mo
+ * then, with clip_sample != 0, x0 = clamp(x0, -clip_sample_range, clip_sample_range); the rest as
+ * dl_lcm_step.  Every mul / sub / div rounded on its own.                                        */
+#define DL_PRED_EPSILON 0
+#define DL_PRED_V 1
+#define DL_PRED_SAMPLE 2
+typedef struct dl_lcm_coeffs_ex {
+  dl_lcm_coeffs k;
+  int prediction_type;      /* DL_PRED_* */
+  int clip_sample;
+  float clip_sample_range;
+} dl_lcm_coeffs_ex;
+int dl_lcm_step_ex(const float* model_output, const float* x, const float* noise, float* x_next,
+                   float* denoised, long long n, const dl_lcm_coeffs_ex* coeffs /* host */, void* stream);
 
 /* ---- CLIP text tower pieces (the step before the hot path: diffusers `encode_prompt` ->
  * transformers CLIPTextModel; SURVEY.md §8f rank 2) ------------------------------------------------
@@ -352,6 +370,11 @@ int dl_lcm_step_inpaint(const float* eps, const float* x, const float* noise, co
                         const float* noise0, const float* mask, float* x_next, float* denoised, long long npix,
                         const dl_lcm_coeffs* k, float sqrt_alpha, float sqrt_one_minus_alpha, int last,
                         void* stream);
+/* dl_lcm_step_inpaint_ex: dl_lcm_step_inpaint with the x0 of dl_lcm_step_ex (prediction type, clamp).        */
+int dl_lcm_step_inpaint_ex(const float* model_output, const float* x, const float* noise,
+                           const float* image_latents, const float* noise0, const float* mask, float* x_next,
+                           float* denoised, long long npix, const dl_lcm_coeffs_ex* k, float sqrt_alpha,
+                           float sqrt_one_minus_alpha, int last, void* stream);
 
 /* ---- tiny autoencoder (diffusers AutoencoderTiny / TAESD) decoder input -------------------------------------------
  * latents fp32 NHWC [npix, 4] -> the 64-channel operand of the decoder's first conv, bf16 (or fp32 for _f32)

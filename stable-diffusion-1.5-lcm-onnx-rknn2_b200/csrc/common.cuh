@@ -7,6 +7,8 @@
 #include <stdint.h>
 #include <stdio.h>
 
+#include "dreamlab_b200.h"
+
 namespace dl {
 
 // ----------------------------------------------------------------------------------------------
@@ -385,6 +387,24 @@ __device__ __forceinline__ float warp_max(float v) {
 #pragma unroll
   for (int o = 16; o > 0; o >>= 1) v = fmaxf(v, __shfl_xor_sync(0xffffffffu, v, o));
   return v;
+}
+
+// LCMScheduler.step's predicted_original_sample from the model output mo (DL_PRED_*), each mul / sub / div rounded
+// on its own as the fp32 torch ops are, then `clip_sample`'s clamp to [-r, r].
+template <int PRED>
+__device__ __forceinline__ float lcm_x0(float mo, float x, float sqrt_alpha_t, float sqrt_beta_t, int clip,
+                                        float r) {
+  static_assert(PRED == DL_PRED_EPSILON || PRED == DL_PRED_V || PRED == DL_PRED_SAMPLE, "prediction type");
+  float x0;
+  if constexpr (PRED == DL_PRED_EPSILON) {
+    x0 = __fdiv_rn(__fsub_rn(x, __fmul_rn(sqrt_beta_t, mo)), sqrt_alpha_t);
+  } else if constexpr (PRED == DL_PRED_V) {
+    x0 = __fsub_rn(__fmul_rn(sqrt_alpha_t, x), __fmul_rn(sqrt_beta_t, mo));
+  } else {
+    x0 = mo;
+  }
+  if (clip) x0 = fminf(fmaxf(x0, -r), r);
+  return x0;
 }
 
 #endif  // __CUDACC__

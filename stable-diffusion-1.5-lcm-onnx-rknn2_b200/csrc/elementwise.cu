@@ -218,9 +218,11 @@ __global__ void nhwc_to_nchw_kernel(const float* __restrict__ x, int nimg, int c
 }
 
 // ---- LCMScheduler.step, fused (fp32 latents; coefficients are the scheduler's fp32 scalars) ---
+// PRED (DL_PRED_*) picks how x0 follows from the model output (lcm_x0 in common.cuh); clip: clamp x0 to [-r, r].
+template <int PRED>
 __global__ void lcm_step_kernel(const float4* __restrict__ eps, const float4* __restrict__ x,
                                 const float4* __restrict__ noise, float4* __restrict__ x_next,
-                                float4* __restrict__ denoised, long long n4, dl_lcm_coeffs k) {
+                                float4* __restrict__ denoised, long long n4, dl_lcm_coeffs k, int clip, float r) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
        i += (long long)gridDim.x * blockDim.x) {
     const float4 e = eps[i], xv = x[i];
@@ -234,8 +236,8 @@ __global__ void lcm_step_kernel(const float4* __restrict__ eps, const float4* __
     float d[4], o[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      // no FMA contraction: keep the reference's op order (mul, sub, div, mul, mul, add)
-      const float x0 = __fdiv_rn(__fsub_rn(xx[j], __fmul_rn(k.sqrt_beta_t, ev[j])), k.sqrt_alpha_t);
+      // no FMA contraction: keep the reference's op order (x0, then mul, mul, add)
+      const float x0 = lcm_x0<PRED>(ev[j], xx[j], k.sqrt_alpha_t, k.sqrt_beta_t, clip, r);
       d[j] = __fadd_rn(__fmul_rn(k.c_out, x0), __fmul_rn(k.c_skip, xx[j]));
       o[j] = (noise != nullptr)
                  ? __fadd_rn(__fmul_rn(k.sqrt_alpha_prev, d[j]), __fmul_rn(k.sqrt_beta_prev, zz[j]))
@@ -578,11 +580,42 @@ extern "C" int dl_lcm_step(const float* eps, const float* x, const float* noise,
                            float* denoised, long long n, const dl_lcm_coeffs* k, void* stream_) {
   DL_CHECK_ARG(eps && x && x_next && denoised && k, "lcm_step: null pointer");
   DL_CHECK_ARG(n % 4 == 0, "lcm_step: n must be a multiple of 4");
-  lcm_step_kernel<<<grid_for(n / 4, 256), 256, 0, STREAM>>>(
+  lcm_step_kernel<DL_PRED_EPSILON><<<grid_for(n / 4, 256), 256, 0, STREAM>>>(
       reinterpret_cast<const float4*>(eps), reinterpret_cast<const float4*>(x),
       reinterpret_cast<const float4*>(noise), reinterpret_cast<float4*>(x_next),
-      reinterpret_cast<float4*>(denoised), n / 4, *k);
+      reinterpret_cast<float4*>(denoised), n / 4, *k, 0, 0.f);
   return check_launch("lcm_step");
+}
+
+extern "C" int dl_lcm_step_ex(const float* mo, const float* x, const float* noise, float* x_next,
+                              float* denoised, long long n, const dl_lcm_coeffs_ex* k, void* stream_) {
+  DL_CHECK_ARG(mo && x && x_next && denoised && k, "lcm_step_ex: null pointer");
+  DL_CHECK_ARG(n % 4 == 0, "lcm_step_ex: n must be a multiple of 4");
+  DL_CHECK_ARG(!k->clip_sample || k->clip_sample_range >= 0.f, "lcm_step_ex: clip_sample_range must be >= 0");
+  const unsigned grid = grid_for(n / 4, 256);
+  const float4* m4 = reinterpret_cast<const float4*>(mo);
+  const float4* x4 = reinterpret_cast<const float4*>(x);
+  const float4* z4 = reinterpret_cast<const float4*>(noise);
+  float4* o4 = reinterpret_cast<float4*>(x_next);
+  float4* d4 = reinterpret_cast<float4*>(denoised);
+  const int clip = k->clip_sample != 0;
+  switch (k->prediction_type) {
+    case DL_PRED_EPSILON:
+      lcm_step_kernel<DL_PRED_EPSILON><<<grid, 256, 0, STREAM>>>(m4, x4, z4, o4, d4, n / 4, k->k, clip,
+                                                                  k->clip_sample_range);
+      break;
+    case DL_PRED_V:
+      lcm_step_kernel<DL_PRED_V><<<grid, 256, 0, STREAM>>>(m4, x4, z4, o4, d4, n / 4, k->k, clip,
+                                                            k->clip_sample_range);
+      break;
+    case DL_PRED_SAMPLE:
+      lcm_step_kernel<DL_PRED_SAMPLE><<<grid, 256, 0, STREAM>>>(m4, x4, z4, o4, d4, n / 4, k->k, clip,
+                                                                 k->clip_sample_range);
+      break;
+    default:
+      DL_CHECK_ARG(false, "lcm_step_ex: unknown prediction_type");
+  }
+  return check_launch("lcm_step_ex");
 }
 
 extern "C" int dl_embed_tokens(const long long* ids, const void* tok_emb, const void* pos_emb, int n, int seq,

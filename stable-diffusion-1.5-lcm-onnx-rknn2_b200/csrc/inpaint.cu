@@ -56,15 +56,17 @@ __global__ void pack_latent_inpaint_kernel(const float* __restrict__ lat, const 
   }
 }
 
-// LCMScheduler.step (same op order as lcm_step_kernel), then the 4-channel UNet's blend:
+// LCMScheduler.step (same op order as lcm_step_kernel, x0 by PRED and the optional clamp), then the 4-channel UNet's
+// blend:
 //   proper = last ? image_latents : sqrt_a * image_latents + sqrt_b * noise0        (add_noise at timesteps[i+1])
 //   x_next = (1 - m) * proper + m * prev_sample
 // fp32 NHWC [.., 4] tensors as float4 (one pixel each), mask fp32 one value per pixel.
+template <int PRED>
 __global__ void lcm_step_inpaint_kernel(const float4* __restrict__ eps, const float4* __restrict__ x,
                                         const float4* __restrict__ noise, const float4* __restrict__ img,
                                         const float4* __restrict__ noise0, const float* __restrict__ mask,
                                         float4* __restrict__ x_next, float4* __restrict__ denoised, long long n4,
-                                        dl_lcm_coeffs k, float sqrt_a, float sqrt_b, int last) {
+                                        dl_lcm_coeffs k, float sqrt_a, float sqrt_b, int last, int clip, float r) {
   for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
        i += (long long)gridDim.x * blockDim.x) {
     const float4 e = eps[i], xv = x[i], iv = img[i];
@@ -85,7 +87,7 @@ __global__ void lcm_step_inpaint_kernel(const float4* __restrict__ eps, const fl
     float d[4], o[4];
 #pragma unroll
     for (int j = 0; j < 4; ++j) {
-      const float x0 = __fdiv_rn(__fsub_rn(xx[j], __fmul_rn(k.sqrt_beta_t, ev[j])), k.sqrt_alpha_t);
+      const float x0 = lcm_x0<PRED>(ev[j], xx[j], k.sqrt_alpha_t, k.sqrt_beta_t, clip, r);
       d[j] = __fadd_rn(__fmul_rn(k.c_out, x0), __fmul_rn(k.c_skip, xx[j]));
       const float prev = (noise != nullptr)
                              ? __fadd_rn(__fmul_rn(k.sqrt_alpha_prev, d[j]), __fmul_rn(k.sqrt_beta_prev, zz[j]))
@@ -143,10 +145,49 @@ extern "C" int dl_lcm_step_inpaint(const float* eps, const float* x, const float
                                    int last, void* stream_) {
   DL_CHECK_ARG(eps && x && image_latents && mask && x_next && denoised && k && npix > 0 && (last || noise0),
                "lcm_step_inpaint: bad args");
-  lcm_step_inpaint_kernel<<<inp_grid(npix, 256), 256, 0, STREAM>>>(
+  lcm_step_inpaint_kernel<DL_PRED_EPSILON><<<inp_grid(npix, 256), 256, 0, STREAM>>>(
       reinterpret_cast<const float4*>(eps), reinterpret_cast<const float4*>(x),
       reinterpret_cast<const float4*>(noise), reinterpret_cast<const float4*>(image_latents),
       reinterpret_cast<const float4*>(noise0), mask, reinterpret_cast<float4*>(x_next),
-      reinterpret_cast<float4*>(denoised), npix, *k, sqrt_alpha, sqrt_one_minus_alpha, last);
+      reinterpret_cast<float4*>(denoised), npix, *k, sqrt_alpha, sqrt_one_minus_alpha, last, 0, 0.f);
   return check_launch("lcm_step_inpaint");
+}
+
+extern "C" int dl_lcm_step_inpaint_ex(const float* mo, const float* x, const float* noise,
+                                      const float* image_latents, const float* noise0, const float* mask,
+                                      float* x_next, float* denoised, long long npix, const dl_lcm_coeffs_ex* k,
+                                      float sqrt_alpha, float sqrt_one_minus_alpha, int last, void* stream_) {
+  DL_CHECK_ARG(mo && x && image_latents && mask && x_next && denoised && k && npix > 0 && (last || noise0),
+               "lcm_step_inpaint_ex: bad args");
+  DL_CHECK_ARG(!k->clip_sample || k->clip_sample_range >= 0.f,
+               "lcm_step_inpaint_ex: clip_sample_range must be >= 0");
+  const unsigned grid = inp_grid(npix, 256);
+  const float4* m4 = reinterpret_cast<const float4*>(mo);
+  const float4* x4 = reinterpret_cast<const float4*>(x);
+  const float4* z4 = reinterpret_cast<const float4*>(noise);
+  const float4* i4 = reinterpret_cast<const float4*>(image_latents);
+  const float4* z04 = reinterpret_cast<const float4*>(noise0);
+  float4* o4 = reinterpret_cast<float4*>(x_next);
+  float4* d4 = reinterpret_cast<float4*>(denoised);
+  const int clip = k->clip_sample != 0;
+  switch (k->prediction_type) {
+    case DL_PRED_EPSILON:
+      lcm_step_inpaint_kernel<DL_PRED_EPSILON><<<grid, 256, 0, STREAM>>>(
+          m4, x4, z4, i4, z04, mask, o4, d4, npix, k->k, sqrt_alpha, sqrt_one_minus_alpha, last, clip,
+          k->clip_sample_range);
+      break;
+    case DL_PRED_V:
+      lcm_step_inpaint_kernel<DL_PRED_V><<<grid, 256, 0, STREAM>>>(
+          m4, x4, z4, i4, z04, mask, o4, d4, npix, k->k, sqrt_alpha, sqrt_one_minus_alpha, last, clip,
+          k->clip_sample_range);
+      break;
+    case DL_PRED_SAMPLE:
+      lcm_step_inpaint_kernel<DL_PRED_SAMPLE><<<grid, 256, 0, STREAM>>>(
+          m4, x4, z4, i4, z04, mask, o4, d4, npix, k->k, sqrt_alpha, sqrt_one_minus_alpha, last, clip,
+          k->clip_sample_range);
+      break;
+    default:
+      DL_CHECK_ARG(false, "lcm_step_inpaint_ex: unknown prediction_type");
+  }
+  return check_launch("lcm_step_inpaint_ex");
 }

@@ -20,7 +20,7 @@ from typing import List, Optional
 import torch
 
 from . import lib
-from .scheduler import LCMSchedule, guidance_scale_embedding
+from .scheduler import DEFAULT_CONFIG, LCMSchedule, SchedulerConfig, guidance_scale_embedding
 from .weights import Packed, has_vae_encoder, pack_taesd_decoder, pack_unet, pack_vae_decoder, pack_vae_encoder
 
 BF16 = torch.bfloat16
@@ -993,12 +993,16 @@ class LCMPipelineB200:
     `backends/cuda_worker.py:532`) share this loop."""
 
     def __init__(self, unet_sd, unet_cfg, vae_sd, vae_cfg, device="cuda:0", vae_tiling: bool = False,
-                 precision: str = "bf16", vae_kind: str = "kl"):
+                 precision: str = "bf16", vae_kind: str = "kl", scheduler_config: SchedulerConfig = DEFAULT_CONFIG):
         """vae_tiling: `pipe.vae.enable_tiling()` (the reference workers always switch it on,
         `backends/cuda_worker.py:91`): requests larger than the VAE's sample_size decode tiled.
-        vae_kind: "kl" (`AutoencoderKL`) or "taesd" (`AutoencoderTiny`, decoder only, always untiled)."""
+        vae_kind: "kl" (`AutoencoderKL`) or "taesd" (`AutoencoderTiny`, decoder only, always untiled).
+        scheduler_config: `LCMScheduler.from_config(model's scheduler config)` (`SchedulerConfig.load`); it is fixed
+        for the pipeline, so its coefficients are baked into the captured graphs like the timesteps are."""
         if vae_kind not in ("kl", "taesd"):
             raise RuntimeError(f"vae_kind must be 'kl' or 'taesd', got {vae_kind!r}")
+        scheduler_config.validate()
+        self.scheduler_config = scheduler_config
         self.device = torch.device(device)
         self.precision = precision
         self.dt = _dt_of(precision)
@@ -1129,9 +1133,10 @@ class LCMPipelineB200:
     def schedule(self, steps: int, strength: Optional[float] = None, inpaint: bool = False) -> LCMSchedule:
         """The pass's schedule: text-to-image (strength None), image-to-image (re-spaced by strength) or
         inpainting (the full schedule truncated by strength)."""
+        cfg = self.scheduler_config
         if inpaint:
-            return LCMSchedule(steps, strength, truncate=True)
-        return LCMSchedule(steps) if strength is None else LCMSchedule(steps, strength)
+            return LCMSchedule(steps, strength, truncate=True, config=cfg)
+        return LCMSchedule(steps, config=cfg) if strength is None else LCMSchedule(steps, strength, config=cfg)
 
     def require_encoder(self) -> VAEEncoderB200:
         if self.vae_kind == "taesd":
@@ -1215,11 +1220,12 @@ class LCMPipelineB200:
                 # latents = (1 - m) * add_noise(image_latents, noise, timesteps[i + 1]) + m * latents; image_latents
                 # itself after the last step
                 last = i == n - 1
-                lib.lcm_step_inpaint(eps, x, z, blend[0], None if last else blend[1], blend[2], x_next, den,
-                                     sched.coeffs(i), (1.0, 0.0) if last else
-                                     sched.add_noise_coeffs(sched.timesteps[i + 1]), last)
+                lib.lcm_step_inpaint_ex(eps, x, z, blend[0], None if last else blend[1], blend[2], x_next, den,
+                                        sched.coeffs(i), (1.0, 0.0) if last else
+                                        sched.add_noise_coeffs(sched.timesteps[i + 1]), last,
+                                        sched.prediction_type, sched.clip_range)
             else:
-                lib.lcm_step(eps, x, z, x_next, den, sched.coeffs(i))
+                lib.lcm_step_ex(eps, x, z, x_next, den, sched.coeffs(i), sched.prediction_type, sched.clip_range)
             if record is not None:
                 record.setdefault("noise_pred", []).append(eps.permute(0, 3, 1, 2).clone())
                 record.setdefault("latents", []).append(x_next.permute(0, 3, 1, 2).clone())
@@ -1291,7 +1297,7 @@ class LCMPipelineB200:
             if tuple(mask_images.shape) != (B, 8 * h, 8 * w) or mask_images.dtype != torch.uint8:
                 raise RuntimeError(f"mask_images: u8 [{B}, {8 * h}, {8 * w}] expected, got "
                                    f"{mask_images.dtype} {list(mask_images.shape)}")
-            k = len(LCMSchedule(steps, strength, truncate=True).timesteps)     # ValueError when no step remains
+            k = len(self.schedule(steps, strength, inpaint=True).timesteps)     # ValueError when no step remains
             if (not nine or strength < 1.0) and (posterior_noise is None or
                                                  tuple(posterior_noise.shape) != (B, 4, h, w)):
                 raise RuntimeError(f"inpainting needs posterior_noise [{B}, 4, {h}, {w}] (the image's posterior draw)")
@@ -1308,7 +1314,7 @@ class LCMPipelineB200:
                                    f"{init_images.dtype} {list(init_images.shape)}")
             if posterior_noise is None or tuple(posterior_noise.shape) != (B, 4, h, w):
                 raise RuntimeError(f"image-to-image needs posterior_noise [{B}, 4, {h}, {w}]")
-            LCMSchedule(steps, strength)                  # ValueError for a strength the schedule cannot serve
+            self.schedule(steps, strength)                # ValueError for a strength the schedule cannot serve
         else:
             strength = None
         if use_graph and record is None and teacher_latents is None:

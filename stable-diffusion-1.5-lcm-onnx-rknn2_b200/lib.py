@@ -32,7 +32,7 @@ EXPORTS = [
     "dl_im2col_s2_pad01", "dl_im2col_s2_pad01_f32", "dl_pack_image_im2col", "dl_pack_image_im2col_f32",
     "dl_vae_sample_latents", "dl_pack_image_im2col_masked", "dl_pack_image_im2col_masked_f32",
     "dl_inpaint_latent_mask", "dl_pack_latent_inpaint", "dl_pack_latent_inpaint_f32", "dl_lcm_step_inpaint",
-    "dl_taesd_latent_in", "dl_taesd_latent_in_f32",
+    "dl_taesd_latent_in", "dl_taesd_latent_in_f32", "dl_lcm_step_ex", "dl_lcm_step_inpaint_ex",
 ]
 
 
@@ -60,6 +60,22 @@ class IgemmDesc(C.Structure):
 class LcmCoeffs(C.Structure):
     _fields_ = [("sqrt_alpha_t", C.c_float), ("sqrt_beta_t", C.c_float), ("c_skip", C.c_float),
                 ("c_out", C.c_float), ("sqrt_alpha_prev", C.c_float), ("sqrt_beta_prev", C.c_float)]
+
+
+class LcmCoeffsEx(C.Structure):
+    _fields_ = [("k", LcmCoeffs), ("prediction_type", C.c_int), ("clip_sample", C.c_int),
+                ("clip_sample_range", C.c_float)]
+
+
+PRED_EPSILON, PRED_V, PRED_SAMPLE = 0, 1, 2
+_PRED = {"epsilon": PRED_EPSILON, "v_prediction": PRED_V, "sample": PRED_SAMPLE}
+
+
+def _coeffs_ex(coeffs, prediction_type, clip_range) -> LcmCoeffsEx:
+    if prediction_type not in _PRED:
+        raise RuntimeError(f"lcm_step: prediction_type must be one of {sorted(_PRED)}, got {prediction_type!r}")
+    return LcmCoeffsEx(LcmCoeffs(*[float(v) for v in coeffs]), _PRED[prediction_type], int(clip_range is not None),
+                       0.0 if clip_range is None else float(clip_range))
 
 
 _lib = None
@@ -178,6 +194,11 @@ def load() -> C.CDLL:
             lib.dl_lcm_step_inpaint.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                 C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong,
                                                 C.POINTER(LcmCoeffs), C.c_float, C.c_float, C.c_int, C.c_void_p]
+            lib.dl_lcm_step_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                           C.c_longlong, C.POINTER(LcmCoeffsEx), C.c_void_p]
+            lib.dl_lcm_step_inpaint_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
+                                                   C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong,
+                                                   C.POINTER(LcmCoeffsEx), C.c_float, C.c_float, C.c_int, C.c_void_p]
             for f in (lib.dl_taesd_latent_in, lib.dl_taesd_latent_in_f32):
                 f.argtypes = [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]
             lib.dl_png_stored_size.restype = C.c_longlong
@@ -602,6 +623,17 @@ def lcm_step_inpaint(eps, x, noise, image_latents, noise0, mask, x_next, denoise
     _count()
 
 
+def lcm_step_inpaint_ex(model_output, x, noise, image_latents, noise0, mask, x_next, denoised, coeffs, add_noise,
+                        last, prediction_type="epsilon", clip_range=None):
+    """`lcm_step_inpaint` with the x0 of `lcm_step_ex` (prediction_type, clamp of x0 to [-clip_range, clip_range])."""
+    k = _coeffs_ex(coeffs, prediction_type, clip_range)
+    _check(load().dl_lcm_step_inpaint_ex(model_output.data_ptr(), x.data_ptr(), _ptr(noise), image_latents.data_ptr(),
+                                         _ptr(noise0), mask.data_ptr(), x_next.data_ptr(), denoised.data_ptr(),
+                                         mask.numel(), C.byref(k), float(add_noise[0]), float(add_noise[1]),
+                                         int(last), _stream()), "lcm_step_inpaint_ex")
+    _count()
+
+
 def vae_sample_latents(moments, eps_s, eps_n, out, *, scaling_factor, sqrt_alpha, sqrt_one_minus_alpha,
                        mean_out=None):
     """moments fp32 NHWC [n,h,w,8]; eps_s / eps_n fp32 NCHW [n,4,h,w]; out (mean_out) fp32 NHWC [n,h,w,4]."""
@@ -668,6 +700,15 @@ def lcm_step(eps, x, noise, x_next, denoised, coeffs):
     k = LcmCoeffs(*[float(v) for v in coeffs])
     _check(load().dl_lcm_step(eps.data_ptr(), x.data_ptr(), _ptr(noise), x_next.data_ptr(),
                               denoised.data_ptr(), x.numel(), C.byref(k), _stream()), "lcm_step")
+    _count()
+
+
+def lcm_step_ex(model_output, x, noise, x_next, denoised, coeffs, prediction_type="epsilon", clip_range=None):
+    """`LCMScheduler.step` of the model's scheduler config: x0 from the model output by prediction_type ("epsilon",
+    "v_prediction", "sample"), clamped to [-clip_range, clip_range] unless clip_range is None."""
+    k = _coeffs_ex(coeffs, prediction_type, clip_range)
+    _check(load().dl_lcm_step_ex(model_output.data_ptr(), x.data_ptr(), _ptr(noise), x_next.data_ptr(),
+                                 denoised.data_ptr(), x.numel(), C.byref(k), _stream()), "lcm_step_ex")
     _count()
 
 

@@ -283,11 +283,10 @@ class PatchParallelDenoiser:
               teacher=None):
         """Device tensors in, final latents NHWC out; no host sync (graph-capturable)."""
         from . import lib
-        from .scheduler import LCMSchedule
         pipe = self.pipe
         dev = pipe.device
         B, C, H, W = lat_nchw.shape
-        sched = LCMSchedule(steps)
+        sched = pipe.schedule(steps)                   # the pipeline's scheduler config
         kvs = pipe.unet.encode_context(pe)
         aug = pipe.unet.addition_embedding(*add) if add is not None else None
         tembs = pipe.unet.time_embeddings(sched.timesteps, B * repeat, we, aug)
@@ -318,7 +317,8 @@ class PatchParallelDenoiser:
             else:
                 eps = e_u.contiguous()
             x_next = torch.empty_like(x)
-            lib.lcm_step(eps, x, noise[i] if sched.has_noise(i) else None, x_next, den, sched.coeffs(i))
+            lib.lcm_step_ex(eps, x, noise[i] if sched.has_noise(i) else None, x_next, den, sched.coeffs(i),
+                            sched.prediction_type, sched.clip_range)
             if record is not None:
                 record.setdefault("noise_pred", []).append(eps.permute(0, 3, 1, 2).clone())
                 record.setdefault("latents", []).append(x_next.permute(0, 3, 1, 2).clone())

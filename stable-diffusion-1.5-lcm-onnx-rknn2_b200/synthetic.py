@@ -353,6 +353,8 @@ def write_model_dir(path: str, unet_cfg=None, vae_cfg=None, seed: int = 0, dtype
                                   if isinstance(unet_cfg.attention_head_dim, (tuple, list)) else unet_cfg.attention_head_dim),
            "norm_num_groups": unet_cfg.norm_num_groups, "norm_eps": unet_cfg.norm_eps,
            "time_cond_proj_dim": unet_cfg.time_cond_proj_dim}
+    if getattr(unet_cfg, "use_linear_projection", False):       # SD2.x-class (and SDXL) transformers
+        ucj["use_linear_projection"] = True
     if getattr(unet_cfg, "addition_embed_type", None):          # SDXL-class keys
         ucj.update(transformer_layers_per_block=list(unet_cfg.transformer_layers_per_block),
                    use_linear_projection=bool(unet_cfg.use_linear_projection),
