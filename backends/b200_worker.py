@@ -24,7 +24,7 @@ import json
 import collections
 import os
 import time
-from typing import List, Sequence, Tuple
+from typing import List, Optional, Sequence, Tuple
 
 import torch
 
@@ -37,6 +37,16 @@ def parse_size(size) -> Tuple[int, int]:
         return int(w_str), int(h_str)
     except Exception:
         raise RuntimeError(f"Invalid size '{size}', expected 'WIDTHxHEIGHT'")
+
+
+def request_sampler(req) -> str:
+    """A request's `sampler` (read with getattr; None means "lcm") -> its name.  RuntimeError for an unknown name,
+    and for a non-LCM sampler on an image-to-image or inpainting request (those run the LCM sampler only)."""
+    from dreamlab_b200.scheduler import check_sampler
+    s = check_sampler(getattr(req, "sampler", None))
+    if s != "lcm" and (getattr(req, "init_image", None) is not None or getattr(req, "mask_image", None) is not None):
+        raise RuntimeError(f"sampler {s!r}: image-to-image and inpainting requests run the LCM sampler only")
+    return s
 
 
 def _device_for(worker_id: int) -> str:
@@ -262,7 +272,7 @@ class B200Worker(PipelineWorker):
         (zeros are an SDXL-only convention, `force_zeros_for_empty_prompt`)."""
         return self._text.encode([""] * n)
 
-    def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True, init=None):
+    def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True, init=None, sampler="lcm"):
         """init (image-to-image): (u8 images [B,H,W,3], posterior draw [B,4,h,w], strength); lat is then the
         add_noise draw.  Inpainting appends (u8 masks [B,H,W], the masked image's posterior draw)."""
         pe = self._text.encode(prompts)
@@ -273,7 +283,7 @@ class B200Worker(PipelineWorker):
             if len(init) > 3:
                 i2i.update(mask_images=init[3], masked_posterior_noise=init[4])
         return self.pipe.generate(pe, lat, noise, steps, gs, return_latents=True, use_graph=self._use_graph,
-                                  negative_prompt_embeds=neg, decode=decode, **i2i)
+                                  negative_prompt_embeds=neg, decode=decode, sampler=sampler, **i2i)
 
     def _check_img2img(self) -> None:
         """Refuse image-to-image where this engine does not implement diffusers' semantics."""
@@ -347,9 +357,10 @@ class B200Worker(PipelineWorker):
         return width, height, seed
 
     def _draw(self, seed: int, h8: int, w8: int, steps: int, raw: bool = False, posterior: bool = False,
-              masked: bool = False):
+              masked: bool = False, draws: Optional[int] = None):
         """The reference's per-request Philox stream (`backends/cuda_worker.py:212-213`,
-        SURVEY.md App. A.5): latents first, then one draw per non-final step.
+        SURVEY.md App. A.5): latents first, then one draw per non-final step (draws: that many step draws instead,
+        what a non-LCM sampler consumes: `scheduler.sampler_noise_draws`).
         posterior (image-to-image): the posterior sample's draw comes first and is returned third; the
         "latents" draw is then the add_noise noise (diffusers' prepare_latents order).
         masked (inpainting): the masked image's posterior draw follows the latents draw (prepare_mask_latents runs
@@ -361,7 +372,7 @@ class B200Worker(PipelineWorker):
         lat = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32)
         eps_m = torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32) if masked else None
         noise = [torch.randn(shape, generator=gen, device=self.device, dtype=torch.float32)
-                 for _ in range(steps - 1)]
+                 for _ in range(steps - 1 if draws is None else draws)]
         if not raw:
             lat = lat.to(self.dtype).float()
             noise = [z.to(self.dtype).float() for z in noise]
@@ -393,6 +404,10 @@ class B200Worker(PipelineWorker):
             for (w, h, _), j in zip(parsed, jobs):
                 if (w, h) != (width, height) or int(j.req.num_inference_steps) != steps:
                     raise RuntimeError("run_batch: jobs must share size and num_inference_steps")
+            samplers = {request_sampler(j.req) for j in jobs}
+            if len(samplers) != 1:
+                raise RuntimeError("run_batch: jobs must share the sampler")
+            sampler = next(iter(samplers))
             inits = [getattr(j.req, "init_image", None) for j in jobs]
             masks = [getattr(j.req, "mask_image", None) for j in jobs]
             inpaint = any(m is not None for m in masks)
@@ -424,15 +439,17 @@ class B200Worker(PipelineWorker):
                     k, posterior = self._inpaint_plan(steps, strength)
             # per-request Philox streams; the round trip through the noise dtype (CUDA_DTYPE) is applied once to
             # the assembled batch instead of per tensor (same values, ~8 fewer launches per request)
-            draws = [self._draw(seed, height // 8, width // 8, k, raw=True, posterior=posterior, masked=inpaint)
-                     for _, _, seed in parsed]
+            from dreamlab_b200.scheduler import sampler_noise_draws
+            nd = k - 1 if sampler == "lcm" else sampler_noise_draws(sampler, steps)
+            draws = [self._draw(seed, height // 8, width // 8, k, raw=True, posterior=posterior, masked=inpaint,
+                                draws=nd) for _, _, seed in parsed]
             if posterior:
                 init[1] = torch.cat([d[2] for d in draws], 0).to(self.dtype).float()
             if inpaint:
                 init[4] = torch.cat([d[3] for d in draws], 0).to(self.dtype).float()
             lat = torch.cat([d[0] for d in draws], 0).to(self.dtype).float()
-            noise = (torch.stack([torch.cat([d[1][i] for d in draws], 0) for i in range(k - 1)]).to(self.dtype).float()
-                     if k > 1 else None)
+            noise = (torch.stack([torch.cat([d[1][i] for d in draws], 0) for i in range(nd)]).to(self.dtype).float()
+                     if nd > 0 else None)
             gs = torch.tensor([float(j.req.guidance_scale) for j in jobs])
             styles = {self._style_of(j.req) for j in jobs}
             if len(styles) != 1:
@@ -441,7 +458,8 @@ class B200Worker(PipelineWorker):
             try:
                 img, final = self._generate([str(j.req.prompt) for j in jobs], lat, noise, steps, gs,
                                             height, width, decode=not latents_only,
-                                            **({"init": tuple(init)} if init is not None else {}))
+                                            **({"init": tuple(init)} if init is not None else {}),
+                                            **({"sampler": sampler} if sampler != "lcm" else {}))
             finally:
                 self._apply_style(None, 0)          # reset: no state bleed into the next job
             from dreamlab_b200 import lib
@@ -547,7 +565,7 @@ class B200SDXLWorker(B200Worker):
         pooled = ucfg.projection_class_embeddings_input_dim - 6 * ucfg.addition_time_embed_dim
         return _SDXLTextEncoder(path, self.device, ucfg.cross_attention_dim, pooled, single=self._single)
 
-    def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True):
+    def _generate(self, prompts, lat, noise, steps, gs, height, width, decode=True, sampler="lcm"):
         pe, pooled = self._text.encode(prompts)
         neg = negp = None
         # `force_zeros_for_empty_prompt` (model_index.json; True for SDXL-base): zeros for the unconditional
@@ -556,7 +574,7 @@ class B200SDXLWorker(B200Worker):
             neg, negp = self._text.encode([""] * len(prompts))
         return self.pipe.generate(pe, lat, noise, steps, gs, return_latents=True, pooled_embeds=pooled,
                                   use_graph=self._use_graph, negative_prompt_embeds=neg,
-                                  negative_pooled_embeds=negp, decode=decode)
+                                  negative_pooled_embeds=negp, decode=decode, sampler=sampler)
 
 
 _ENCODERS = None

@@ -16,6 +16,12 @@ Pixels with L >= 128 are repainted, the others kept.  `strength` then defaults t
 schedule (int(steps * strength) of its last steps run).  A model whose UNet has 9 input channels (an inpainting UNet)
 serves only such requests.
 
+A request may name its sampler in `sampler`, also read with `getattr`: None or "lcm" (`LCMScheduler`, the default),
+"euler" (`EulerDiscreteScheduler`), "euler_a" (`EulerAncestralDiscreteScheduler`), "ddim" (`DDIMScheduler`, eta 0),
+"dpmpp_2m" (`DPMSolverMultistepScheduler`, DPM++ 2M) or "dpmpp_2m_karras" (the same on Karras sigmas), each built
+from the model's scheduler config.  These are the samplers guided models (vanilla SD1.5, SD2.x, SDXL base) are run
+with.  An unknown name is refused listing the accepted ones; image-to-image and inpainting requests run LCM only.
+
 Only names, fields and return conventions are shared with the reference — they ARE the
 interface; everything a caller can observe is pinned by `tests/test_worker_pool.py` and
 `tests/test_worker_factory.py`.
@@ -66,6 +72,7 @@ class GenSpec:
     init_image: Any = None                   # image-to-image: image bytes or HxWx3 uint8 array
     strength: Optional[float] = None         # image-to-image strength (None: 0.8; inpainting: 1.0)
     mask_image: Any = None                   # inpainting: image bytes or HxW uint8 array, with init_image
+    sampler: Optional[str] = None            # None / "lcm", "euler", "euler_a", "ddim", "dpmpp_2m", "dpmpp_2m_karras"
 
 
 @dataclass

@@ -125,7 +125,8 @@ def _batch_key(job, same_guidance: bool = False):
     """Generation jobs that may share one batched pass: same size, step count and style (and,
     for workers that run classifier-free guidance on a doubled batch, the same guidance scale).
     Image-to-image requests (an `init_image`) also share their strength: ("img2img", strength) is appended;
-    inpainting requests (a `mask_image`) append ("inpaint", strength) instead (default strength 1.0)."""
+    inpainting requests (a `mask_image`) append ("inpaint", strength) instead (default strength 1.0).  A request
+    with a non-LCM `sampler` appends ("sampler", name); the LCM sampler (the default) appends nothing."""
     req = getattr(job, "req", None)
     try:
         if same_guidance:
@@ -141,6 +142,9 @@ def _batch_key(job, same_guidance: bool = False):
         elif getattr(req, "init_image", None) is not None:
             st = getattr(req, "strength", None)
             key += (("img2img", 0.8 if st is None else float(st)),)
+        sampler = getattr(req, "sampler", None)
+        if sampler is not None and sampler != "lcm":
+            key += (("sampler", str(sampler)),)
         return key
     except Exception:
         return None

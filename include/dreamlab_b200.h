@@ -262,6 +262,33 @@ int dl_image_crop_u8(const float* src, int nimg, int hs, int ws, int c, int crop
 int dl_cfg_combine(const float* eps_uncond, const float* eps_text, float guidance_scale,
                    float* out, long long n, void* stream);
 
+/* ---- sampler step of the guided-model samplers (diffusers EulerDiscreteScheduler (s_churn 0),
+ * EulerAncestralDiscreteScheduler, DDIMScheduler (eta 0), DPMSolverMultistepScheduler (dpmsolver++, order 2,
+ * midpoint)), classifier-free guidance fused in.  One linear form restates each class's `step`:
+ *   e      = out_uncond + guidance_scale * (out_text - out_uncond)   (cfg_combine's roundings; out_text NULL: e = out_uncond)
+ *   x0     = a_x x + a_e e, clamped to [-clip_sample_range, clip_sample_range] when clip_sample != 0
+ *   x_next = c_x x + c_e e + c_0 x0 + c_1 x0_prev + c_n noise        (x0_prev / noise NULL: that term is left out)
+ * The host computes the coefficients (scheduler.py) from the diffusers lines:
+ *   Euler    pred_original_sample = sample - sigma * model_output (epsilon) |
+ *            model_output * (-sigma / (sigma**2 + 1) ** 0.5) + sample / (sigma**2 + 1) (v_prediction);
+ *            prev_sample = sample + (sample - pred_original_sample) / sigma * (sigma_next - sigma)
+ *   Euler-a  as Euler with sigma_down for sigma_next, + noise * sigma_up
+ *   DDIM     prev_sample = alpha_prod_t_prev ** 0.5 * pred_original_sample + (1 - alpha_prod_t_prev) ** 0.5 * pred_epsilon
+ *            (pred_epsilon from the unclamped model output: c_x, c_e)
+ *   DPM++    x_t = (sigma_t / sigma_s0) * sample - (alpha_t * (exp(-h) - 1)) * D0 - 0.5 * (alpha_t * (exp(-h) - 1)) * D1,
+ *            D0 = m0, D1 = (1 / r0) * (m0 - m1): c_0 / c_1 on x0 and x0_prev
+ * Every mul / add / sub is rounded on its own.  fp32 in and out; n % 4 == 0, operands 16-byte aligned.  x0 receives
+ * the step's x0 (the next step's x0_prev, and `denoised`).                                                     */
+typedef struct dl_sampler_coeffs {
+  float a_x, a_e;
+  float c_x, c_e, c_0, c_1, c_n;
+  int clip_sample;
+  float clip_sample_range;
+} dl_sampler_coeffs;
+int dl_sampler_step(const float* out_uncond, const float* out_text, float guidance_scale, const float* x,
+                    const float* x0_prev, const float* noise, float* x_next, float* x0, long long n,
+                    const dl_sampler_coeffs* coeffs /* host */, void* stream);
+
 /* ---- run_job_with_latents tail: fp32 adaptive_avg_pool2d -> (8,8) -> fp16 NCHW ------------- *
  * (reference `backends/cuda_worker.py:297-304`).  lat: fp32 NHWC [nimg,h,w,c]; out: fp16
  * [nimg,c,8,8].  Any h, w >= 1: adaptive_avg_pool2d bins [floor(i*h/8), ceil((i+1)*h/8)).      */

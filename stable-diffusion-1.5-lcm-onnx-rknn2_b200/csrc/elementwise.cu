@@ -358,6 +358,50 @@ __global__ void cfg_combine_kernel(const float4* __restrict__ u, const float4* _
   }
 }
 
+// ---- sampler step (Euler, Euler ancestral, DDIM, DPM++ 2M): guidance + one linear form, fused ----------------
+// e = u + gs (t - u) (cfg_combine's roundings; t == null: e = u);  x0 = clamp(a_x x + a_e e);
+// x_next = c_x x + c_e e + c_0 x0 + c_1 x0_prev + c_n z, every mul / add rounded on its own, summed left to right
+__global__ void sampler_step_kernel(const float4* __restrict__ u, const float4* __restrict__ t, float gs,
+                                    const float4* __restrict__ x, const float4* __restrict__ x0_prev,
+                                    const float4* __restrict__ noise, float4* __restrict__ x_next,
+                                    float4* __restrict__ x0_out, long long n4, dl_sampler_coeffs k) {
+  for (long long i = (long long)blockIdx.x * blockDim.x + threadIdx.x; i < n4;
+       i += (long long)gridDim.x * blockDim.x) {
+    const float4 uv = u[i], xv = x[i];
+    float e[4] = {uv.x, uv.y, uv.z, uv.w};
+    const float xx[4] = {xv.x, xv.y, xv.z, xv.w};
+    if (t != nullptr) {
+      const float4 tv = t[i];
+      const float tt[4] = {tv.x, tv.y, tv.z, tv.w};
+#pragma unroll
+      for (int j = 0; j < 4; ++j) e[j] = __fadd_rn(e[j], __fmul_rn(gs, __fsub_rn(tt[j], e[j])));
+    }
+    float pp[4] = {0.f, 0.f, 0.f, 0.f}, zz[4] = {0.f, 0.f, 0.f, 0.f};
+    if (x0_prev != nullptr) {
+      const float4 p = x0_prev[i];
+      pp[0] = p.x; pp[1] = p.y; pp[2] = p.z; pp[3] = p.w;
+    }
+    if (noise != nullptr) {
+      const float4 z = noise[i];
+      zz[0] = z.x; zz[1] = z.y; zz[2] = z.z; zz[3] = z.w;
+    }
+    float d[4], o[4];
+#pragma unroll
+    for (int j = 0; j < 4; ++j) {
+      float x0 = __fadd_rn(__fmul_rn(k.a_x, xx[j]), __fmul_rn(k.a_e, e[j]));
+      if (k.clip_sample) x0 = fminf(fmaxf(x0, -k.clip_sample_range), k.clip_sample_range);
+      float v = __fadd_rn(__fmul_rn(k.c_x, xx[j]), __fmul_rn(k.c_e, e[j]));
+      v = __fadd_rn(v, __fmul_rn(k.c_0, x0));
+      if (x0_prev != nullptr) v = __fadd_rn(v, __fmul_rn(k.c_1, pp[j]));
+      if (noise != nullptr) v = __fadd_rn(v, __fmul_rn(k.c_n, zz[j]));
+      d[j] = x0;
+      o[j] = v;
+    }
+    x0_out[i] = make_float4(d[0], d[1], d[2], d[3]);
+    x_next[i] = make_float4(o[0], o[1], o[2], o[3]);
+  }
+}
+
 // ---- fp32 adaptive_avg_pool2d -> (8,8) -> fp16, NHWC in, NCHW out -----------------------------
 __global__ void latent_pool8_kernel(const float* __restrict__ lat, int nimg, int h, int w, int c,
                                     __half* __restrict__ out) {
@@ -675,6 +719,25 @@ extern "C" int dl_cfg_combine(const float* eps_uncond, const float* eps_text, fl
       reinterpret_cast<const float4*>(eps_uncond), reinterpret_cast<const float4*>(eps_text),
       guidance_scale, reinterpret_cast<float4*>(out), n / 4);
   return check_launch("cfg_combine");
+}
+
+extern "C" int dl_sampler_step(const float* out_uncond, const float* out_text, float guidance_scale, const float* x,
+                               const float* x0_prev, const float* noise, float* x_next, float* x0, long long n,
+                               const dl_sampler_coeffs* k, void* stream_) {
+  DL_CHECK_ARG(out_uncond && x && x_next && x0 && k, "sampler_step: null pointer");
+  DL_CHECK_ARG(n > 0 && n % 4 == 0, "sampler_step: n must be a positive multiple of 4 (got %lld)", n);
+  const float* ptrs[] = {out_uncond, out_text, x, x0_prev, noise, x_next, x0};
+  for (const float* p : ptrs)
+    DL_CHECK_ARG(reinterpret_cast<uintptr_t>(p) % 16 == 0, "sampler_step: operands must be 16-byte aligned");
+  DL_CHECK_ARG(x0_prev != nullptr || k->c_1 == 0.f, "sampler_step: c_1 != 0 needs x0_prev");
+  DL_CHECK_ARG(noise != nullptr || k->c_n == 0.f, "sampler_step: c_n != 0 needs noise");
+  DL_CHECK_ARG(!k->clip_sample || k->clip_sample_range >= 0.f, "sampler_step: clip_sample_range must be >= 0");
+  sampler_step_kernel<<<grid_for(n / 4, 256), 256, 0, STREAM>>>(
+      reinterpret_cast<const float4*>(out_uncond), reinterpret_cast<const float4*>(out_text), guidance_scale,
+      reinterpret_cast<const float4*>(x), reinterpret_cast<const float4*>(x0_prev),
+      reinterpret_cast<const float4*>(noise), reinterpret_cast<float4*>(x_next), reinterpret_cast<float4*>(x0),
+      n / 4, *k);
+  return check_launch("sampler_step");
 }
 
 extern "C" int dl_latent_pool8(const float* lat, int nimg, int h, int w, int c, void* out_f16,

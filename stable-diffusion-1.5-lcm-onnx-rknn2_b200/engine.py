@@ -20,7 +20,8 @@ from typing import List, Optional
 import torch
 
 from . import lib
-from .scheduler import DEFAULT_CONFIG, LCMSchedule, SchedulerConfig, guidance_scale_embedding
+from .scheduler import (DEFAULT_CONFIG, LCMSchedule, SchedulerConfig, check_sampler, guidance_scale_embedding,
+                        sampler_schedule)
 from .weights import Packed, has_vae_encoder, pack_taesd_decoder, pack_unet, pack_vae_decoder, pack_vae_encoder
 
 BF16 = torch.bfloat16
@@ -404,7 +405,8 @@ class UNetB200:
 
     @torch.no_grad()
     def forward(self, latents_nhwc: torch.Tensor, temb: torch.Tensor, kvs: List[List[torch.Tensor]],
-                eps_out: Optional[torch.Tensor] = None, repeat: int = 1, comm=None, inpaint_cond=None) -> torch.Tensor:
+                eps_out: Optional[torch.Tensor] = None, repeat: int = 1, comm=None, inpaint_cond=None,
+                in_scale: float = 1.0) -> torch.Tensor:
         """latents_nhwc fp32 [b,h,w,4] -> noise_pred fp32 [b*repeat,h,w,4].  repeat=2 is the
         classifier-free-guidance doubled batch `cat([latents]*2)`: the same latents are packed
         twice, temb / kvs carry the [uncond, cond] halves.
@@ -412,6 +414,8 @@ class UNetB200:
         inpaint_cond (a 9-channel inpainting UNet, and only there): (latent mask fp32 [b,h,w], masked_image_latents
         fp32 NHWC [b,h,w,4]); the UNet input is cat([latents, mask, masked_image_latents]) per image, doubled
         together with the latents under guidance.
+
+        in_scale: the samplers' `scale_model_input` (Euler: 1 / sqrt(sigma^2 + 1)), applied as the latents are packed.
 
         comm (patch parallel, SURVEY.md §8e): this rank computes rows
         [rank*h/R, (rank+1)*h/R) of every image and returns that strip [b*repeat, h/R, w, 4];
@@ -442,7 +446,7 @@ class UNetB200:
                 lib.pack_latent_inpaint(latents_nhwc, inpaint_cond[0], inpaint_cond[1], xin, repeat=repeat)
             else:
                 for r in range(repeat):
-                    lib.pack_latent(latents_nhwc, xin[r * b0:(r + 1) * b0], cin=Cin)
+                    lib.pack_latent(latents_nhwc, xin[r * b0:(r + 1) * b0], cin=Cin, scale=in_scale)
         else:
             n_lv = len(ch)
             if H % (comm.world << (n_lv - 1)):
@@ -454,7 +458,8 @@ class UNetB200:
             xp = torch.zeros(B, hl + 2, W, 64, device=self.device, dtype=self.dt)
             for r in range(repeat):
                 for i in range(b0):
-                    lib.pack_latent(latents_nhwc[i, lo:hi], xp[r * b0 + i, lo - (r0 - 1):hi - (r0 - 1)], cin=Cin)
+                    lib.pack_latent(latents_nhwc[i, lo:hi], xp[r * b0 + i, lo - (r0 - 1):hi - (r0 - 1)], cin=Cin,
+                                    scale=in_scale)
             xin = Padded(xp)
             H = hl
         h = conv3x3(ctx, xin, P["conv_in_w"], P["conv_in_b"], ch[0], feeds_norm=True)
@@ -934,10 +939,11 @@ class _StaticGraph:
     """One captured CUDA graph of the whole hot path for a fixed (B, h, w, steps[, gs][, strength][, inpaint]).
     strength set: image-to-image; the init images and the posterior draw are static inputs too, and `lat`
     holds the add_noise draw.  inpaint: the masks and the masked image's posterior draw are static inputs as well,
-    and `noise` holds one draw per non-final step of the truncated schedule."""
+    and `noise` holds one draw per non-final step of the truncated schedule.  sampler (text-to-image only): `noise`
+    holds the draws the sampler consumes (none for the deterministic ones; a one-entry placeholder then)."""
 
     def __init__(self, pipe: "LCMPipelineB200", B, h, w, steps, cfg_scale=None, decode=True, strength=None,
-                 inpaint=False):
+                 inpaint=False, sampler="lcm"):
         dev = pipe.device
         ucfg = pipe.unet.cfg
         D = ucfg.cross_attention_dim
@@ -951,8 +957,11 @@ class _StaticGraph:
             self.add = (torch.zeros(Bc, pdim, device=dev, dtype=torch.float32),
                         torch.zeros(Bc, 6, device=dev, dtype=torch.float32))
         self.lat = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
-        k = len(pipe.schedule(steps, strength, inpaint).timesteps) if inpaint else steps
-        self.noise = torch.zeros(max(k - 1, 1), B, 4, h, w, device=dev, dtype=torch.float32)
+        if sampler != "lcm":
+            nd = pipe.schedule(steps, sampler=sampler).n_draws
+        else:
+            nd = (len(pipe.schedule(steps, strength, inpaint).timesteps) if inpaint else steps) - 1
+        self.noise = torch.zeros(max(nd, 1), B, 4, h, w, device=dev, dtype=torch.float32)
         self.steps = steps
         self.init_u8 = self.eps_s = self.mask_u8 = self.eps_m = None
         if strength is not None:
@@ -963,7 +972,7 @@ class _StaticGraph:
             self.eps_m = torch.zeros(B, 4, h, w, device=dev, dtype=torch.float32)
         args = (self.pe, self.w_emb, self.lat, self.noise, steps)
         kw = dict(add=self.add, cfg_scale=cfg_scale, decode=decode, init_u8=self.init_u8, eps_s=self.eps_s,
-                  strength=strength, mask_u8=self.mask_u8, eps_m=self.eps_m)
+                  strength=strength, mask_u8=self.mask_u8, eps_m=self.eps_m, sampler=sampler)
         with CAPTURE_LOCK:
             # warm-up on a side stream (lazy per-device init: smem attributes, module load)
             s = torch.cuda.Stream(device=dev)
@@ -1044,7 +1053,8 @@ class LCMPipelineB200:
     @torch.no_grad()
     def run_static(self, pe_bf16, w_emb, lat_nchw, noise_nchw, steps: int, record: dict = None,
                    add=None, cfg_scale: Optional[float] = None, teacher=None, decode: bool = True,
-                   init_u8=None, eps_s=None, strength: Optional[float] = None, mask_u8=None, eps_m=None):
+                   init_u8=None, eps_s=None, strength: Optional[float] = None, mask_u8=None, eps_m=None,
+                   sampler: str = "lcm"):
         """Everything on device, no host sync, graph-capturable.  Returns (u8 images, latents).
         pe_bf16 / add carry 2B rows ([uncond, cond]) when cfg_scale is set.
         init_u8 (image-to-image): u8 NHWC init images; the pass becomes encode -> posterior sample with eps_s ->
@@ -1053,7 +1063,7 @@ class LCMPipelineB200:
         posterior draw, the schedule is the truncated one and noise_nchw holds its non-final steps' draws."""
         B = lat_nchw.shape[0]
         Bu = 2 * B if cfg_scale is not None else B
-        sched = self.schedule(steps, strength if init_u8 is not None else None, mask_u8 is not None)
+        sched = self.schedule(steps, strength if init_u8 is not None else None, mask_u8 is not None, sampler)
         kvs = self.unet.encode_context(pe_bf16)
         aug = self.unet.addition_embedding(*add) if add is not None else None
         tembs = self.unet.time_embeddings(sched.timesteps, Bu, w_emb, aug)
@@ -1130,10 +1140,15 @@ class LCMPipelineB200:
                 record["masked_image_latents"] = masked.permute(0, 3, 1, 2).clone()
         return start, dict(cond=(mask, masked) if nine else None, blend=None if nine else (image, noise, mask))
 
-    def schedule(self, steps: int, strength: Optional[float] = None, inpaint: bool = False) -> LCMSchedule:
+    def schedule(self, steps: int, strength: Optional[float] = None, inpaint: bool = False, sampler: str = "lcm"):
         """The pass's schedule: text-to-image (strength None), image-to-image (re-spaced by strength) or
-        inpainting (the full schedule truncated by strength)."""
+        inpainting (the full schedule truncated by strength).  sampler: "lcm" (`LCMSchedule`), or one of the
+        guided-model samplers of `scheduler.SAMPLERS` (text-to-image only)."""
         cfg = self.scheduler_config
+        if check_sampler(sampler) != "lcm":
+            if strength is not None or inpaint:
+                raise RuntimeError(f"sampler {sampler!r}: image-to-image and inpainting run the LCM sampler only")
+            return sampler_schedule(sampler, steps, cfg)
         if inpaint:
             return LCMSchedule(steps, strength, truncate=True, config=cfg)
         return LCMSchedule(steps, config=cfg) if strength is None else LCMSchedule(steps, strength, config=cfg)
@@ -1157,8 +1172,11 @@ class LCMPipelineB200:
             self._pool = torch.cuda.graph_pool_handle()
         return self._pool
 
-    def graph_for(self, B, h, w, steps, cfg_scale=None, decode=True, strength=None, inpaint=False) -> _StaticGraph:
+    def graph_for(self, B, h, w, steps, cfg_scale=None, decode=True, strength=None, inpaint=False,
+                  sampler="lcm") -> _StaticGraph:
         key = (B, h, w, steps, cfg_scale, decode)
+        if sampler != "lcm":                                     # the LCM keys stay as they were
+            key += ("sampler", sampler)
         if inpaint:                                              # inpainting: its own graph per strength
             key += ("inpaint", strength)
         elif strength is not None:                               # image-to-image: its own graph per strength
@@ -1168,7 +1186,7 @@ class LCMPipelineB200:
             while len(self._graphs) >= self.max_graphs:          # least recently used goes first
                 self._graphs.pop(next(iter(self._graphs)))
             with torch.cuda.device(self.device):
-                g = _StaticGraph(self, B, h, w, steps, cfg_scale, decode, strength, inpaint)
+                g = _StaticGraph(self, B, h, w, steps, cfg_scale, decode, strength, inpaint, sampler)
         self._graphs[key] = g                                     # dict order = recency
         return g
 
@@ -1182,7 +1200,10 @@ class LCMPipelineB200:
         blend fused into the scheduler step.
         teacher (parity tests): fp32 NCHW [steps,B,4,h,w] — the latents fed to the UNet at step i
         come from this tensor (an oracle trajectory) instead of from the previous step, so every
-        step's noise_pred is compared on identical inputs (teacher forcing)."""
+        step's noise_pred is compared on identical inputs (teacher forcing).
+        A guided-model sampler's schedule (not `LCMSchedule`) runs `_denoise_sampler`."""
+        if not isinstance(sched, LCMSchedule):
+            return self._denoise_sampler(latents_nchw, step_noise_nchw, sched, kvs, tembs, record, cfg_scale, teacher)
         B, C, H, W = latents_nchw.shape
         if start_nhwc is not None:
             x = start_nhwc
@@ -1232,6 +1253,63 @@ class LCMPipelineB200:
             x = x_next
         return x
 
+    def _denoise_sampler(self, latents_nchw, step_noise_nchw, sched, kvs, tembs, record, cfg_scale, teacher):
+        """Text-to-image with a guided-model sampler: latents * init_noise_sigma, then per step the UNet on
+        x * in_scale(i) and one `lib.sampler_step` (guidance fused).  step_noise holds sched.n_draws draws.  The
+        x0 of the previous step (DPM++'s second-order term) stays in one of two device buffers."""
+        B, C, H, W = latents_nchw.shape
+        n = len(sched.timesteps)
+        f32 = dict(device=self.device, dtype=torch.float32)
+        x = torch.empty(B, H, W, C, **f32)
+        lib.nchw_to_nhwc_f32(latents_nchw, x)
+        if sched.init_noise_sigma != 1.0:
+            # latents * init_noise_sigma as the step's x0 with a_x = sigma (a_e = 0 leaves e out of the product)
+            x_init = torch.empty_like(x)
+            lib.sampler_step(x, None, 1.0, x, None, None, torch.empty_like(x), x_init,
+                             (sched.init_noise_sigma, 0.0, 0.0, 0.0, 0.0, 0.0, 0.0))
+            x = x_init
+        noise = None
+        if sched.n_draws:
+            noise = torch.empty(sched.n_draws, B, H, W, C, **f32)
+            lib.nchw_to_nhwc_f32(step_noise_nchw[:sched.n_draws].reshape(sched.n_draws * B, C, H, W),
+                                 noise.view(sched.n_draws * B, H, W, C))
+        den = (torch.empty_like(x), torch.empty_like(x))
+        tx = None
+        if teacher is not None:
+            tx = torch.empty(n, B, H, W, C, **f32)
+            lib.nchw_to_nhwc_f32(teacher.to(self.device, torch.float32).reshape(n * B, C, H, W).contiguous(),
+                                 tx.view(n * B, H, W, C))
+        k = 0                                                   # draws consumed so far
+        for i in range(n):
+            if tx is not None:
+                x = tx[i]
+            s = sched.in_scale(i)
+            if cfg_scale is None:
+                out = self.unet.forward(x, tembs[i], kvs, in_scale=s)
+                u, t = out, None
+            else:
+                out = self.unet.forward(x, tembs[i], kvs, repeat=2, in_scale=s)
+                u, t = out[:B], out[B:]
+            z = None
+            if sched.has_noise(i):
+                z, k = noise[k], k + 1
+            x_next = torch.empty_like(x)
+            lib.sampler_step(u, t, 1.0 if cfg_scale is None else cfg_scale, x,
+                             den[(i + 1) % 2] if sched.uses_prev_x0(i) else None, z, x_next, den[i % 2],
+                             sched.coeffs(i), sched.clip_range)
+            if record is not None:
+                if t is None:
+                    record.setdefault("noise_pred", []).append(out.permute(0, 3, 1, 2).clone())
+                else:
+                    guided = torch.empty_like(x)
+                    lib.cfg_combine(u, t, cfg_scale, guided)
+                    record.setdefault("noise_pred", []).append(guided.permute(0, 3, 1, 2).clone())
+                    record.setdefault("noise_pred_raw", []).append(out.permute(0, 3, 1, 2).clone())
+                record.setdefault("latents", []).append(x_next.permute(0, 3, 1, 2).clone())
+                record.setdefault("denoised", []).append(den[i % 2].permute(0, 3, 1, 2).clone())
+            x = x_next
+        return x
+
     def _conditioning(self, prompt_embeds, pooled_embeds, time_ids, negative_prompt_embeds,
                       negative_pooled_embeds, cfg_scale, height, width):
         """-> (context rows, (pooled, time_ids) or None), doubled [uncond, cond] under CFG.
@@ -1262,7 +1340,7 @@ class LCMPipelineB200:
                  use_graph: bool = False, pooled_embeds=None, time_ids=None,
                  negative_prompt_embeds=None, negative_pooled_embeds=None, teacher_latents=None,
                  decode: bool = True, init_images=None, strength: Optional[float] = None, posterior_noise=None,
-                 mask_images=None, masked_posterior_noise=None):
+                 mask_images=None, masked_posterior_noise=None, sampler: str = "lcm"):
         """Public entry: host or device tensors in -> u8 images [B,H,W,3] on device (and the
         final latents NHWC fp32 if asked).  With use_graph the whole pass is one CUDA-graph
         replay; the returned tensors are the graph's static outputs (consume before next call).
@@ -1277,11 +1355,18 @@ class LCMPipelineB200:
         latents_nchw is the latents / add_noise draw, posterior_noise the image's posterior draw (needed by a 4-channel
         UNet, and by a 9-channel one at strength < 1), masked_posterior_noise the masked image's (9-channel UNets);
         step_noise_nchw holds len(truncated schedule) - 1 draws.  A 9-channel (inpainting) UNet serves nothing else;
-        classifier-free guidance applies as for text-to-image."""
+        classifier-free guidance applies as for text-to-image.
+
+        sampler: "lcm" (`LCMScheduler`, the default), or "euler", "euler_a", "ddim", "dpmpp_2m", "dpmpp_2m_karras"
+        (text-to-image only; `scheduler.sampler_schedule`).  step_noise_nchw then holds the draws the sampler consumes:
+        num_inference_steps for "euler_a", none for the others (None is accepted)."""
         B, _, h, w = latents_nchw.shape
         steps = int(num_inference_steps)
         nine = getattr(self.unet.cfg, "in_channels", 4) == 9
         inpaint = mask_images is not None
+        sampler = check_sampler(sampler)
+        if sampler != "lcm" and (init_images is not None or inpaint):
+            raise RuntimeError(f"sampler {sampler!r}: image-to-image and inpainting run the LCM sampler only")
         k = steps                                         # steps that run (inpainting: the truncated schedule's)
         if nine and not inpaint:
             raise RuntimeError("this model's UNet has in_channels=9 (an inpainting UNet): it serves inpainting only "
@@ -1317,6 +1402,10 @@ class LCMPipelineB200:
             self.schedule(steps, strength)                # ValueError for a strength the schedule cannot serve
         else:
             strength = None
+        # step noise draws the pass consumes
+        nd = k - 1 if sampler == "lcm" else self.schedule(steps, sampler=sampler).n_draws
+        if nd > 0 and (step_noise_nchw is None or step_noise_nchw.shape[0] < nd):
+            raise RuntimeError(f"step_noise_nchw: {nd} draws [{nd}, {B}, 4, {h}, {w}] expected")
         if use_graph and record is None and teacher_latents is None:
             Bp = next((b for b in self.batch_buckets if b >= B), B)
             if Bp != B:
@@ -1330,14 +1419,14 @@ class LCMPipelineB200:
                     return torch.cat([t] + [t[tuple(idx)]] * (Bp - B), dim)
                 gs = torch.as_tensor(guidance_scale, dtype=torch.float32).reshape(-1)
                 out = self.generate(pad(prompt_embeds), pad(latents_nchw),
-                                    pad(step_noise_nchw, 1) if k > 1 else step_noise_nchw, steps,
+                                    pad(step_noise_nchw, 1) if nd > 0 else step_noise_nchw, steps,
                                     pad(gs) if gs.numel() > 1 else guidance_scale, return_latents=True, use_graph=True,
                                     pooled_embeds=pad(pooled_embeds), time_ids=pad(time_ids),
                                     negative_prompt_embeds=pad(negative_prompt_embeds),
                                     negative_pooled_embeds=pad(negative_pooled_embeds), decode=decode,
                                     init_images=pad(init_images), strength=strength,
                                     posterior_noise=pad(posterior_noise), mask_images=pad(mask_images),
-                                    masked_posterior_noise=pad(masked_posterior_noise))
+                                    masked_posterior_noise=pad(masked_posterior_noise), sampler=sampler)
                 img, lat = out
                 img = img[:B] if img is not None else None
                 return (img, lat[:B]) if return_latents else img
@@ -1347,7 +1436,7 @@ class LCMPipelineB200:
                                          negative_pooled_embeds, cfg_scale, 8 * h, 8 * w)
         with torch.cuda.device(self.device):
             if use_graph and record is None and teacher_latents is None:
-                g = self.graph_for(B, h, w, steps, cfg_scale, decode, strength, inpaint)
+                g = self.graph_for(B, h, w, steps, cfg_scale, decode, strength, inpaint, sampler)
                 # host inputs go through pinned staging: a copy from PAGEABLE host memory first waits for the stream to
                 # drain (CUDA's documented behaviour), i.e. for the previous batch — the thread could then not enqueue
                 # this batch behind it
@@ -1358,8 +1447,8 @@ class LCMPipelineB200:
                     g.add[0].copy_(_pinned(add[0]), non_blocking=True)
                     g.add[1].copy_(_pinned(add[1]), non_blocking=True)
                 g.lat.copy_(_pinned(latents_nchw), non_blocking=True)
-                if k > 1:
-                    g.noise.copy_(_pinned(step_noise_nchw), non_blocking=True)
+                if nd > 0:
+                    g.noise.copy_(_pinned(step_noise_nchw[:nd]), non_blocking=True)
                 if strength is not None:
                     g.init_u8.copy_(_pinned(init_images), non_blocking=True)
                     if posterior_noise is not None:
@@ -1377,7 +1466,7 @@ class LCMPipelineB200:
                     add = (add[0].to(self.device), add[1].to(self.device))
                 lat0 = latents_nchw.to(self.device, torch.float32).contiguous()
                 nz = (step_noise_nchw.to(self.device, torch.float32).contiguous()
-                      if k > 1 else None)
+                      if nd > 0 else None)
                 init = eps = mask = eps_m = None
                 if strength is not None:
                     init = init_images.to(self.device).contiguous()
@@ -1389,5 +1478,5 @@ class LCMPipelineB200:
                         eps_m = masked_posterior_noise.to(self.device, torch.float32).contiguous()
                 img, lat = self.run_static(pe, we, lat0, nz, steps, record, add=add, cfg_scale=cfg_scale,
                                            teacher=teacher_latents, decode=decode, init_u8=init, eps_s=eps,
-                                           strength=strength, mask_u8=mask, eps_m=eps_m)
+                                           strength=strength, mask_u8=mask, eps_m=eps_m, sampler=sampler)
         return (img, lat) if return_latents else img

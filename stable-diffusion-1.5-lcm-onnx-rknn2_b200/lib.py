@@ -32,7 +32,7 @@ EXPORTS = [
     "dl_im2col_s2_pad01", "dl_im2col_s2_pad01_f32", "dl_pack_image_im2col", "dl_pack_image_im2col_f32",
     "dl_vae_sample_latents", "dl_pack_image_im2col_masked", "dl_pack_image_im2col_masked_f32",
     "dl_inpaint_latent_mask", "dl_pack_latent_inpaint", "dl_pack_latent_inpaint_f32", "dl_lcm_step_inpaint",
-    "dl_taesd_latent_in", "dl_taesd_latent_in_f32", "dl_lcm_step_ex", "dl_lcm_step_inpaint_ex",
+    "dl_taesd_latent_in", "dl_taesd_latent_in_f32", "dl_lcm_step_ex", "dl_lcm_step_inpaint_ex", "dl_sampler_step",
 ]
 
 
@@ -65,6 +65,11 @@ class LcmCoeffs(C.Structure):
 class LcmCoeffsEx(C.Structure):
     _fields_ = [("k", LcmCoeffs), ("prediction_type", C.c_int), ("clip_sample", C.c_int),
                 ("clip_sample_range", C.c_float)]
+
+
+class SamplerCoeffs(C.Structure):
+    _fields_ = [("a_x", C.c_float), ("a_e", C.c_float), ("c_x", C.c_float), ("c_e", C.c_float), ("c_0", C.c_float),
+                ("c_1", C.c_float), ("c_n", C.c_float), ("clip_sample", C.c_int), ("clip_sample_range", C.c_float)]
 
 
 PRED_EPSILON, PRED_V, PRED_SAMPLE = 0, 1, 2
@@ -199,6 +204,9 @@ def load() -> C.CDLL:
             lib.dl_lcm_step_inpaint_ex.argtypes = [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p,
                                                    C.c_void_p, C.c_void_p, C.c_void_p, C.c_longlong,
                                                    C.POINTER(LcmCoeffsEx), C.c_float, C.c_float, C.c_int, C.c_void_p]
+            lib.dl_sampler_step.argtypes = [C.c_void_p, C.c_void_p, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p,
+                                            C.c_void_p, C.c_void_p, C.c_longlong, C.POINTER(SamplerCoeffs),
+                                            C.c_void_p]
             for f in (lib.dl_taesd_latent_in, lib.dl_taesd_latent_in_f32):
                 f.argtypes = [C.c_void_p, C.c_longlong, C.c_void_p, C.c_void_p]
             lib.dl_png_stored_size.restype = C.c_longlong
@@ -765,6 +773,26 @@ def image_crop_u8(src, crop_h, crop_w, dst_window):
 def cfg_combine(eps_uncond, eps_text, guidance_scale, out):
     _check(load().dl_cfg_combine(eps_uncond.data_ptr(), eps_text.data_ptr(), float(guidance_scale),
                                  out.data_ptr(), out.numel(), _stream()), "cfg_combine")
+    _count()
+
+
+def sampler_step(out_uncond, out_text, guidance_scale, x, x0_prev, noise, x_next, x0, coeffs, clip_range=None):
+    """One step of a guided-model sampler (`scheduler.py` schedules): e = out_uncond + guidance_scale * (out_text -
+    out_uncond) (out_text None: e = out_uncond), x0 = a_x x + a_e e clamped to [-clip_range, clip_range] unless
+    clip_range is None, x_next = c_x x + c_e e + c_0 x0 + c_1 x0_prev + c_n noise.  coeffs = (a_x, a_e, c_x, c_e,
+    c_0, c_1, c_n); fp32 tensors of x's size."""
+    n = x.numel()
+    for name, t in (("out_uncond", out_uncond), ("out_text", out_text), ("x0_prev", x0_prev), ("noise", noise),
+                    ("x_next", x_next), ("x0", x0)):
+        if t is not None and (t.numel() != n or t.dtype != torch.float32 or not t.is_contiguous()):
+            raise RuntimeError(f"sampler_step: {name} must be a contiguous fp32 tensor of {n} elements")
+    k = SamplerCoeffs(*[float(v) for v in coeffs], int(clip_range is not None),
+                      0.0 if clip_range is None else float(clip_range))
+    with _timed("sampler_step", 0.0, 4.0 * n * (4 + (out_text is not None) + (x0_prev is not None)
+                                               + (noise is not None))):
+        _check(load().dl_sampler_step(out_uncond.data_ptr(), _ptr(out_text), float(guidance_scale), x.data_ptr(),
+                                      _ptr(x0_prev), _ptr(noise), x_next.data_ptr(), x0.data_ptr(), n, C.byref(k),
+                                      _stream()), "sampler_step")
     _count()
 
 
